@@ -2,7 +2,7 @@
 """Benchmark of the warp + SSIM/L1 photometric-loss hot path (BASELINE.json metric:
 "warp+SSIM/L1 loss fwd+bwd frames/s at 192x640").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload kitti|scannet]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload kitti|scannet] [--dump-outputs DIR]
 
 One *step* = one `Compute_Loss.forward` + `.backward()` over one synthetic minibatch
 (config 2 of BASELINE.json: B=8 KITTI-shaped 3-frame snippets at 192x640, forward and
@@ -30,6 +30,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark leaves the tree as it found it (which may be read-only)
 # stdout must carry exactly one JSON line, but NCCL writes its version banner to fd 1: park the
 # real stdout and route everything else that lands on fd 1 to stderr
 _REAL_STDOUT = os.dup(1)
@@ -114,6 +115,8 @@ def make_inputs(wl, seed, device, pin=False, slab=False):
 
 
 def run_step(loss_mod, inp, n_src, need_value=False):
+    """One training-step loss: forward + backward.  Returns the loss dict (every entry [1]); the gradients are left
+    in `.grad` of the disparity / pose tensors of `inp`."""
     n_scales = loss_mod.num_scales
     disps = [inp["disp%d" % j].requires_grad_(True) for j in range(1 + n_src)]
     extra = [[inp["disp%d_s%d" % (j, sc)].requires_grad_(True) for sc in range(1, n_scales)] for j in range(1 + n_src)]
@@ -123,9 +126,28 @@ def run_step(loss_mod, inp, n_src, need_value=False):
         t.grad = None
     out = loss_mod([inp["source%d" % j] for j in range(n_src)], inp["target"], [poses, poses_inv],
                    [[d] + ex for d, ex in zip(disps, extra)], inp["K"])
-    total = out["total"]            # [1]; backward() on it directly, like train_mono.py:193
-    total.backward()
-    return total
+    out["total"].backward()         # [1]; backward() on it directly, like train_mono.py:193
+    return out
+
+
+def step_outputs(out, inp):
+    """Host copies of what one run_step call gave its caller: the loss terms and the gradients of its inputs."""
+    arrays = {"loss_" + k: v for k, v in out.items()}
+    arrays.update({"grad_" + k: t.grad for k, t in inp.items() if t.grad is not None})
+    return {k: v.detach().cpu().numpy() for k, v in arrays.items()}
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(arrays, out_dir):
+    import numpy as np
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:        # every workload of WORKLOADS stays far below (kitti: 11.8 MB)
+        raise SystemExit("--dump-outputs: %d bytes of outputs exceed the %d-byte limit" % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 class ClockSampler(threading.Thread):
@@ -588,8 +610,15 @@ def main():
                          "'fast' keeps geometry, warp and masks bit-exact and evaluates the SSIM statistics at tolerance level")
     ap.add_argument("--only", default=None, choices=["loss"], help="'loss': skip the pft / train / eager-CUDA sub-benchmarks")
     ap.add_argument("--sequence-frames", type=int, default=0, help="PFT workloads: also time a whole sequence of this many frames")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="loss-step workloads: write what the last timed step returned (loss terms, gradients of the "
+                         "disparities and poses; rank 0) to DIR/<name>.npy")
     args = ap.parse_args()
     ref_arm = args.impl == "reference"
+    if args.dump_outputs and (ref_arm or args.workload not in WORKLOADS):
+        ap.error("--dump-outputs needs --impl ours and one of the workloads %s" % ", ".join(sorted(WORKLOADS)))
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.steps is None:
         args.steps = 20 if ref_arm else 2000
     if args.warmup is None:
@@ -660,11 +689,13 @@ def main():
                 out_ = run_step(loss_mod, s_, n_src)
             graphs.append((g_, out_))
 
+    eager_out = [None]          # without graphs: the loss dict of the latest step
+
     def step_resident(i):
         if graphs is not None:
             graphs[i % N_INPUT_SETS][0].replay()
         else:
-            run_step(loss_mod, sets[i % N_INPUT_SETS], n_src)
+            eager_out[0] = run_step(loss_mod, sets[i % N_INPUT_SETS], n_src)
 
     # End-to-end arm: every step copies its inputs from pinned host memory and reads the loss back to the host.  Two
     # device-side input buffers are used so that the copy of step i+1 (copy stream) overlaps the compute of step i
@@ -684,7 +715,7 @@ def main():
         h = host_sets[i % 2]
         if e2e is None:
             inp = {k: v.to(dev, non_blocking=True) for k, v in h.items()}
-            loss_holder[0] = float(run_step(loss_mod, inp, n_src).detach())   # device -> host read of the loss
+            loss_holder[0] = float(run_step(loss_mod, inp, n_src)["total"].detach())   # device -> host read of the loss
             return
         k = i % 2
         with torch.cuda.stream(copy_stream), torch.no_grad():
@@ -695,7 +726,7 @@ def main():
         main.wait_event(e2e["h2d_done"][k])
         graph_k, loss_k = e2e["in"][k]
         graph_k.replay()
-        e2e["loss_host"][k].copy_(loss_k.detach(), non_blocking=True)
+        e2e["loss_host"][k].copy_(loss_k["total"].detach(), non_blocking=True)
         e2e["compute_done"][k].record(main)
         if i > 0:                                                     # read the previous step's loss
             e2e["compute_done"][1 - k].synchronize()
@@ -710,6 +741,10 @@ def main():
     ms_total = R.timed(step_resident, args.steps)
     launches = _timing.LAUNCH_COUNT - launches0
     clocks = sampler.summary() if sampler else None
+    if args.dump_outputs and rank == 0:
+        # now: the passes below run the step again into the same tensors, one of them with the other arithmetic
+        last = (args.steps - 1) % N_INPUT_SETS
+        dump_outputs(step_outputs(graphs[last][1] if graphs is not None else eager_out[0], sets[last]), args.dump_outputs)
 
     # per-launch device time of the library calls, live over a second (eager) pass of the same steps
     # (the device is first parked on a ~2 ms spin so that the whole step is already queued when it starts executing:
@@ -762,7 +797,7 @@ def main():
             main.wait_event(e2e["h2d_done"][k])
             graph_k, loss_k = e2e["in"][k]
             graph_k.replay()
-            e2e["loss_host"][k].copy_(loss_k.detach(), non_blocking=True)
+            e2e["loss_host"][k].copy_(loss_k["total"].detach(), non_blocking=True)
             e2e["compute_done"][k].record(main)
             if i > 0:
                 e2e["compute_done"][1 - k].synchronize()

@@ -1,9 +1,14 @@
-"""Generates tests/golden/*.npz from the UNMODIFIED reference (``/root/reference``)
-imported on CPU in the build container.  Run:  python tests/golden/make_golden.py
+"""Generates tests/golden/*.npz and tests/golden/fresh/ from the UNMODIFIED
+reference imported on CPU.
+Run:  TCSFM_REFERENCE_ROOT=<checkout of the reference> python tests/golden/make_golden.py
 
 The reference ships no golden vectors of its own (SURVEY.md §4/§8c); these
 fixtures are the pin for ``oracle/`` and for the CUDA path.  Inputs are stored
-next to the outputs so that the fixtures do not depend on RNG reproducibility.
+next to the outputs of the cases so that they do not depend on RNG
+reproducibility; the fresh fixture stores a digest of its seeded inputs instead.
+
+``--fresh-from-oracle`` writes only the fresh fixture, from oracle/ref_torch.py,
+for where the reference is not at hand; its ``source`` entry says so.
 """
 import os
 import sys
@@ -17,11 +22,12 @@ ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 sys.path.insert(0, ROOT)
 
+import goldens  # noqa: E402
 import refshim  # noqa: E402
 from tcsfm_b200 import synth  # noqa: E402
 
 torch.set_num_threads(1)
-ref = refshim.load_reference()
+ref = None                  # the reference modules, loaded in __main__
 
 TRAIN_CFG = {"l1_weight": 0.15, "l_ssim_weight": 0.85, "l_smooth_weight": 0.05, "num_scales": 1,
              "l_depth_consist_weight": 0.14, "min_depth": 0.06, "max_depth": 2.67, "l_smooth": False,
@@ -156,7 +162,26 @@ def gen_case(name, b, h, w, seed, yaw):
     print(name, "->", path, "%.1f KB" % (os.path.getsize(path) / 1024))
 
 
+def gen_fresh(fns, source):
+    fr = synth.make_frames(**goldens.FRESH_FRAMES)
+    out = {k: v.numpy() for k, v in goldens.fresh_outputs(fr, **fns).items()}
+    for k in out:               # 0/1 masks are stored as bytes
+        if k.endswith("valid_mask"):
+            assert set(np.unique(out[k]).tolist()) <= {0.0, 1.0}, k
+            out[k] = out[k].astype(np.uint8)
+    out["in/sha256"] = np.array(goldens.fresh_inputs_digest(fr))
+    out["source"] = np.array(source)
+    os.makedirs(os.path.dirname(goldens.FRESH_PATH), exist_ok=True)
+    np.savez_compressed(goldens.FRESH_PATH, **out)
+    print("fresh ->", goldens.FRESH_PATH, "%.1f KB" % (os.path.getsize(goldens.FRESH_PATH) / 1024))
+
+
 if __name__ == "__main__":
+    if sys.argv[1:] == ["--fresh-from-oracle"]:
+        gen_fresh(goldens.fresh_fns_oracle(), "oracle/ref_torch.py")
+        sys.exit(0)
+    ref = refshim.load_reference()
     gen_case("small_b2_24x40", 2, 24, 40, seed=1, yaw=0.01)
     gen_case("mid_b2_64x96", 2, 64, 96, seed=2, yaw=0.01)
     gen_case("yaw_b2_32x48", 2, 32, 48, seed=3, yaw=0.09)     # ~5 deg: large OOB band
+    gen_fresh(goldens.fresh_fns_reference(ref), "reference")

@@ -1,22 +1,23 @@
 """Import harness for the upstream reference (test infrastructure only).
 
-The reference (``/root/reference``) is pure Python/PyTorch but imports a few
-packages that are not installed here (``liegroups``, ``pykitti``,
-``matplotlib``) from modules the hot path never touches.  This harness
-registers empty stand-ins for them and returns the reference's own modules so
-that golden vectors can be generated from, and the oracle pinned against, the
-real thing.  It is only usable where ``/root/reference`` exists (this
-container); nothing marked ``gpu``, ``smoke()`` or ``bench.py`` may call it.
+The reference (a checkout of utiasSTARS/tightly-coupled-SfM named by the
+environment variable ``TCSFM_REFERENCE_ROOT``) is pure Python/PyTorch but
+imports a few packages that need not be installed (``liegroups``,
+``pykitti``, ``matplotlib``) from modules the hot path never touches.  This
+harness registers empty stand-ins for them and returns the reference's own
+modules so that golden vectors can be generated from, and the oracle pinned
+against, the real thing.  Without that checkout the tests that need it skip;
+nothing marked ``gpu``, ``smoke()`` or ``bench.py`` may call it.
 """
 import os
 import sys
 import types
 
-REF_ROOT = os.environ.get("TCSFM_REFERENCE_ROOT", "/root/reference")
+REF_ROOT = os.environ.get("TCSFM_REFERENCE_ROOT", "")
 
 
 def reference_available() -> bool:
-    return os.path.isfile(os.path.join(REF_ROOT, "models", "stn.py"))
+    return bool(REF_ROOT) and os.path.isfile(os.path.join(REF_ROOT, "models", "stn.py"))
 
 
 def _stub(name, **attrs):
@@ -30,7 +31,7 @@ def load_reference():
     """Returns a namespace with the reference modules ``stn``, ``losses``,
     ``train_mono``, ``optimizer``, ``helpers`` and ``learning_helpers``."""
     if not reference_available():
-        raise RuntimeError("reference tree not found at %s" % REF_ROOT)
+        raise RuntimeError("reference tree not found: set TCSFM_REFERENCE_ROOT to a checkout of the reference")
     dummy = type("Dummy", (), {})
     _stub("liegroups", SE3=dummy, SO3=dummy)
     _stub("liegroups.torch", SE3=dummy, SO3=dummy)

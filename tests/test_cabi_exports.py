@@ -29,7 +29,10 @@ def test_library_builds_and_exports_header_symbols():
 
 
 def test_library_targets_sm_100a():
-    out = subprocess.run(["cuobjdump", "-lelf", _lib.LIB_PATH], capture_output=True, text=True).stdout
+    # the cuobjdump of the toolkit that built the library, which need not be on PATH; when nvcc itself was found only
+    # through PATH, build._nvcc() returns the bare "nvcc" and cuobjdump is looked up on PATH as well
+    cuobjdump = os.path.join(os.path.dirname(build._nvcc()), "cuobjdump")
+    out = subprocess.run([cuobjdump, "-lelf", _lib.LIB_PATH], capture_output=True, text=True).stdout
     assert "sm_100a" in out, out
 
 

@@ -1,6 +1,7 @@
 """Pins oracle/ref_torch.py (the CPU restatement) to the reference: bit-for-bit
-against the committed golden vectors that the unmodified reference produced, and
-against the live reference where /root/reference is present."""
+against the committed golden vectors that the unmodified reference produced; the
+stored fresh-input vectors are also checked against the live reference where
+TCSFM_REFERENCE_ROOT names a checkout of it."""
 import types
 
 import pytest
@@ -133,20 +134,21 @@ def test_photometric_error_matches_golden(case):
         assert same(res[k], g.t("photo/%s" % k)), k
 
 
-@pytest.mark.skipif(not refshim.reference_available(), reason="reference tree not present")
 def test_oracle_matches_live_reference_on_fresh_inputs():
+    """Inputs that none of the golden cases uses (the second source warped with the outer depths, both euler2mat, the
+    smoothness loss, the pairwise diff / mask), against the outputs stored in tests/golden/fresh/ (its `source` entry
+    names what wrote them; test_fresh_fixture_matches_live_reference checks them against the reference itself)."""
+    fr = synth.make_frames(**goldens.FRESH_FRAMES)
+    stored = goldens.load_fresh()
+    assert goldens.fresh_inputs_digest(fr) == str(stored["in/sha256"]), "the seeded inputs changed"
+    for k, v in goldens.fresh_outputs(fr, **goldens.fresh_fns_oracle()).items():
+        assert same(v, torch.from_numpy(stored[k])), k
+
+
+@pytest.mark.skipif(not refshim.reference_available(), reason="needs TCSFM_REFERENCE_ROOT: a checkout of the reference")
+def test_fresh_fixture_matches_live_reference():
     ref = refshim.load_reference()
-    fr = synth.make_frames(2, 40, 56, n_src=2, seed=11, yaw=0.03)
-    ref.stn.pixel_coords = None
-    a = ref.stn.inverse_warp2(fr["sources"][1], fr["depths"][0], fr["depths"][2], -fr["poses"][1], fr["K"], "zeros")
-    b = O.inverse_warp2(fr["sources"][1], fr["depths"][0], fr["depths"][2], -fr["poses"][1], fr["K"])
-    for x, y in zip(a, b):
-        assert same(x, y)
-    assert same(ref.stn.euler2mat(fr["poses"][0][:, 3:]), O.euler_to_matrix(fr["poses"][0][:, 3:]))
-    assert same(ref.geometry_helpers.euler2mat(fr["poses"][0][:, 3:]), O.euler_to_matrix(fr["poses"][0][:, 3:]))
-    assert same(ref.losses.get_smooth_loss(fr["disps"][0], fr["target"]), O.smooth_loss(fr["disps"][0], fr["target"]))
-    cfg = goldens.FULL_CFG
-    ra = ref.losses.Compute_Loss(cfg).compute_pairwise_loss(fr["target"], fr["sources"][0], fr["depths"][0],
-                                                            fr["depths"][1], -fr["poses"][0], fr["K"], 5)
-    rb = O.pairwise_loss(cfg, fr["target"], fr["sources"][0], fr["depths"][0], fr["depths"][1], -fr["poses"][0], fr["K"])
-    assert same(ra[2], rb[2]) and same(ra[3], rb[3])
+    fr = synth.make_frames(**goldens.FRESH_FRAMES)
+    stored = goldens.load_fresh()
+    for k, v in goldens.fresh_outputs(fr, **goldens.fresh_fns_reference(ref)).items():
+        assert same(v, torch.from_numpy(stored[k])), k
