@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define TCSFM_ABI_VERSION 16
+#define TCSFM_ABI_VERSION 17
 
 /* ---- flags ------------------------------------------------------------------ */
 /* Arithmetic flavour.  Eager PyTorch rounds after every operator, but a few ATen
@@ -265,30 +265,21 @@ typedef struct tcsfm_frame_cfg {
     int64_t n_min_pixels;   /* B*H*W: the mean of losses.py:132                                     */
 } tcsfm_frame_cfg;
 
-/* out_sum[0] = sum_i min_j base[j*stride + i], j < count, i < n  (losses.py:129-131). */
-int tcsfm_min_reduce(const float* base, int64_t stride, int count, int64_t n, float* out_sum, void* stream);
-/* tcsfm_min_reduce + tcsfm_frame_finalize as one launch: the last block to add its partial sum computes the loss
- * terms.  ticket [1]: scratch. */
-int tcsfm_min_reduce_finalize(const float* base, int64_t stride, int count, int64_t n, float* out_sum, int* ticket,
-                              const float* sums, const tcsfm_frame_cfg* cfg, float* out, float* total, void* stream);
+/* out_sum[0] = sum_i min_j base[j*stride + i], j < count, i < n  (losses.py:129-131).  With `cfg` != NULL the
+ * launch also does tcsfm_frame_finalize(sums, out_sum, cfg, out, total): the last block to add its partial sum
+ * computes the loss terms; ticket [1]: scratch.  With `cfg` == NULL, ticket, sums, out and total are ignored. */
+int tcsfm_min_reduce(const float* base, int64_t stride, int count, int64_t n, float* out_sum, int* ticket,
+                     const float* sums, const tcsfm_frame_cfg* cfg, float* out, float* total, void* stream);
 
-/* Near-ties of that minimum: the same sum, plus (tie_list [capacity], tie_count [1], both device int32) the flat
- * indices i whose two smallest candidates differ by less than `band` (or involve a NaN).  tcsfm_pair_tie_resolve
- * then overwrites diff_img[i] of every listed group with the value the exact arithmetic gives, so that the arg-min
- * routing of the backward (torch.min, first index on ties) is the reference's even when the maps were produced by
- * TCSFM_ARITH_FAST.  groups: the competing (forward) groups in candidate order, forward fields filled. */
-int tcsfm_min_reduce_ties(const float* base, int64_t stride, int count, int64_t n, float* out_sum, float band,
-                          int* tie_list, int* tie_count, int capacity, void* stream);
-int tcsfm_pair_tie_resolve(const tcsfm_pair_group* groups, int n_groups, int B, int H, int W,
-                           float w_l1, float w_ssim, int flags, const int* tie_list, const int* tie_count, int capacity,
-                           void* stream);
-
-/* The two calls above as ONE launch (no tie list in global memory): every block takes the min of its pixels,
- * keeps its near-ties in shared memory and re-evaluates them with the exact arithmetic right away.  out_sum [1]:
- * sum over the B*H*W pixels of the min over the groups' diff_img (values as the forward produced them);
- * counters [2]: (number of pixels re-evaluated, scratch).  With `cfg` != NULL the last block to finish also does
- * tcsfm_frame_finalize(sums, out_sum, cfg, out_terms, out_total).  Replaces torch.min(reconstruction_errors, 1)[0]
- * of losses.py:129-131 under the fast arithmetic. */
+/* The same minimum over the diff_img of `groups` (the competing forward groups in candidate order, forward fields
+ * filled), with its near-ties re-decided:
+ * every block takes the min of its pixels, keeps in shared memory those whose two smallest candidates differ by less
+ * than `band` (or involve a NaN) and overwrites their diff_img entries in every group with the value the exact
+ * arithmetic gives, so that the arg-min routing of the backward (torch.min, first index on ties) is the reference's
+ * even when the maps were produced by TCSFM_ARITH_FAST.  out_sum [1]: sum over the B*H*W pixels of the min over the
+ * groups' diff_img (values as the forward produced them); counters [2]: (number of pixels re-evaluated, scratch).
+ * With `cfg` != NULL the last block to finish also does tcsfm_frame_finalize(sums, out_sum, cfg, out_terms,
+ * out_total).  Replaces torch.min(reconstruction_errors, 1)[0] of losses.py:129-131 under the fast arithmetic. */
 int tcsfm_pair_min_resolve(const tcsfm_pair_group* groups, int n_groups, int B, int H, int W,
                            float w_l1, float w_ssim, int flags, float band, float* out_sum, int* counters,
                            const float* sums, const tcsfm_frame_cfg* cfg, float* out_terms, float* out_total,
@@ -302,13 +293,11 @@ int tcsfm_pair_min_resolve(const tcsfm_pair_group* groups, int n_groups, int B, 
 int tcsfm_frame_finalize(const float* sums, const float* min_sum, const tcsfm_frame_cfg* cfg, float* out, float* total,
                          void* stream);
 /* Upstream gradients of the three terms (g_out[3], may be NULL) and of their sum (g_total[1],
- * may be NULL) -> g_scalars [G,2] and g_min [1], the upstream scalars tcsfm_pair_loss_bwd consumes. */
+ * may be NULL) -> g_scalars [G,2] and g_min [1], the upstream scalars tcsfm_pair_loss_bwd consumes.
+ * With `zero` != NULL the launch also zero-fills it (n_zero floats, 16-byte aligned, n_zero % 4 == 0): the
+ * accumulated depth-gradient buffer of the shared-gradient backward pair launch.  NULL = no fill. */
 int tcsfm_frame_bwd_prepare(const float* g_out, const float* g_total, const tcsfm_frame_cfg* cfg, float* g_scalars,
-                            float* g_min, void* stream);
-/* The same, and the launch also zero-fills `zero` (n_zero floats, 16-byte aligned, n_zero % 4 == 0): the accumulated
- * depth-gradient buffer of the shared-gradient backward pair launch. */
-int tcsfm_frame_bwd_prepare_zero(const float* g_out, const float* g_total, const tcsfm_frame_cfg* cfg, float* g_scalars,
-                                 float* g_min, float* zero, int64_t n_zero, void* stream);
+                            float* g_min, float* zero, int64_t n_zero, void* stream);
 
 #ifdef __cplusplus
 }

@@ -159,7 +159,7 @@ def test_pair_loss_multi_group_and_partial_tiles():
         assert rel_l2(g_rd[i], rd_l.grad) < 1e-4
 
 
-def test_bad_arguments_report_errors():
+def test_bad_arguments_return_errors():
     fr = synth.make_frames(1, 8, 8, seed=0)
     kinv, proj = stn.projection_matrices(-fr["poses"][0], fr["K"])
     with pytest.raises(RuntimeError, match="bad shape"):
@@ -181,7 +181,7 @@ def test_bad_arguments_report_errors():
     assert rc != 0 and b"channel stride out of range" in emu().tcsfm_last_error()
     # the frame-level upstream needs at least one of its two gradient pointers
     cfg = _raw.make_frame_cfg([0, 1], 0.3, 0.14, 64)
-    rc = emu().tcsfm_frame_bwd_prepare(None, None, ctypes.byref(cfg), dummy.data_ptr(), dummy.data_ptr(), None)
+    rc = emu().tcsfm_frame_bwd_prepare(None, None, ctypes.byref(cfg), dummy.data_ptr(), dummy.data_ptr(), None, 0, None)
     assert rc != 0 and b"tcsfm_frame_bwd_prepare" in emu().tcsfm_last_error()
 
 

@@ -824,10 +824,11 @@ def test_graphed_train_step_matches_eager():
         assert float((p - q).abs().mean()) < 2e-5, float((p - q).abs().mean())
 
 
-def test_min_resolve_one_launch_equals_the_two_launch_form():
-    """tcsfm_pair_min_resolve (per-pixel min + exact re-evaluation of its near-ties, ties kept in shared memory) against
-    tcsfm_min_reduce_ties + tcsfm_pair_tie_resolve at config 2: same patched diff maps, same tie count, same sum; the
-    patched values are the exact kernels' and the arg-min over the sources is the exact arithmetic's everywhere."""
+def test_min_resolve_restores_the_reference_routing():
+    """tcsfm_pair_min_resolve (per-pixel min + exact re-evaluation of its near-ties, ties kept in shared memory) at
+    config 2 re-evaluates exactly the near-ties found on the host from the forward's maps: their values become the
+    exact kernels', every other value is left as it was, the arg-min over the sources is the exact arithmetic's
+    everywhere, and the sum is the one of the maps as the forward produced them."""
     from tcsfm_b200 import _raw
     L = _lib.lib()
     fr = frames(8, 192, 640, 0.01, synth.KITTI_DEPTH_RANGE, seed=31)
@@ -845,19 +846,20 @@ def test_min_resolve_one_launch_equals_the_two_launch_form():
 
     _, d_exact = forward(flags)
     fast = flags | _cabi.ARITH_FAST
-    batch_a, d_a = forward(fast)
-    n_px = d_a[0].numel()
-    sum_a, tie_list, tie_count = _raw.min_reduce_ties(L, d_a[0], n_px, 2, n_px)
-    _raw.pair_tie_resolve(L, batch_a, [0, 1], 0.15, 0.85, fast, tie_list, tie_count)
-    batch_b, d_b = forward(fast)
-    sum_b, count_b = _raw.pair_min_resolve(L, batch_b, [0, 1], 0.15, 0.85, fast)
-    assert int(count_b) == int(tie_count) > 0
-    assert torch.equal(d_a, d_b)
-    assert abs(float(sum_a) - float(sum_b)) <= 1e-5 * abs(float(sum_a))
-    idx = tie_list[:int(tie_count)].long()
+    batch, d = forward(fast)
+    before = d.clone()
+    # the kernel's rule in fp32: a NaN in either candidate, or the two closer than the band
+    a, b = before.reshape(2, -1)
+    band = torch.tensor(_raw.TIE_BAND, dtype=torch.float32, device=a.device)
+    ties = a.isnan() | b.isnan() | ~(torch.maximum(a, b) - torch.minimum(a, b) >= band)
+    min_sum, tie_count = _raw.pair_min_resolve(L, batch, [0, 1], 0.15, 0.85, fast)
+    assert int(tie_count) == int(ties.sum()) > 0
     for j in range(2):
-        assert torch.equal(d_b[j].flatten()[idx], d_exact[j].flatten()[idx])
-    assert torch.equal(torch.min(d_b.reshape(2, -1), 0)[1], torch.min(d_exact.reshape(2, -1), 0)[1])
+        assert torch.equal(d[j].flatten()[ties], d_exact[j].flatten()[ties])
+        assert torch.equal(d[j].flatten()[~ties], before[j].flatten()[~ties])
+    assert torch.equal(torch.min(d.reshape(2, -1), 0)[1], torch.min(d_exact.reshape(2, -1), 0)[1])
+    want = float(torch.min(before.reshape(2, -1), 0)[0].sum())
+    assert abs(float(min_sum) - want) <= 1e-5 * abs(want)
 
 
 def test_intrinsics_inverse_bit_exact_vs_torch_cuda():

@@ -2,7 +2,7 @@
 package loader and by the test-only emulator binding)."""
 import ctypes as C
 
-ABI_VERSION = 16
+ABI_VERSION = 17
 
 ARITH_CPU = 1 << 0
 AUTO_MASK = 1 << 1
@@ -78,22 +78,17 @@ SIGNATURES = {
                                                    C.c_int, C.c_int, C.c_int, C.c_float, C.c_float, C.c_void_p]),
     "tcsfm_disp_upsample_to_depth_bwd": (C.c_int, [C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.c_int,
                                                    C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, C.c_void_p]),
-    "tcsfm_min_reduce": (C.c_int, [_fp, _i64, C.c_int, _i64, _fp, C.c_void_p]),
+    "tcsfm_min_reduce": (C.c_int, [_fp, _i64, C.c_int, _i64, _fp, _fp, _fp, C.POINTER(FrameCfg), _fp, _fp, C.c_void_p]),
     "tcsfm_u8_to_float": (C.c_int, [_fp, _fp, _i64, C.c_void_p]),
     "tcsfm_intrinsics_inverse": (C.c_int, [_fp, _fp, C.c_int, C.c_void_p]),
     "tcsfm_frame_prologue": (C.c_int, [C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.c_int, _i64, C.c_float, C.c_float,
                                        C.POINTER(C.c_void_p), C.c_int, C.c_int, C.c_float, _fp, C.c_int, _fp, _fp, C.c_int, C.c_void_p]),
     "tcsfm_frame_epilogue": (C.c_int, [C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.c_int, _i64, C.c_float,
                                        C.POINTER(C.c_void_p), C.c_int, C.c_int, C.c_float, _fp, C.c_int, _fp, _fp, C.c_void_p]),
-    "tcsfm_min_reduce_ties": (C.c_int, [_fp, _i64, C.c_int, _i64, _fp, C.c_float, _fp, _fp, C.c_int, C.c_void_p]),
-    "tcsfm_pair_tie_resolve": (C.c_int, [C.POINTER(PairGroup), C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, C.c_float,
-                                         C.c_int, _fp, _fp, C.c_int, C.c_void_p]),
     "tcsfm_pair_min_resolve": (C.c_int, [C.POINTER(PairGroup), C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, C.c_float,
                                          C.c_int, C.c_float, _fp, _fp, _fp, C.POINTER(FrameCfg), _fp, _fp, C.c_void_p]),
-    "tcsfm_min_reduce_finalize": (C.c_int, [_fp, _i64, C.c_int, _i64, _fp, _fp, _fp, C.POINTER(FrameCfg), _fp, _fp, C.c_void_p]),
     "tcsfm_frame_finalize": (C.c_int, [_fp, _fp, C.POINTER(FrameCfg), _fp, _fp, C.c_void_p]),
-    "tcsfm_frame_bwd_prepare": (C.c_int, [_fp, _fp, C.POINTER(FrameCfg), _fp, _fp, C.c_void_p]),
-    "tcsfm_frame_bwd_prepare_zero": (C.c_int, [_fp, _fp, C.POINTER(FrameCfg), _fp, _fp, _fp, _i64, C.c_void_p]),
+    "tcsfm_frame_bwd_prepare": (C.c_int, [_fp, _fp, C.POINTER(FrameCfg), _fp, _fp, _fp, _i64, C.c_void_p]),
 }
 
 

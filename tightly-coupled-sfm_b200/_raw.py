@@ -23,6 +23,15 @@ def _stream(t):
     return None
 
 
+def _call(lib, fn, name, is_cuda, *args, launches=1):
+    """fn(*args), one entry point of `lib`: timed as `name` while a kernel timer is recording (CUDA calls only), its
+    return code checked, and the `launches` kernels it issues added to the launch count."""
+    with _timing.launch(name, is_cuda):
+        rc = fn(*args)
+    _cabi.check(lib, rc)
+    _timing.count_launch(launches)
+
+
 def _f32c(t, name):
     if t is None:
         return None
@@ -74,12 +83,10 @@ def warp_fwd(lib, img, depth, ref_depth, kinv, proj, flags=0, need_depths=True, 
     if stack_target is not None:
         tgt, tsb, tsc = image_view(stack_target, "stack_target")
         stack = torch.empty((b, 6, h, w), dtype=torch.float32, device=img.device)
-    with _timing.launch("warp_fwd", img.is_cuda):
-        rc = lib.tcsfm_warp_fwd(_ptr(img), sb, sc, _ptr(depth), _ptr(ref_depth), _ptr(kinv), _ptr(proj),
-                                _ptr(out_img), _ptr(out_valid), _ptr(out_pd), _ptr(out_cd),
-                                _ptr(tgt), tsb, tsc, _ptr(stack), b, h, w, flags, _stream(img))
-    _cabi.check(lib, rc)
-    _timing.count_launch()
+    _call(lib, lib.tcsfm_warp_fwd, "warp_fwd", img.is_cuda,
+          _ptr(img), sb, sc, _ptr(depth), _ptr(ref_depth), _ptr(kinv), _ptr(proj),
+          _ptr(out_img), _ptr(out_valid), _ptr(out_pd), _ptr(out_cd),
+          _ptr(tgt), tsb, tsc, _ptr(stack), b, h, w, flags, _stream(img))
     if stack_target is not None:
         return out_img, out_valid, out_pd, out_cd, stack
     return out_img, out_valid, out_pd, out_cd
@@ -107,13 +114,11 @@ def warp_bwd(lib, img, depth, ref_depth, kinv, proj, g_img, g_pd, g_cd, flags=0,
     g_ref = torch.empty((b, 1, h, w), dtype=torch.float32, device=dev) if need_ref_depth_grad else None
     g_proj = torch.empty((b, 3, 4), dtype=torch.float32, device=dev)
     g_src = torch.empty((b, 3, h, w), dtype=torch.float32, device=dev) if need_img_grad else None
-    with _timing.launch("warp_bwd", img.is_cuda):
-        rc = lib.tcsfm_warp_bwd(_ptr(img), sb, sc, _ptr(depth), _ptr(ref_depth), _ptr(kinv), _ptr(proj),
-                                _ptr(g_img), _ptr(g_pd), _ptr(g_cd), _ptr(g_stack),
-                                _ptr(g_depth), _ptr(g_ref), _ptr(g_proj), _ptr(g_src),
-                                b, h, w, flags, _stream(img))
-    _cabi.check(lib, rc)
-    _timing.count_launch()
+    _call(lib, lib.tcsfm_warp_bwd, "warp_bwd", img.is_cuda,
+          _ptr(img), sb, sc, _ptr(depth), _ptr(ref_depth), _ptr(kinv), _ptr(proj),
+          _ptr(g_img), _ptr(g_pd), _ptr(g_cd), _ptr(g_stack),
+          _ptr(g_depth), _ptr(g_ref), _ptr(g_proj), _ptr(g_src),
+          b, h, w, flags, _stream(img))
     return g_depth, g_ref, g_proj, g_src
 
 
@@ -123,10 +128,7 @@ def ssim_fwd(lib, x, y, flags=0):
         raise ValueError("ssim: x and y must be [B,C,H,W] of equal shape")
     b, c, h, w = x.shape
     out = torch.empty_like(x)
-    with _timing.launch("ssim_fwd", x.is_cuda):
-        rc = lib.tcsfm_ssim_fwd(_ptr(x), _ptr(y), _ptr(out), b * c, h, w, flags, _stream(x))
-    _cabi.check(lib, rc)
-    _timing.count_launch()
+    _call(lib, lib.tcsfm_ssim_fwd, "ssim_fwd", x.is_cuda, _ptr(x), _ptr(y), _ptr(out), b * c, h, w, flags, _stream(x))
     return out
 
 
@@ -135,10 +137,8 @@ def ssim_bwd(lib, x, y, g_out, need_x=True, need_y=True, flags=0):
     b, c, h, w = x.shape
     g_x = torch.empty_like(x) if need_x else None
     g_y = torch.empty_like(x) if need_y else None
-    with _timing.launch("ssim_bwd", x.is_cuda):
-        rc = lib.tcsfm_ssim_bwd(_ptr(x), _ptr(y), _ptr(g_out), _ptr(g_x), _ptr(g_y), b * c, h, w, flags, _stream(x))
-    _cabi.check(lib, rc)
-    _timing.count_launch()
+    _call(lib, lib.tcsfm_ssim_bwd, "ssim_bwd", x.is_cuda,
+          _ptr(x), _ptr(y), _ptr(g_out), _ptr(g_x), _ptr(g_y), b * c, h, w, flags, _stream(x))
     return g_x, g_y
 
 
@@ -149,10 +149,7 @@ def ssim_mean_fwd(lib, x, y, flags=0):
         raise ValueError("ssim: x and y must be [B,C,H,W] of equal shape")
     b, c, h, w = x.shape
     out = torch.empty((1,), dtype=torch.float32, device=x.device)
-    with _timing.launch("ssim_mean_fwd", x.is_cuda):
-        rc = lib.tcsfm_ssim_mean_fwd(_ptr(x), _ptr(y), _ptr(out), b * c, h, w, flags, _stream(x))
-    _cabi.check(lib, rc)
-    _timing.count_launch()
+    _call(lib, lib.tcsfm_ssim_mean_fwd, "ssim_mean_fwd", x.is_cuda, _ptr(x), _ptr(y), _ptr(out), b * c, h, w, flags, _stream(x))
     return out
 
 
@@ -161,10 +158,8 @@ def ssim_mean_bwd(lib, x, y, g_mean, need_x=True, need_y=True, flags=0):
     b, c, h, w = x.shape
     g_x = torch.empty_like(x) if need_x else None
     g_y = torch.empty_like(x) if need_y else None
-    with _timing.launch("ssim_mean_bwd", x.is_cuda):
-        rc = lib.tcsfm_ssim_mean_bwd(_ptr(x), _ptr(y), _ptr(g_mean), _ptr(g_x), _ptr(g_y), b * c, h, w, flags, _stream(x))
-    _cabi.check(lib, rc)
-    _timing.count_launch()
+    _call(lib, lib.tcsfm_ssim_mean_bwd, "ssim_mean_bwd", x.is_cuda,
+          _ptr(x), _ptr(y), _ptr(g_mean), _ptr(g_x), _ptr(g_y), b * c, h, w, flags, _stream(x))
     return g_x, g_y
 
 
@@ -173,10 +168,7 @@ def intrinsics_inverse(lib, K):
     _expect(K, (K.shape[0], 3, 3), "intrinsics")
     K = _f32c(K, "intrinsics")
     out = torch.empty_like(K)
-    with _timing.launch("intrinsics_inverse", K.is_cuda):
-        rc = lib.tcsfm_intrinsics_inverse(_ptr(K), _ptr(out), K.shape[0], _stream(K))
-    _cabi.check(lib, rc)
-    _timing.count_launch()
+    _call(lib, lib.tcsfm_intrinsics_inverse, "intrinsics_inverse", K.is_cuda, _ptr(K), _ptr(out), K.shape[0], _stream(K))
     return out
 
 
@@ -190,10 +182,7 @@ def u8_to_float(lib, src, out=None):
         out = torch.empty(src.shape, dtype=torch.float32, device=src.device)
     elif out.dtype != torch.float32 or out.shape != src.shape or not out.is_contiguous():
         raise ValueError("u8_to_float: `out` must be a contiguous fp32 tensor of the input's shape")
-    with _timing.launch("u8_to_float", src.is_cuda):
-        rc = lib.tcsfm_u8_to_float(_ptr(src), _ptr(out), src.numel(), _stream(src))
-    _cabi.check(lib, rc)
-    _timing.count_launch()
+    _call(lib, lib.tcsfm_u8_to_float, "u8_to_float", src.is_cuda, _ptr(src), _ptr(out), src.numel(), _stream(src))
     return out
 
 
@@ -245,10 +234,8 @@ def pair_loss_fwd(lib, batch, w_l1, w_ssim, flags, want_diff=True, want_grad=Tru
         a.mask = _ptr(mask[i])
         a.sums = _ptr(sums[i])
         a.coef = _ptr(coef[i]) if want_grad else None
-    with _timing.launch("pair_loss_fwd", dev.type == "cuda"):
-        rc = lib.tcsfm_pair_loss_fwd(batch.arr, g, b, h, w, w_l1, w_ssim, flags, batch.stream())
-    _cabi.check(lib, rc)
-    _timing.count_launch()
+    _call(lib, lib.tcsfm_pair_loss_fwd, "pair_loss_fwd", dev.type == "cuda",
+          batch.arr, g, b, h, w, w_l1, w_ssim, flags, batch.stream())
     return diff, mask, sums, coef
 
 
@@ -268,10 +255,8 @@ def pair_loss_bwd(lib, batch, mask, sums, coef, g_diff, g_scalars, w_l1, w_ssim,
         a.g_tgt_depth = _ptr(g_td[i])
         a.g_ref_depth = _ptr(g_rd[i]) if need_ref_depth_grad else None
         a.g_proj = _ptr(g_proj[i])
-    with _timing.launch("pair_loss_bwd", dev.type == "cuda"):
-        rc = lib.tcsfm_pair_loss_bwd(batch.arr, g, b, h, w, w_l1, w_ssim, flags, batch.stream())
-    _cabi.check(lib, rc)
-    _timing.count_launch()
+    _call(lib, lib.tcsfm_pair_loss_bwd, "pair_loss_bwd", dev.type == "cuda",
+          batch.arr, g, b, h, w, w_l1, w_ssim, flags, batch.stream())
     return g_td, g_rd, g_proj
 
 
@@ -284,10 +269,8 @@ def pose_proj_fwd(lib, pose, K, sign, flags=0):
     pose, K = _f32c(pose, "pose"), _f32c(K, "K")
     n = pose.shape[0]
     proj = torch.empty((n, 3, 4), dtype=torch.float32, device=pose.device)
-    with _timing.launch("pose_proj_fwd", pose.is_cuda):
-        rc = lib.tcsfm_pose_proj_fwd(_ptr(pose), sign, _ptr(K), K.shape[0], _ptr(proj), n, flags, _stream(pose))
-    _cabi.check(lib, rc)
-    _timing.count_launch()
+    _call(lib, lib.tcsfm_pose_proj_fwd, "pose_proj_fwd", pose.is_cuda,
+          _ptr(pose), sign, _ptr(K), K.shape[0], _ptr(proj), n, flags, _stream(pose))
     return proj
 
 
@@ -295,55 +278,37 @@ def pose_proj_bwd(lib, pose, K, sign, g_proj):
     pose, K, g_proj = _f32c(pose, "pose"), _f32c(K, "K"), _f32c(g_proj, "g_proj")
     n = pose.shape[0]
     g_pose = torch.empty((n, 6), dtype=torch.float32, device=pose.device)
-    with _timing.launch("pose_proj_bwd", pose.is_cuda):
-        rc = lib.tcsfm_pose_proj_bwd(_ptr(pose), sign, _ptr(K), K.shape[0], _ptr(g_proj), _ptr(g_pose), n, _stream(pose))
-    _cabi.check(lib, rc)
-    _timing.count_launch()
+    _call(lib, lib.tcsfm_pose_proj_bwd, "pose_proj_bwd", pose.is_cuda,
+          _ptr(pose), sign, _ptr(K), K.shape[0], _ptr(g_proj), _ptr(g_pose), n, _stream(pose))
     return g_pose
 
 
-def min_reduce(lib, first, stride, count, n):
-    """sum_i min_j first.flatten()[j*stride + i]; `first` is the first competing map."""
-    out = torch.empty((1,), dtype=torch.float32, device=first.device)
-    with _timing.launch("min_reduce", first.is_cuda):
-        rc = lib.tcsfm_min_reduce(_ptr(first), stride, count, n, _ptr(out), _stream(first))
-    _cabi.check(lib, rc)
-    _timing.count_launch()
+def min_reduce(lib, first, stride, count, n, sums=None, cfg=None):
+    """sum_i min_j first.flatten()[j*stride + i] as [1]; `first` is the first competing map.  With `sums` [G,4] and
+    `cfg` the launch also finalises the frame: the return value gains (terms [3], total [1]) like frame_finalize."""
+    dev = first.device
+    out = torch.empty((1,), dtype=torch.float32, device=dev)
+    ticket = terms = total = None
+    if cfg is not None:
+        ticket = torch.empty((1,), dtype=torch.int32, device=dev)
+        terms = torch.empty((3,), dtype=torch.float32, device=dev)
+        total = torch.empty((1,), dtype=torch.float32, device=dev)
+    _call(lib, lib.tcsfm_min_reduce, "min_reduce", first.is_cuda,
+          _ptr(first), stride, count, n, _ptr(out), _ptr(ticket), _ptr(sums) if cfg is not None else None,
+          C.byref(cfg) if cfg is not None else None, _ptr(terms), _ptr(total), _stream(first))
+    if cfg is not None:
+        return out, terms, total
     return out
 
 
 TIE_BAND = 2e-4     # |second smallest - smallest| below which the per-pixel min is re-decided with the exact arithmetic
 
 
-def min_reduce_ties(lib, first, stride, count, n):
-    """min_reduce plus the list of near-tie pixels: returns (sum [1], tie_list int32 [cap], tie_count int32 [1])."""
-    out = torch.empty((1,), dtype=torch.float32, device=first.device)
-    cap = max(1024, n // 16)
-    tie_list = torch.empty((cap,), dtype=torch.int32, device=first.device)
-    tie_count = torch.empty((1,), dtype=torch.int32, device=first.device)
-    with _timing.launch("min_reduce", first.is_cuda):
-        rc = lib.tcsfm_min_reduce_ties(_ptr(first), stride, count, n, _ptr(out), TIE_BAND, _ptr(tie_list), _ptr(tie_count), cap,
-                                       _stream(first))
-    _cabi.check(lib, rc)
-    _timing.count_launch()
-    return out, tie_list, tie_count
-
-
-def pair_tie_resolve(lib, batch, group_ids, w_l1, w_ssim, flags, tie_list, tie_count):
-    """Overwrites diff_img of the listed competing groups at the near-tie pixels with the exact arithmetic's value."""
-    sub = (PairGroup * len(group_ids))(*[batch.arr[i] for i in group_ids])
-    with _timing.launch("pair_tie_resolve", batch.device.type == "cuda"):
-        rc = lib.tcsfm_pair_tie_resolve(sub, len(group_ids), batch.b, batch.h, batch.w, w_l1, w_ssim, flags,
-                                        _ptr(tie_list), _ptr(tie_count), tie_list.numel(), batch.stream())
-    _cabi.check(lib, rc)
-    _timing.count_launch()
-
-
 def pair_min_resolve(lib, batch, group_ids, w_l1, w_ssim, flags, sums=None, cfg=None):
-    """min_reduce_ties + pair_tie_resolve as one launch: returns (sum [1] of the per-pixel min over the listed groups'
-    diff_img, tie_count int32 [1]); the groups' diff_img entries at the near-tie pixels now hold the exact
-    arithmetic's values.  With `sums` [G,4] and `cfg` the launch also finalises the frame: the return value gains
-    (terms [3], total [1]) like frame_finalize."""
+    """Per-pixel min over the listed groups' diff_img with its near-ties re-decided, one launch: returns (sum [1] of that
+    min, tie_count int32 [1]); the groups' diff_img entries at the near-tie pixels now hold the exact arithmetic's
+    values.  With `sums` [G,4] and `cfg` the launch also finalises the frame: the return value gains (terms [3],
+    total [1]) like frame_finalize."""
     sub = (PairGroup * len(group_ids))(*[batch.arr[i] for i in group_ids])
     dev = batch.device
     out = torch.empty((1,), dtype=torch.float32, device=dev)
@@ -352,30 +317,13 @@ def pair_min_resolve(lib, batch, group_ids, w_l1, w_ssim, flags, sums=None, cfg=
     if cfg is not None:
         terms = torch.empty((3,), dtype=torch.float32, device=dev)
         total = torch.empty((1,), dtype=torch.float32, device=dev)
-    with _timing.launch("pair_min_resolve", dev.type == "cuda"):
-        rc = lib.tcsfm_pair_min_resolve(sub, len(group_ids), batch.b, batch.h, batch.w, w_l1, w_ssim, flags, TIE_BAND,
-                                        _ptr(out), _ptr(counters), _ptr(sums) if cfg is not None else None,
-                                        C.byref(cfg) if cfg is not None else None, _ptr(terms), _ptr(total), batch.stream())
-    _cabi.check(lib, rc)
-    _timing.count_launch()
+    _call(lib, lib.tcsfm_pair_min_resolve, "pair_min_resolve", dev.type == "cuda",
+          sub, len(group_ids), batch.b, batch.h, batch.w, w_l1, w_ssim, flags, TIE_BAND,
+          _ptr(out), _ptr(counters), _ptr(sums) if cfg is not None else None,
+          C.byref(cfg) if cfg is not None else None, _ptr(terms), _ptr(total), batch.stream())
     if cfg is not None:
         return out, counters[0:1], terms, total
     return out, counters[0:1]
-
-
-def min_reduce_finalize(lib, first, stride, count, n, sums, cfg):
-    """min_reduce + frame_finalize as one launch: (terms [3], total [1])."""
-    dev = first.device
-    out = torch.empty((1,), dtype=torch.float32, device=dev)
-    ticket = torch.empty((1,), dtype=torch.int32, device=dev)
-    terms = torch.empty((3,), dtype=torch.float32, device=dev)
-    total = torch.empty((1,), dtype=torch.float32, device=dev)
-    with _timing.launch("min_reduce", first.is_cuda):
-        rc = lib.tcsfm_min_reduce_finalize(_ptr(first), stride, count, n, _ptr(out), _ptr(ticket), _ptr(sums), C.byref(cfg),
-                                           _ptr(terms), _ptr(total), _stream(first))
-    _cabi.check(lib, rc)
-    _timing.count_launch()
-    return terms, total
 
 
 def make_frame_cfg(roles, w_inverse, w_depth, n_min_pixels):
@@ -391,10 +339,8 @@ def frame_finalize(lib, sums, min_sum, cfg):
     """-> terms [3] = (l_reconstruct_inverse, l_reconstruct_forward, l_depth), total [1] = their sum."""
     out = torch.empty((3,), dtype=torch.float32, device=sums.device)
     total = torch.empty((1,), dtype=torch.float32, device=sums.device)
-    with _timing.launch("frame_finalize", sums.is_cuda):
-        rc = lib.tcsfm_frame_finalize(_ptr(sums), _ptr(min_sum), C.byref(cfg), _ptr(out), _ptr(total), _stream(sums))
-    _cabi.check(lib, rc)
-    _timing.count_launch()
+    _call(lib, lib.tcsfm_frame_finalize, "frame_finalize", sums.is_cuda,
+          _ptr(sums), _ptr(min_sum), C.byref(cfg), _ptr(out), _ptr(total), _stream(sums))
     return out, total
 
 
@@ -406,16 +352,12 @@ def frame_bwd_prepare(lib, g_terms, g_total, cfg, zero=None):
     g_total = None if g_total is None else _f32c(g_total, "g_total")
     g_scalars = torch.empty((cfg.n_groups, 2), dtype=torch.float32, device=ref.device)
     g_min = torch.empty((1,), dtype=torch.float32, device=ref.device)
-    with _timing.launch("frame_bwd_prepare", ref.is_cuda):
-        if zero is not None and zero.numel() % 4 == 0 and zero.data_ptr() % 16 == 0 and zero.is_contiguous():
-            rc = lib.tcsfm_frame_bwd_prepare_zero(_ptr(g_terms), _ptr(g_total), C.byref(cfg), _ptr(g_scalars), _ptr(g_min),
-                                                  _ptr(zero), zero.numel(), _stream(ref))
-        else:
-            if zero is not None:
-                zero.zero_()
-            rc = lib.tcsfm_frame_bwd_prepare(_ptr(g_terms), _ptr(g_total), C.byref(cfg), _ptr(g_scalars), _ptr(g_min), _stream(ref))
-    _cabi.check(lib, rc)
-    _timing.count_launch()
+    if zero is not None and not (zero.numel() % 4 == 0 and zero.data_ptr() % 16 == 0 and zero.is_contiguous()):
+        zero.zero_()            # the launch fills 16-byte aligned float4s only
+        zero = None
+    _call(lib, lib.tcsfm_frame_bwd_prepare, "frame_bwd_prepare", ref.is_cuda,
+          _ptr(g_terms), _ptr(g_total), C.byref(cfg), _ptr(g_scalars), _ptr(g_min),
+          _ptr(zero), zero.numel() if zero is not None else 0, _stream(ref))
     return g_scalars, g_min
 
 
@@ -442,10 +384,8 @@ def pair_loss_bwd_shared(lib, batch, mask, sums, coef, g_scalars, g_min, min_inf
             a.g_min = _ptr(g_min)
         else:
             a.min_base, a.g_min = None, None
-    with _timing.launch("pair_loss_bwd", dev.type == "cuda"):
-        rc = lib.tcsfm_pair_loss_bwd(batch.arr, g, b, h, w, w_l1, w_ssim, flags | _cabi.SHARED_GRADS, batch.stream())
-    _cabi.check(lib, rc)
-    _timing.count_launch()
+    _call(lib, lib.tcsfm_pair_loss_bwd, "pair_loss_bwd", dev.type == "cuda",
+          batch.arr, g, b, h, w, w_l1, w_ssim, flags | _cabi.SHARED_GRADS, batch.stream())
     return g_proj
 
 
@@ -469,12 +409,10 @@ def photo_fwd(lib, tgt, src, rec, proj_depth, comp_depth, w_l1, w_ssim, flags=0,
     dev = rec.device
     outs = [torch.empty((n, 1, h, w), dtype=torch.float32, device=dev) for _ in range(4)]
     coef = torch.empty((n, lib.tcsfm_photo_coef_planes(), h, w), dtype=torch.float32, device=dev) if want_grad else None
-    with _timing.launch("photo_fwd", rec.is_cuda):
-        rc = lib.tcsfm_photo_fwd(_ptr(tgt), tsb, tsc, _ptr(src), ssb, ssc, _ptr(rec), _ptr(pd), _ptr(cd),
-                                 _ptr(outs[0]), _ptr(outs[1]), _ptr(outs[2]), _ptr(outs[3]), _ptr(coef), _ptr(valid),
-                                 n, h, w, w_l1, w_ssim, flags, _stream(rec))
-    _cabi.check(lib, rc)
-    _timing.count_launch()
+    _call(lib, lib.tcsfm_photo_fwd, "photo_fwd", rec.is_cuda,
+          _ptr(tgt), tsb, tsc, _ptr(src), ssb, ssc, _ptr(rec), _ptr(pd), _ptr(cd),
+          _ptr(outs[0]), _ptr(outs[1]), _ptr(outs[2]), _ptr(outs[3]), _ptr(coef), _ptr(valid),
+          n, h, w, w_l1, w_ssim, flags, _stream(rec))
     return outs[0], outs[1], outs[2], outs[3], coef
 
 
@@ -487,11 +425,9 @@ def photo_bwd(lib, tgt, rec, proj_depth, comp_depth, coef, g_diff, g_weight, w_l
     g_rec = torch.empty((n, 3, h, w), dtype=torch.float32, device=dev)
     g_pd = torch.empty((n, 1, h, w), dtype=torch.float32, device=dev)
     g_cd = torch.empty((n, 1, h, w), dtype=torch.float32, device=dev)
-    with _timing.launch("photo_bwd", rec.is_cuda):
-        rc = lib.tcsfm_photo_bwd(_ptr(tgt), tsb, tsc, _ptr(rec), _ptr(pd), _ptr(cd), _ptr(coef), _ptr(g_diff), _ptr(g_weight),
-                                 _ptr(g_rec), _ptr(g_pd), _ptr(g_cd), n, h, w, w_l1, w_ssim, flags, _stream(rec))
-    _cabi.check(lib, rc)
-    _timing.count_launch()
+    _call(lib, lib.tcsfm_photo_bwd, "photo_bwd", rec.is_cuda,
+          _ptr(tgt), tsb, tsc, _ptr(rec), _ptr(pd), _ptr(cd), _ptr(coef), _ptr(g_diff), _ptr(g_weight),
+          _ptr(g_rec), _ptr(g_pd), _ptr(g_cd), n, h, w, w_l1, w_ssim, flags, _stream(rec))
     return g_rec, g_pd, g_cd
 
 
@@ -512,19 +448,16 @@ def disp_to_depth_fwd(lib, disps, min_disp, disp_range, out_hw=None):
         raise ValueError("disp_to_depth_fwd: the maps of one launch must share a shape")
     if out_hw is None or tuple(out_hw) == (h, w):
         depths = [torch.empty_like(d) for d in disps]
-        with _timing.launch("disp_to_depth_fwd", disps[0].is_cuda):
-            rc = lib.tcsfm_disp_to_depth_fwd(_ptr_table(disps), _ptr_table(depths), len(disps), disps[0].numel(),
-                                             min_disp, disp_range, _stream(disps[0]))
+        _call(lib, lib.tcsfm_disp_to_depth_fwd, "disp_to_depth_fwd", disps[0].is_cuda,
+              _ptr_table(disps), _ptr_table(depths), len(disps), disps[0].numel(), min_disp, disp_range, _stream(disps[0]))
     else:
         if disps[0].dim() != 4 or disps[0].shape[1] != 1:
             raise ValueError("disp_to_depth_fwd: upsampling expects [B,1,h,w] maps")
         big_h, big_w = int(out_hw[0]), int(out_hw[1])
         depths = [torch.empty((b, 1, big_h, big_w), dtype=torch.float32, device=d.device) for d in disps]
-        with _timing.launch("disp_to_depth_fwd", disps[0].is_cuda):
-            rc = lib.tcsfm_disp_upsample_to_depth_fwd(_ptr_table(disps), _ptr_table(depths), len(disps), b, h, w, big_h, big_w,
-                                                      min_disp, disp_range, _stream(disps[0]))
-    _cabi.check(lib, rc)
-    _timing.count_launch()
+        _call(lib, lib.tcsfm_disp_upsample_to_depth_fwd, "disp_to_depth_fwd", disps[0].is_cuda,
+              _ptr_table(disps), _ptr_table(depths), len(disps), b, h, w, big_h, big_w, min_disp, disp_range,
+              _stream(disps[0]))
     return depths
 
 
@@ -535,17 +468,15 @@ def disp_to_depth_bwd(lib, g_depths, depths, disp_range, disp_hw=None):
     b, big_h, big_w = depths[0].shape[0], depths[0].shape[-2], depths[0].shape[-1]
     if disp_hw is None or tuple(disp_hw) == (big_h, big_w):
         g_disps = [torch.empty_like(d) for d in depths]
-        with _timing.launch("disp_to_depth_bwd", depths[0].is_cuda):
-            rc = lib.tcsfm_disp_to_depth_bwd(_ptr_table(g_depths), _ptr_table(depths), _ptr_table(g_disps), len(depths),
-                                             depths[0].numel(), disp_range, _stream(depths[0]))
+        _call(lib, lib.tcsfm_disp_to_depth_bwd, "disp_to_depth_bwd", depths[0].is_cuda,
+              _ptr_table(g_depths), _ptr_table(depths), _ptr_table(g_disps), len(depths), depths[0].numel(), disp_range,
+              _stream(depths[0]))
     else:
         h, w = int(disp_hw[0]), int(disp_hw[1])
         g_disps = [torch.empty((b, 1, h, w), dtype=torch.float32, device=d.device) for d in depths]
-        with _timing.launch("disp_to_depth_bwd", depths[0].is_cuda):
-            rc = lib.tcsfm_disp_upsample_to_depth_bwd(_ptr_table(g_depths), _ptr_table(depths), _ptr_table(g_disps), len(depths),
-                                                      b, h, w, big_h, big_w, disp_range, _stream(depths[0]))
-    _cabi.check(lib, rc)
-    _timing.count_launch()
+        _call(lib, lib.tcsfm_disp_upsample_to_depth_bwd, "disp_to_depth_bwd", depths[0].is_cuda,
+              _ptr_table(g_depths), _ptr_table(depths), _ptr_table(g_disps), len(depths), b, h, w, big_h, big_w, disp_range,
+              _stream(depths[0]))
     return g_disps
 
 
@@ -576,12 +507,9 @@ def frame_prologue(lib, disps, min_disp, disp_range, poses, pose_stride, K, sign
     depths = [torch.empty_like(d) for d in disps]
     proj = torch.empty((len(poses) * b, 3, 4), dtype=torch.float32, device=K.device)
     kinv = torch.empty((b, 3, 3), dtype=torch.float32, device=K.device) if want_kinv else None
-    with _timing.launch("frame_prologue", K.is_cuda):
-        rc = lib.tcsfm_frame_prologue(_ptr_table(disps), _ptr_table(depths), len(disps), disps[0].numel(), min_disp, disp_range,
-                                      _ptr_table(poses), len(poses), pose_stride, sign, _ptr(K), b, _ptr(proj), _ptr(kinv), flags,
-                                      _stream(K))
-    _cabi.check(lib, rc)
-    _timing.count_launch()
+    _call(lib, lib.tcsfm_frame_prologue, "frame_prologue", K.is_cuda,
+          _ptr_table(disps), _ptr_table(depths), len(disps), disps[0].numel(), min_disp, disp_range,
+          _ptr_table(poses), len(poses), pose_stride, sign, _ptr(K), b, _ptr(proj), _ptr(kinv), flags, _stream(K))
     return depths, proj, kinv
 
 
@@ -595,12 +523,9 @@ def frame_epilogue(lib, g_depths, depths, disp_range, poses, pose_stride, K, sig
         raise ValueError("frame_epilogue: poses / gradients disagree with the forward's shapes")
     g_disps = [torch.empty_like(d) for d in depths]
     g_pose = torch.empty((len(poses) * b, 6), dtype=torch.float32, device=K.device)
-    with _timing.launch("frame_epilogue", K.is_cuda):
-        rc = lib.tcsfm_frame_epilogue(_ptr_table(g_depths), _ptr_table(depths), _ptr_table(g_disps), len(depths), depths[0].numel(),
-                                      disp_range, _ptr_table(poses), len(poses), pose_stride, sign, _ptr(K), b, _ptr(g_proj),
-                                      _ptr(g_pose), _stream(K))
-    _cabi.check(lib, rc)
-    _timing.count_launch()
+    _call(lib, lib.tcsfm_frame_epilogue, "frame_epilogue", K.is_cuda,
+          _ptr_table(g_depths), _ptr_table(depths), _ptr_table(g_disps), len(depths), depths[0].numel(), disp_range,
+          _ptr_table(poses), len(poses), pose_stride, sign, _ptr(K), b, _ptr(g_proj), _ptr(g_pose), _stream(K))
     return g_disps, g_pose
 
 
@@ -610,10 +535,8 @@ def smooth_fwd(lib, disp, img):
     b, _, h, w = disp.shape
     ws = torch.empty((2 * b + 2,), dtype=torch.float32, device=disp.device)
     out = torch.empty((), dtype=torch.float32, device=disp.device)
-    with _timing.launch("smooth_fwd", disp.is_cuda):
-        rc = lib.tcsfm_smooth_fwd(_ptr(disp), _ptr(img), sb, sc, _ptr(ws), _ptr(out), b, h, w, _stream(disp))
-    _cabi.check(lib, rc)
-    _timing.count_launch(3)
+    _call(lib, lib.tcsfm_smooth_fwd, "smooth_fwd", disp.is_cuda,
+          _ptr(disp), _ptr(img), sb, sc, _ptr(ws), _ptr(out), b, h, w, _stream(disp), launches=3)
     return out, ws
 
 
@@ -622,10 +545,8 @@ def smooth_bwd(lib, disp, img, ws, g_out):
     img, sb, sc = image_view(img, "img")
     b, _, h, w = disp.shape
     g_disp = torch.empty_like(disp)
-    with _timing.launch("smooth_bwd", disp.is_cuda):
-        rc = lib.tcsfm_smooth_bwd(_ptr(disp), _ptr(img), sb, sc, _ptr(ws), _ptr(g_out), _ptr(g_disp), b, h, w, _stream(disp))
-    _cabi.check(lib, rc)
-    _timing.count_launch(2)
+    _call(lib, lib.tcsfm_smooth_bwd, "smooth_bwd", disp.is_cuda,
+          _ptr(disp), _ptr(img), sb, sc, _ptr(ws), _ptr(g_out), _ptr(g_disp), b, h, w, _stream(disp), launches=2)
     return g_disp
 
 
@@ -653,11 +574,8 @@ def pft_reduce_fwd(lib, diff, valid, auto_err, auto_mask, weight, bsz, n_src, fl
     dev = diff.device
     sums = torch.empty((8,), dtype=torch.float32, device=dev)
     loss = torch.empty((1,), dtype=torch.float32, device=dev)
-    with _timing.launch("pft_reduce_fwd", diff.is_cuda):
-        rc = lib.tcsfm_pft_reduce_fwd(d_f, v_f, a_f, w_f, d_i, v_i, m_i, w_i, bsz, n_src, n, flags, w_depth,
-                                      _ptr(sums), _ptr(loss), _stream(diff))
-    _cabi.check(lib, rc)
-    _timing.count_launch()
+    _call(lib, lib.tcsfm_pft_reduce_fwd, "pft_reduce_fwd", diff.is_cuda,
+          d_f, v_f, a_f, w_f, d_i, v_i, m_i, w_i, bsz, n_src, n, flags, w_depth, _ptr(sums), _ptr(loss), _stream(diff))
     return loss, sums, [k[0] for k in keep]
 
 
@@ -669,12 +587,9 @@ def pft_reduce_bwd(lib, maps, sums, g_loss, bsz, n_src, flags, w_depth):
     half = split * n * 4
     g_loss = _f32c(g_loss, "g_loss")
     g_diff, g_weight = torch.empty_like(diff), torch.empty_like(weight)
-    with _timing.launch("pft_reduce_bwd", diff.is_cuda):
-        rc = lib.tcsfm_pft_reduce_bwd(diff.data_ptr(), valid.data_ptr(), auto_err.data_ptr(), weight.data_ptr(),
-                                      diff.data_ptr() + half, valid.data_ptr() + half, auto_mask.data_ptr() + half,
-                                      weight.data_ptr() + half, bsz, n_src, n, flags, w_depth, _ptr(sums), _ptr(g_loss),
-                                      g_diff.data_ptr(), g_weight.data_ptr(), g_diff.data_ptr() + half,
-                                      g_weight.data_ptr() + half, _stream(diff))
-    _cabi.check(lib, rc)
-    _timing.count_launch()
+    _call(lib, lib.tcsfm_pft_reduce_bwd, "pft_reduce_bwd", diff.is_cuda,
+          diff.data_ptr(), valid.data_ptr(), auto_err.data_ptr(), weight.data_ptr(),
+          diff.data_ptr() + half, valid.data_ptr() + half, auto_mask.data_ptr() + half, weight.data_ptr() + half,
+          bsz, n_src, n, flags, w_depth, _ptr(sums), _ptr(g_loss),
+          g_diff.data_ptr(), g_weight.data_ptr(), g_diff.data_ptr() + half, g_weight.data_ptr() + half, _stream(diff))
     return g_diff, g_weight

@@ -413,48 +413,6 @@ min_reduce_kernel(const float* __restrict__ base, int64_t stride, int count, int
     finalize_by_last_block(fin, out);
 }
 
-// The same sum, plus the list of pixels whose two smallest candidates are closer than `band` (or involve a NaN): the
-// near-ties of the per-pixel min (losses.py:129-132) that the "fast" pair arithmetic re-evaluates exactly
-// (tcsfm_pair_tie_resolve) so that the arg-min routing of the backward stays the reference's.
-constexpr int kTieBuf = 1024;       // near-ties a block collects in shared memory before it reserves list space
-
-__global__ void __launch_bounds__(kReduceThreads)
-min_reduce_ties_kernel(const float* __restrict__ base, int64_t stride, int count, int64_t n, float* __restrict__ out,
-                       float band, int* __restrict__ tie_list, int* __restrict__ tie_count, int capacity) {
-    TCSFM_SHARED float red[kReduceThreads / 32];
-    TCSFM_SHARED int buf[kTieBuf];
-    TCSFM_SHARED int n_buf, list_at;
-    if (threadIdx.x == 0) n_buf = 0;
-    __syncthreads();
-    float part[1] = {0.f};
-    for (int64_t i = (int64_t)blockIdx.x * kReduceThreads + threadIdx.x; i < n; i += (int64_t)gridDim.x * kReduceThreads) {
-        float m = __ldg(base + i), second = INFINITY;
-        bool odd = m != m;
-        for (int j = 1; j < count; ++j) {
-            const float v = __ldg(base + j * stride + i);
-            odd = odd || v != v;
-            if (v < m) { second = m; m = v; }
-            else if (v < second) second = v;
-        }
-        part[0] += m;
-        if (count > 1 && (odd || !(second - m >= band))) {
-            const int at = atomicAdd(&n_buf, 1);                  // shared-memory counter: one global atomic per block below
-            if (at < kTieBuf) buf[at] = (int)i;
-            else {                                                // (a block with more than kTieBuf ties: straight to the list)
-                const int g_at = atomicAdd(tie_count, 1);
-                if (g_at < capacity) tie_list[g_at] = (int)i;
-            }
-        }
-    }
-    __syncthreads();
-    const int mine = n_buf < kTieBuf ? n_buf : kTieBuf;
-    if (threadIdx.x == 0) list_at = mine ? atomicAdd(tie_count, mine) : 0;
-    __syncthreads();
-    for (int k = threadIdx.x; k < mine; k += kReduceThreads)
-        if (list_at + k < capacity) tie_list[list_at + k] = buf[k];
-    block_atomic_accumulate<1>(part, red, out, threadIdx.x, kReduceThreads);
-}
-
 __global__ void frame_finalize_kernel(const float* __restrict__ sums, const float* __restrict__ min_sum, tcsfm_frame_cfg cfg,
                                       float* __restrict__ out, float* __restrict__ total) {
     if (threadIdx.x != 0 || blockIdx.x != 0) return;
@@ -498,21 +456,6 @@ extern "C" int tcsfm_u8_to_float(const unsigned char* src, float* dst, int64_t n
     if (blocks >= ((int64_t)1 << 31)) { set_error("tcsfm_u8_to_float: too many elements"); return 1; }
     TCSFM_LAUNCH(u8_to_float_kernel, dim3((unsigned)blocks), dim3(256), 0, stream, src, dst, n);
     return check_launch("tcsfm_u8_to_float");
-}
-
-extern "C" int tcsfm_min_reduce_ties(const float* base, int64_t stride, int count, int64_t n, float* out_sum, float band,
-                                     int* tie_list, int* tie_count, int capacity, void* stream) {
-    if (!base || !out_sum || !tie_list || !tie_count || count <= 0 || n <= 0 || capacity <= 0) {
-        set_error("tcsfm_min_reduce_ties: bad arguments"); return 1;
-    }
-    if (n >= ((int64_t)1 << 31)) { set_error("tcsfm_min_reduce_ties: more than 2^31 pixels"); return 1; }
-    cudaMemsetAsync(out_sum, 0, sizeof(float), (cudaStream_t)stream);
-    cudaMemsetAsync(tie_count, 0, sizeof(int), (cudaStream_t)stream);
-    const int64_t blocks = (n + kReduceThreads - 1) / kReduceThreads;
-    const int grid = (int)(blocks < 148 * 8 ? blocks : 148 * 8);
-    TCSFM_LAUNCH(min_reduce_ties_kernel, dim3(grid), dim3(kReduceThreads), 0, stream, base, stride, count, n, out_sum, band,
-                 tie_list, tie_count, capacity);
-    return check_launch("tcsfm_min_reduce_ties");
 }
 
 extern "C" int tcsfm_pose_proj_fwd(const float* pose, float sign, const float* K, int Bk, float* proj, int N, int flags,
@@ -594,31 +537,22 @@ extern "C" int tcsfm_disp_upsample_to_depth_bwd(const float* const* g_depth, con
     return check_launch("tcsfm_disp_upsample_to_depth_bwd");
 }
 
-extern "C" int tcsfm_min_reduce(const float* base, int64_t stride, int count, int64_t n, float* out_sum, void* stream) {
+extern "C" int tcsfm_min_reduce(const float* base, int64_t stride, int count, int64_t n, float* out_sum, int* ticket,
+                                const float* sums, const tcsfm_frame_cfg* cfg, float* out, float* total, void* stream) {
     if (!base || !out_sum || count <= 0 || n <= 0) { set_error("tcsfm_min_reduce: bad arguments"); return 1; }
+    if (cfg && (!ticket || !sums || !out || cfg->n_groups <= 0 || cfg->n_groups > 8)) { set_error("tcsfm_min_reduce: bad finalize arguments"); return 1; }
     cudaMemsetAsync(out_sum, 0, sizeof(float), (cudaStream_t)stream);
-    int64_t blocks = (n + kReduceThreads * 8 - 1) / (kReduceThreads * 8);
-    if (blocks > 148 * 8) blocks = 148 * 8;
-    if (blocks < 1) blocks = 1;
     FrameFinalize fin;
     memset(&fin, 0, sizeof(fin));
-    TCSFM_LAUNCH(min_reduce_kernel, dim3((unsigned)blocks), dim3(kReduceThreads), 0, stream, base, stride, count, n, out_sum, fin);
-    return check_launch("tcsfm_min_reduce");
-}
-
-extern "C" int tcsfm_min_reduce_finalize(const float* base, int64_t stride, int count, int64_t n, float* out_sum, int* ticket,
-                                         const float* sums, const tcsfm_frame_cfg* cfg, float* out, float* total, void* stream) {
-    if (!base || !out_sum || count <= 0 || n <= 0) { set_error("tcsfm_min_reduce_finalize: bad arguments"); return 1; }
-    if (!ticket || !sums || !cfg || !out || cfg->n_groups <= 0 || cfg->n_groups > 8) { set_error("tcsfm_min_reduce_finalize: bad finalize arguments"); return 1; }
-    cudaMemsetAsync(out_sum, 0, sizeof(float), (cudaStream_t)stream);
-    cudaMemsetAsync(ticket, 0, sizeof(int), (cudaStream_t)stream);
+    if (cfg) {
+        cudaMemsetAsync(ticket, 0, sizeof(int), (cudaStream_t)stream);
+        fin.sums = sums; fin.cfg = *cfg; fin.out = out; fin.total = total; fin.ticket = ticket;
+    }
     int64_t blocks = (n + kReduceThreads * 8 - 1) / (kReduceThreads * 8);
     if (blocks > 148 * 8) blocks = 148 * 8;
     if (blocks < 1) blocks = 1;
-    FrameFinalize fin;
-    fin.sums = sums; fin.cfg = *cfg; fin.out = out; fin.total = total; fin.ticket = ticket;
     TCSFM_LAUNCH(min_reduce_kernel, dim3((unsigned)blocks), dim3(kReduceThreads), 0, stream, base, stride, count, n, out_sum, fin);
-    return check_launch("tcsfm_min_reduce_finalize");
+    return check_launch("tcsfm_min_reduce");
 }
 
 extern "C" int tcsfm_frame_finalize(const float* sums, const float* min_sum, const tcsfm_frame_cfg* cfg, float* out, float* total,
@@ -629,22 +563,16 @@ extern "C" int tcsfm_frame_finalize(const float* sums, const float* min_sum, con
 }
 
 extern "C" int tcsfm_frame_bwd_prepare(const float* g_out, const float* g_total, const tcsfm_frame_cfg* cfg, float* g_scalars,
-                                       float* g_min, void* stream) {
+                                       float* g_min, float* zero, int64_t n_zero, void* stream) {
     if ((!g_out && !g_total) || !cfg || !g_scalars || !g_min || cfg->n_groups <= 0 || cfg->n_groups > 8) { set_error("tcsfm_frame_bwd_prepare: bad arguments"); return 1; }
-    TCSFM_LAUNCH(frame_bwd_prepare_kernel, dim3(1), dim3(256), 0, stream, g_out, g_total, *cfg, g_scalars, g_min, (float4*)nullptr, (int64_t)0);
-    return check_launch("tcsfm_frame_bwd_prepare");
-}
-
-extern "C" int tcsfm_frame_bwd_prepare_zero(const float* g_out, const float* g_total, const tcsfm_frame_cfg* cfg, float* g_scalars,
-                                            float* g_min, float* zero, int64_t n_zero, void* stream) {
-    if ((!g_out && !g_total) || !cfg || !g_scalars || !g_min || cfg->n_groups <= 0 || cfg->n_groups > 8) { set_error("tcsfm_frame_bwd_prepare_zero: bad arguments"); return 1; }
-    if (!zero || n_zero <= 0 || n_zero % 4 || ((uintptr_t)zero & 15)) { set_error("tcsfm_frame_bwd_prepare_zero: the buffer must be 16-byte aligned with a multiple of 4 elements"); return 1; }
-    const int64_t n4 = n_zero / 4;
+    if (zero && (n_zero <= 0 || n_zero % 4 || ((uintptr_t)zero & 15))) { set_error("tcsfm_frame_bwd_prepare: the buffer must be 16-byte aligned with a multiple of 4 elements"); return 1; }
+    const int64_t n4 = zero ? n_zero / 4 : 0;
     int64_t blocks = (n4 + 1023) / 1024;
     if (blocks > 148 * 8) blocks = 148 * 8;
+    if (blocks < 1) blocks = 1;
     TCSFM_LAUNCH(frame_bwd_prepare_kernel, dim3((unsigned)blocks), dim3(256), 0, stream, g_out, g_total, *cfg, g_scalars, g_min,
                  reinterpret_cast<float4*>(zero), n4);
-    return check_launch("tcsfm_frame_bwd_prepare_zero");
+    return check_launch("tcsfm_frame_bwd_prepare");
 }
 
 

@@ -723,10 +723,9 @@ pair_bwd_kernel(const __grid_constant__ PairLaunch L) {
 // ---------------------------------------------------------------------------
 // diff_img of single pixels exactly as pair_fwd_kernel computes it (every rounding step of eager PyTorch): the 3x3
 // window of (target, warped) per channel, avg_pool2d-ordered statistics, IEEE SSIM ratio, L1 blend, channel mean,
-// depth-consistency weight.  Sixteen lanes share one (listed pixel, competing group) task: lanes 0..8 warp one window
+// depth-consistency weight.  Sixteen lanes share one (near-tie pixel, competing group) task: lanes 0..8 warp one window
 // position each (one round of dependent gathers instead of nine), then every lane accumulates the window in
 // avg_pool2d's row-major order from the shuffled values and lane 0 overwrites the group's diff_img entry.
-constexpr int kTieTasksPerBlock = 8;
 
 // One (pixel, group) task on the 16 lanes [seg, seg + 16) of a warp; every lane of the warp must call it (full-mask
 // shuffles), dead tasks (live = false) compute on pixel 0 and write nothing.
@@ -781,20 +780,6 @@ __device__ __forceinline__ void resolve_tie(const PairLaunch& L, int j, int pix,
     }
     const float diff0 = mean3_of_sum<F>(esum, A);
     if (live && sub == 0) g.diff_img[pix] = need_depth ? __fmul_rn(diff0, __fsub_rn(1.0f, dd)) : diff0;
-}
-
-
-template <int F>
-__global__ void __launch_bounds__(16 * kTieTasksPerBlock)
-tie_resolve_kernel(const __grid_constant__ PairLaunch L, int n_groups, const int* __restrict__ tie_list,
-                   const int* __restrict__ tie_count, int capacity) {
-    const int n_tasks = min(__ldg(tie_count), capacity) * n_groups;
-    const int task0 = blockIdx.x * kTieTasksPerBlock;
-    if (task0 >= n_tasks) return;                          // the grid covers the list's capacity: most blocks are idle
-    const int sub = threadIdx.x & 15, task = task0 + (threadIdx.x >> 4);
-    const bool live = task < n_tasks;
-    const int e = live ? task / n_groups : 0, j = live ? task - e * n_groups : 0;
-    resolve_tie<F>(L, j, __ldg(tie_list + e), sub, live);
 }
 
 // Per-pixel min over the competing forward groups (losses.py:129-132) and the exact re-evaluation of its near-ties in
@@ -1017,27 +1002,9 @@ extern "C" int tcsfm_pair_loss_bwd(const tcsfm_pair_group* groups, int n_groups,
     return 0;
 }
 
-/* The competing forward groups' diff_img entries at the listed pixels (tcsfm_min_reduce_ties) are recomputed with the
- * exact arithmetic, whatever arithmetic produced the maps. */
-extern "C" int tcsfm_pair_tie_resolve(const tcsfm_pair_group* groups, int n_groups, int B, int H, int W,
-                                      float w_l1, float w_ssim, int flags, const int* tie_list, const int* tie_count,
-                                      int capacity, void* stream) {
-    if (!groups || n_groups <= 0 || n_groups > kMaxGroups) { set_error("tcsfm_pair_tie_resolve: 1..%d groups", kMaxGroups); return 1; }
-    if (!tie_list || !tie_count || capacity <= 0) { set_error("tcsfm_pair_tie_resolve: null tie list"); return 1; }
-    PairLaunch L;
-    memset(&L, 0, sizeof(L));
-    if (int rc = fill_launch(L, groups, n_groups, B, H, W, w_l1, w_ssim, flags & ~TCSFM_ARITH_FAST, "tcsfm_pair_tie_resolve", false)) return rc;
-    for (int i = 0; i < n_groups; ++i)
-        if (!L.g[i].diff_img) { set_error("tcsfm_pair_tie_resolve: group %d has no diff_img", i); return 1; }
-    const int64_t tasks = (int64_t)capacity * n_groups;
-    dim3 grid((unsigned)((tasks + kTieTasksPerBlock - 1) / kTieTasksPerBlock)), block(16 * kTieTasksPerBlock);
-    TCSFM_DISPATCH_FLAVOUR(flags, TCSFM_LAUNCH(tie_resolve_kernel<F>, grid, block, 0, stream, L, n_groups, tie_list, tie_count, capacity));
-    return check_launch("tcsfm_pair_tie_resolve");
-}
-
-/* tcsfm_min_reduce_ties + tcsfm_pair_tie_resolve (+ tcsfm_frame_finalize when `cfg` is given) as one launch (no tie list
- * in global memory): out_sum [1] = the sum over the B*H*W pixels of the min over the groups' diff_img, counters [2] =
- * (number of pixels re-evaluated, scratch ticket). */
+/* Per-pixel min over the groups' diff_img and the exact re-evaluation of its near-ties (+ tcsfm_frame_finalize when
+ * `cfg` is given) as one launch: out_sum [1] = the sum over the B*H*W pixels of that min, counters [2] = (number of
+ * pixels re-evaluated, scratch ticket). */
 extern "C" int tcsfm_pair_min_resolve(const tcsfm_pair_group* groups, int n_groups, int B, int H, int W,
                                       float w_l1, float w_ssim, int flags, float band, float* out_sum, int* counters,
                                       const float* sums, const tcsfm_frame_cfg* cfg, float* out_terms, float* out_total,

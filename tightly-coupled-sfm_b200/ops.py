@@ -333,7 +333,7 @@ class FrameLossFn(torch.autograd.Function):
                 _, LAST_TIE_COUNT, terms, total = _raw.pair_min_resolve(lib(), batch, fwd_idx, meta["w_l1"], meta["w_ssim"], flags,
                                                                         sums=sums, cfg=cfg)
             elif fwd_idx:
-                terms, total = _raw.min_reduce_finalize(lib(), diff[fwd_idx[0]], step * n_px, len(fwd_idx), n_px, sums, cfg)
+                _, terms, total = _raw.min_reduce(lib(), diff[fwd_idx[0]], step * n_px, len(fwd_idx), n_px, sums=sums, cfg=cfg)
             else:
                 terms, total = _raw.frame_finalize(lib(), sums, None, cfg)
         if want_grad:

@@ -84,7 +84,7 @@ for line in out.splitlines():
 with open("profiles/%s_sass_pair_kernels.txt" % tag, "w") as f:
     f.write("cuobjdump -sass libtcsfm_b200.so (sm_100a): instruction mnemonics per kernel (pair / warp kernels, flavour 0)\n\n")
     for fn, c in hist.items():
-        if ("pair_" in fn or "tie_resolve" in fn) and ("ILi0" in fn):
+        if "pair_" in fn and "ILi0" in fn:
             tot = sum(c.values())
             pick = ["UTMALDG", "SYNCS", "LDGSTS", "LDG", "STG", "LDS", "STS", "FFMA", "FFMA2", "FADD", "FADD2", "FMUL", "FMUL2", "MUFU", "RED", "REDG", "ATOMG", "SHFL", "BAR", "IMAD", "LDL", "STL"]
             f.write("%s\n  %d SASS instructions; %s\n\n" % (fn, tot, ", ".join("%s %d" % (k, c[k]) for k in pick if c[k])))
