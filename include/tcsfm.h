@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define TCSFM_ABI_VERSION 17
+#define TCSFM_ABI_VERSION 18
 
 /* ---- flags ------------------------------------------------------------------ */
 /* Arithmetic flavour.  Eager PyTorch rounds after every operator, but a few ATen
@@ -170,6 +170,24 @@ int tcsfm_photo_bwd(const float* tgt, int64_t tgt_sb, int64_t tgt_sc, const floa
                     const float* proj_depth, const float* comp_depth, const float* coef,
                     const float* g_diff, const float* g_weight, float* g_rec, float* g_pd, float* g_cd,
                     int N, int H, int W, float w_l1, float w_ssim, int flags, void* stream);
+
+/* ---- compute_photometric_error (optimization_experiments/helpers.py:8-23) for N pose hypotheses of ONE frame
+ *      pair, reduced to the loss-surface value of plot_loss_surface.py:11-87 -----------------------------------
+ * tgt / src are [1,3,H,W] views (channel strides given; a single pair has no batch stride), tgt_depth / src_depth
+ * [1,1,H,W] contiguous, kinv [9], proj [N,12] (hypothesis n's K @ [R|t], as tcsfm_pose_proj_fwd forms it).  For each
+ * n, with the warp of tcsfm_warp_fwd under proj[n] and the maps of tcsfm_photo_fwd (valid folded into the mask):
+ *   sums[n] = ( sum((diff * mask) * weight), sum(mask) )
+ * The per-pixel products carry the eager expression's roundings; the sums are added in a fixed order (the same
+ * inputs give the same bits on every call).  The optional maps rec [N,3,H,W] and diff / mask / weight [N,1,H,W]
+ * (NULL = not written) are those of a batch-1 compute_photometric_error call with the same `flags`.
+ * scratch [H,W] and partials [tcsfm_photo_sweep_partial_floats(N, H, W)]: workspace, overwritten.
+ * Three launches on `stream`. */
+int64_t tcsfm_photo_sweep_partial_floats(int N, int H, int W);
+int tcsfm_photo_sweep(const float* tgt, int64_t tgt_sc, const float* src, int64_t src_sc,
+                      const float* tgt_depth, const float* src_depth, const float* kinv, const float* proj,
+                      float* scratch, float* partials, float* sums,
+                      float* rec, float* diff, float* mask, float* weight,
+                      int N, int H, int W, float w_l1, float w_ssim, int flags, void* stream);
 
 /* ---- DepthOptimizer.compute_optimization_loss (optimization_experiments/optimizer.py:45-86): the
  *      reduction of the error maps of solve_pose_iteratively(return_errors=True) to the PFT loss --------

@@ -431,6 +431,38 @@ def photo_bwd(lib, tgt, rec, proj_depth, comp_depth, coef, g_diff, g_weight, w_l
     return g_rec, g_pd, g_cd
 
 
+def photo_sweep(lib, tgt, src, tgt_depth, src_depth, kinv, proj, w_l1, w_ssim, flags=0, want_maps=False):
+    """compute_photometric_error of ONE pair (tgt / src [1,3,H,W] views, depths [1,1,H,W], kinv [1,3,3]) under each of
+    the N projections proj [N,3,4], three launches.  Returns (sums [N,2] = (sum(diff * mask * weight), sum(mask)),
+    maps) with maps = (rec [N,3,H,W], diff, mask, weight [N,1,H,W]) when `want_maps`, else None."""
+    n = proj.shape[0]
+    h, w = tgt.shape[-2], tgt.shape[-1]
+    _expect(tgt, (1, 3, h, w), "tgt")
+    _expect(src, (1, 3, h, w), "src")
+    _expect(tgt_depth, (1, 1, h, w), "tgt_depth")
+    _expect(src_depth, (1, 1, h, w), "src_depth")
+    _expect(kinv, (1, 3, 3), "kinv")
+    _expect(proj, (n, 3, 4), "proj")
+    tgt, _, tsc = image_view(tgt, "tgt")
+    src, _, ssc = image_view(src, "src")
+    td, sd = _f32c(tgt_depth, "tgt_depth"), _f32c(src_depth, "src_depth")
+    kinv, proj = _f32c(kinv, "kinv"), _f32c(proj, "proj")
+    dev = tgt.device
+    scratch = torch.empty((h, w), dtype=torch.float32, device=dev)
+    partials = torch.empty((lib.tcsfm_photo_sweep_partial_floats(n, h, w),), dtype=torch.float32, device=dev)
+    sums = torch.empty((n, 2), dtype=torch.float32, device=dev)
+    maps = None
+    if want_maps:
+        maps = (torch.empty((n, 3, h, w), dtype=torch.float32, device=dev),) + \
+            tuple(torch.empty((n, 1, h, w), dtype=torch.float32, device=dev) for _ in range(3))
+    rec, diff, mask, weight = maps if want_maps else (None,) * 4
+    _call(lib, lib.tcsfm_photo_sweep, "photo_sweep", tgt.is_cuda,
+          _ptr(tgt), tsc, _ptr(src), ssc, _ptr(td), _ptr(sd), _ptr(kinv), _ptr(proj),
+          _ptr(scratch), _ptr(partials), _ptr(sums), _ptr(rec), _ptr(diff), _ptr(mask), _ptr(weight),
+          n, h, w, w_l1, w_ssim, flags, _stream(tgt), launches=3)
+    return sums, maps
+
+
 def _ptr_table(tensors):
     arr = (C.c_void_p * len(tensors))()
     for i, t in enumerate(tensors):

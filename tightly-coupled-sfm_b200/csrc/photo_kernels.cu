@@ -255,6 +255,183 @@ photo_bwd_kernel(const __grid_constant__ PhotoArgs P) {
     }
 }
 
+// ---------------------------------------------------------------------------
+// compute_photometric_error for N pose hypotheses of ONE frame pair (the loss-surface sweeps of
+// plot_loss_surface.py:11-87): per hypothesis the warp of inverse_warp2, the maps above and the masked sums
+//   error_sum = sum((diff * auto_mask * valid) * weight)      valid_sum = sum(auto_mask * valid)
+// Three launches: the pose-independent auto-mask error once, one CTA per (hypothesis, tile), and a
+// fixed-order reduction of the per-CTA partials (no float atomics: the sums are deterministic).
+// ---------------------------------------------------------------------------
+struct SweepArgs {
+    PhotoArgs P;                          // tgt / src views, auto_err scratch [H,W], weights, SSIM constants, arithmetic
+    const float* tdep; const float* sdep; // [H,W]
+    const float* kinv; const float* proj; // [9], [N,12]
+    float* partials;                      // [tiles][N][2]: per-CTA (sum of products, sum of the mask)
+    float* rec; float* diff; float* mask; float* weight;   // optional maps [N,3,H,W], [N,1,H,W] x 3
+    int N, tiles;
+};
+
+// auto_err = mean_c(w_l1 * clamp|tgt - src| + w_ssim * SSIM(tgt, src)) of the pair: photo_fwd_kernel's e_src
+template <int F>
+__global__ void __launch_bounds__(kTileThreads)
+photo_auto_err_kernel(const __grid_constant__ PhotoArgs P) {
+    using T1 = Tile<1>;
+    TCSFM_DYN_SMEM(float2, ts);                                  // [3][cells] (target, src)
+    const int H = P.A.H, W = P.A.W;
+    const int tiles_x = (W + kTileW - 1) / kTileW;
+    const int tile_y = blockIdx.x / tiles_x, tile_x = blockIdx.x - tile_y * tiles_x;
+    const int x0 = tile_x * kTileW, y0 = tile_y * kTileH;
+    for (int cell = threadIdx.x; cell < T1::kCells; cell += kTileThreads) {
+        int ry = 0, rx = 0;
+        const bool ok = T1::cell_to_reflected(cell, x0, y0, H, W, ry, rx);
+        const int pix = ok ? ry * W + rx : 0;
+#pragma unroll
+        for (int ch = 0; ch < 3; ++ch)
+            ts[ch * T1::kCells + cell] = ok ? make_float2(__ldg(P.tgt + ch * P.tgt_sc + pix), __ldg(P.src + ch * P.src_sc + pix))
+                                            : make_float2(0.f, 0.f);
+    }
+    __syncthreads();
+    const int tx = threadIdx.x & (kTileW - 1);
+    const int ty0 = (threadIdx.x >> 6) * kPixPerThread;
+    const int gx = x0 + tx;
+    float e[kPixPerThread];
+#pragma unroll
+    for (int ch = 0; ch < 3; ++ch) strip_channel<false>(ts + ch * T1::kCells, tx, ty0, P, ch == 0, e, nullptr, gx, y0 + ty0, 0);
+#pragma unroll
+    for (int k = 0; k < kPixPerThread; ++k) {
+        const int gy = y0 + ty0 + k;
+        if (gx < W && gy < H) P.auto_err[gy * W + gx] = mean3_of_sum<F>(e[k], P.A);
+    }
+}
+
+// Fills one cell of the (target, warped source) tile with the image pixel (rx, ry) under the camera `cam`, exactly as
+// warp_fwd_kernel forms projected_img there; returns the warp and its taps.
+template <int F>
+__device__ __forceinline__ TapIdx sweep_fill_cell(const SweepArgs& S, const Cam& cam, int rx, int ry, float2* tw, int cell,
+                                                  WarpPt& p) {
+    const Arith& A = S.P.A;
+    const int pix = ry * A.W + rx;
+    warp_point<F>(cam, A, rx, ry, __ldg(S.tdep + pix), p);
+    const TapIdx ti = make_taps(p, A.H, A.W);
+#pragma unroll
+    for (int ch = 0; ch < 3; ++ch) {
+        const float w = blend(load_taps(S.P.src, (int)(ch * S.P.src_sc), ti, A.W), ti);
+        tw[ch * Tile<1>::kCells + cell] = make_float2(__ldg(S.P.tgt + (ch * S.P.tgt_sc + pix)), w);
+    }
+    return ti;
+}
+
+// The halo ring of a Tile<1>, enumerated 0 .. kSweepRingCells - 1 (top row, bottom row, left column, right column).
+constexpr int kSweepRingCells = 2 * (kTileW + 2) + 2 * kTileH;
+__device__ __forceinline__ void sweep_ring_cell(int r, int& cx, int& cy) {
+    if (r < kTileW + 2) { cx = r - 1; cy = -1; }
+    else if (r < 2 * (kTileW + 2)) { cx = r - (kTileW + 2) - 1; cy = kTileH; }
+    else if (r < 2 * (kTileW + 2) + kTileH) { cx = -1; cy = r - 2 * (kTileW + 2); }
+    else { cx = kTileW; cy = r - 2 * (kTileW + 2) - kTileH; }
+}
+
+template <int F>
+__global__ void __launch_bounds__(kTileThreads, 3)
+photo_sweep_kernel(const __grid_constant__ SweepArgs S) {
+    using T1 = Tile<1>;
+    TCSFM_DYN_SMEM(float2, tw);                                  // [3][cells] (target, warped source)
+    TCSFM_SHARED float red[2 * (kTileThreads / 32)];
+    const Arith& A = S.P.A;
+    const int H = A.H, W = A.W, n = H * W;
+    const int hyp = blockIdx.x / S.tiles, tile = blockIdx.x - hyp * S.tiles;
+    const int tiles_x = (W + kTileW - 1) / kTileW;
+    const int tile_y = tile / tiles_x, tile_x = tile - tile_y * tiles_x;
+    const int x0 = tile_x * kTileW, y0 = tile_y * kTileH;
+    const Cam cam = load_cam(S.kinv, S.proj + (int64_t)hyp * 12, 0);
+    const int tx = threadIdx.x & (kTileW - 1);
+    const int ty0 = (threadIdx.x >> 6) * kPixPerThread;
+    const int gx = x0 + tx;
+    // own pixels: the cell, plus valid and weight = 1 - depth_inconsistency(computed, projected depth) of the warp.
+    // Own cells that no consumer reads (partial tiles) are filled from a clamped pixel, as in the pair forward.
+    bool valid[kPixPerThread];
+    float wgt[kPixPerThread];
+#pragma unroll
+    for (int k = 0; k < kPixPerThread; ++k) {
+        const int gy = y0 + ty0 + k;
+        const int sx = min(max(gx < W ? gx : 2 * W - 2 - gx, 0), W - 1);
+        const int sy = min(max(gy < H ? gy : 2 * H - 2 - gy, 0), H - 1);
+        WarpPt p;
+        const TapIdx ti = sweep_fill_cell<F>(S, cam, sx, sy, tw, T1::cell(tx, ty0 + k), p);
+        valid[k] = p.valid;
+        wgt[k] = __fsub_rn(1.0f, depth_inconsistency(p.Z, blend(load_taps(S.sdep, 0, ti, W), ti)));
+    }
+    if (threadIdx.x < kSweepRingCells) {
+        int cx, cy, ry = 0, rx = 0;
+        sweep_ring_cell(threadIdx.x, cx, cy);
+        const int cell = T1::cell(cx, cy);
+        if (T1::cell_to_reflected(cell, x0, y0, H, W, ry, rx)) {
+            WarpPt p;
+            sweep_fill_cell<F>(S, cam, rx, ry, tw, cell, p);
+        } else {
+#pragma unroll
+            for (int ch = 0; ch < 3; ++ch) tw[ch * T1::kCells + cell] = make_float2(0.f, 0.f);
+        }
+    }
+    __syncthreads();
+    float esum[kPixPerThread];
+#pragma unroll
+    for (int ch = 0; ch < 3; ++ch) strip_channel<false>(tw + ch * T1::kCells, tx, ty0, S.P, ch == 0, esum, nullptr, gx, y0 + ty0, n);
+    float part_e = 0.f, part_m = 0.f;
+#pragma unroll
+    for (int k = 0; k < kPixPerThread; ++k) {
+        const int gy = y0 + ty0 + k;
+        if (gx < W && gy < H) {
+            const int pix = gy * W + gx;
+            const float diff = mean3_of_sum<F>(esum[k], A);
+            const float m = (diff < __ldg(S.P.auto_err + pix)) ? (valid[k] ? 1.f : 0.f) : 0.f;
+            // (diff_img * valid_mask) * weight_mask, each product rounded like the eager expression
+            part_e = __fadd_rn(part_e, __fmul_rn(__fmul_rn(diff, m), wgt[k]));
+            part_m = __fadd_rn(part_m, m);
+            const int64_t o = (int64_t)hyp * n + pix;
+            if (S.diff) S.diff[o] = diff;
+            if (S.mask) S.mask[o] = m;
+            if (S.weight) S.weight[o] = wgt[k];
+            if (S.rec) {
+#pragma unroll
+                for (int ch = 0; ch < 3; ++ch) S.rec[((int64_t)hyp * 3 + ch) * n + pix] = tw[ch * T1::kCells + T1::cell(tx, ty0 + k)].y;
+            }
+        }
+    }
+    // fixed-order block sum: butterfly within each warp, then the warps in index order
+    part_e = warp_sum(part_e);
+    part_m = warp_sum(part_m);
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    if (lane == 0) { red[warp] = part_e; red[kTileThreads / 32 + warp] = part_m; }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        float se = red[0], sm = red[kTileThreads / 32];
+        for (int w = 1; w < kTileThreads / 32; ++w) { se = __fadd_rn(se, red[w]); sm = __fadd_rn(sm, red[kTileThreads / 32 + w]); }
+        float* dst = S.partials + ((int64_t)tile * S.N + hyp) * 2;
+        dst[0] = se;
+        dst[1] = sm;
+    }
+}
+
+// sums[n] = (error_sum, valid_sum) of hypothesis n: its per-CTA partials added in tile order, the products in double
+// (one rounding to fp32 at the end), the mask counts in fp32 (exact: integers below 2^24).
+constexpr int kSweepFinishThreads = 128;
+__global__ void __launch_bounds__(kSweepFinishThreads)
+photo_sweep_finish_kernel(const float* __restrict__ partials, int tiles, int N, float* __restrict__ sums) {
+    const int hyp = blockIdx.x * kSweepFinishThreads + threadIdx.x;
+    if (hyp >= N) return;
+    double e = 0.0;
+    float m = 0.f;
+    for (int t = 0; t < tiles; ++t) {
+        const float* p = partials + ((int64_t)t * N + hyp) * 2;
+        e += (double)__ldg(p);
+        m = __fadd_rn(m, __ldg(p + 1));
+    }
+    sums[2 * hyp] = (float)e;
+    sums[2 * hyp + 1] = m;
+}
+
+static int sweep_tiles(int H, int W) { return ((W + kTileW - 1) / kTileW) * ((H + kTileH - 1) / kTileH); }
+
 static int fill_photo(PhotoArgs& P, int N, int H, int W, float w_l1, float w_ssim, int flags, const char* who) {
     if (N <= 0 || H < 2 || W < 2) { set_error("%s: bad shape N=%d H=%d W=%d", who, N, H, W); return 1; }
     if (N > 65535) { set_error("%s: N=%d exceeds 65535", who, N); return 1; }
@@ -308,4 +485,44 @@ extern "C" int tcsfm_photo_bwd(const float* tgt, int64_t tgt_sb, int64_t tgt_sc,
     dim3 grid(((W + kTileW - 1) / kTileW) * ((H + kTileH - 1) / kTileH), N), block(kTileThreads);
     TCSFM_LAUNCH(photo_bwd_kernel, grid, block, smem, stream, P);
     return check_launch("tcsfm_photo_bwd");
+}
+
+extern "C" int64_t tcsfm_photo_sweep_partial_floats(int N, int H, int W) {
+    if (N <= 0 || H <= 0 || W <= 0) return 0;
+    return 2 * (int64_t)N * sweep_tiles(H, W);
+}
+
+extern "C" int tcsfm_photo_sweep(const float* tgt, int64_t tgt_sc, const float* src, int64_t src_sc,
+                                 const float* tgt_depth, const float* src_depth, const float* kinv, const float* proj,
+                                 float* scratch, float* partials, float* sums,
+                                 float* rec, float* diff, float* mask, float* weight,
+                                 int N, int H, int W, float w_l1, float w_ssim, int flags, void* stream) {
+    const char* who = "tcsfm_photo_sweep";
+    if (N <= 0 || H < 2 || W < 2) { set_error("%s: bad shape N=%d H=%d W=%d", who, N, H, W); return 1; }
+    if (!tgt || !src || !tgt_depth || !src_depth || !kinv || !proj) { set_error("%s: null input pointer", who); return 1; }
+    if (!scratch || !partials || !sums) { set_error("%s: null scratch, partials or sums", who); return 1; }
+    const int tiles = sweep_tiles(H, W);
+    if ((int64_t)tiles * N > 0x7fffffff) { set_error("%s: N=%d hypotheses of %d tiles exceed the grid", who, N, tiles); return 1; }
+    // the kernels address a channel plane with 32-bit offsets
+    const int64_t n = (int64_t)H * W;
+    if (tgt_sc < 0 || src_sc < 0 || 2 * tgt_sc + n > 0x7fffffff || 2 * src_sc + n > 0x7fffffff) {
+        set_error("%s: channel strides %lld / %lld out of range", who, (long long)tgt_sc, (long long)src_sc); return 1;
+    }
+    SweepArgs S;
+    memset(&S, 0, sizeof(S));
+    S.P.tgt = tgt; S.P.tgt_sc = tgt_sc; S.P.src = src; S.P.src_sc = src_sc; S.P.auto_err = scratch;
+    S.P.A = make_arith(H, W, flags);
+    S.P.w_l1 = w_l1; S.P.w_ssim = w_ssim;
+    S.P.C1 = (float)(0.01 * 0.01); S.P.C2 = (float)(0.03 * 0.03);
+    S.tdep = tgt_depth; S.sdep = src_depth; S.kinv = kinv; S.proj = proj; S.partials = partials;
+    S.rec = rec; S.diff = diff; S.mask = mask; S.weight = weight;
+    S.N = N; S.tiles = tiles;
+    const size_t smem = 3 * Tile<1>::kCells * sizeof(float2);
+    TCSFM_DISPATCH_FLAVOUR(flags, TCSFM_LAUNCH(photo_auto_err_kernel<F>, dim3(tiles), dim3(kTileThreads), smem, stream, S.P));
+    if (int rc = check_launch(who)) return rc;
+    TCSFM_DISPATCH_FLAVOUR(flags, TCSFM_LAUNCH(photo_sweep_kernel<F>, dim3((unsigned)(tiles * N)), dim3(kTileThreads), smem, stream, S));
+    if (int rc = check_launch(who)) return rc;
+    TCSFM_LAUNCH(photo_sweep_finish_kernel, dim3((N + kSweepFinishThreads - 1) / kSweepFinishThreads), dim3(kSweepFinishThreads), 0,
+                 stream, partials, tiles, N, sums);
+    return check_launch(who);
 }

@@ -3,10 +3,12 @@
 optimizer.py:29-97) and ``compute_photometric_error`` (optimization_experiments/
 helpers.py:8-23).  The optimisation driver itself (deep copies of the depth net,
 Adam, plotting; optimizer.py:136-297) is the reference's harness and calls these.
+``photometric_loss_surface`` evaluates ``compute_photometric_error`` for N pose hypotheses of one pair in one call
+(the loss-surface plots, plot_loss_surface.py:11-87).
 """
 import torch
 
-from . import _cabi, ops
+from . import _cabi, _raw, ops, stn
 from .losses import get_smooth_loss
 from .stn import inverse_warp2
 
@@ -74,3 +76,40 @@ def compute_photometric_error(target_img, source_img, target_depth, source_depth
         target_img.detach(), source_img.detach(), img_rec, projected_depth, computed_depth, 0.15, 0.85, valid_mask)
     return {'diff_img': diff_img, 'img_rec': img_rec, 'valid_mask': masked,
             'weight_mask': weight_mask, 'poses': pose}
+
+
+def photometric_loss_surface(target_img, source_img, target_depth, source_depth, poses, intrinsics, return_maps=False):
+    """compute_photometric_error (helpers.py:8-23) of one frame pair under N pose hypotheses, reduced per hypothesis to
+    the loss-surface value sum(diff_img * valid_mask * weight_mask) / sum(valid_mask) of plot_loss_surface.py:11-87.
+
+    target_img / source_img [1,3,H,W] (may be channel slices), target_depth / source_depth [1,1,H,W], poses [N,6] or
+    [N,8] (columns 0:6, un-negated like `pose` of compute_photometric_error), intrinsics [1,3,3].  Returns
+    {'loss': [N], 'error_sum': [N], 'valid_sum': [N]}; with return_maps=True also 'diff_img', 'img_rec', 'valid_mask'
+    and 'weight_mask' stacked over the N hypotheses.  The maps are bit-identical to N batch-1 calls of
+    compute_photometric_error; the sums are added in a fixed order (deterministic), loss = error_sum / valid_sum
+    (NaN where no pixel is valid).  Six launches whatever N is: K^-1, K @ [R|t] of every hypothesis, the three of
+    tcsfm_photo_sweep and the division.  Forward only."""
+    ops._require_cuda(target_img, source_img, target_depth, source_depth, poses, intrinsics)
+    if torch.is_grad_enabled() and any(t.requires_grad for t in (target_img, source_img, target_depth, source_depth,
+                                                                     poses, intrinsics)):
+        raise NotImplementedError("photometric_loss_surface is forward only: no gradient of the surface is implemented")
+    if target_img.dim() != 4 or target_img.shape[0] != 1:
+        raise ValueError("photometric_loss_surface: one frame pair (batch 1) per call, got target_img %s"
+                         % list(target_img.shape))
+    if poses.dim() != 2 or poses.shape[0] < 1 or poses.shape[1] not in (6, 8):
+        raise ValueError("photometric_loss_surface: poses must be [N,6] or [N,8] with N >= 1, got %s" % list(poses.shape))
+    h, w = target_img.shape[2], target_img.shape[3]
+    kinv = stn.inverse_intrinsics(intrinsics)
+    with ops._guard(poses):
+        # every hypothesis as the batch-1 call of compute_photometric_error forms it: K @ [R|t] of -pose with the
+        # batch-1 rounding of the pose algebra, and the batch-1 warp arithmetic, whatever N is
+        if intrinsics.is_cuda:
+            proj = _raw.pose_proj_fwd(ops.lib(), poses[:, 0:6], intrinsics, -1.0, ops.pose_flags(1))
+        else:       # CPU tensors (test builds): the eager operators stn.projection_matrices takes there
+            proj = intrinsics @ stn.pose_vec2mat(-poses[:, 0:6])
+        sums, maps = _raw.photo_sweep(ops.lib(), target_img, source_img, target_depth, source_depth, kinv, proj,
+                                      0.15, 0.85, ops.arith_flags(1, h, w), want_maps=return_maps)
+    out = {'loss': sums[:, 0] / sums[:, 1], 'error_sum': sums[:, 0], 'valid_sum': sums[:, 1]}
+    if return_maps:
+        out['img_rec'], out['diff_img'], out['valid_mask'], out['weight_mask'] = maps
+    return out

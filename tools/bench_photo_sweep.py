@@ -1,0 +1,130 @@
+"""Loss-surface sweeps of the demo (plot_loss_surface.py:11-87) two ways on one GPU, printed as one JSON line:
+
+  loop   the batch-1 loop `bench.py --workload sweep` times: one pft.compute_photometric_error call and the masked
+         mean (diff_img * valid_mask * weight_mask).sum() / valid_mask.sum() per pose sample;
+  batch  one pft.photometric_loss_surface call over all samples.
+
+Input: what `bench.py --workload sweep` evaluates, make_frames(1, 192, 640, n_src=2, seed=0, KITTI intrinsics) with a
+line of forward-translation (pose column 2) and a line of yaw (column 4) samples, linspace(-0.05, 0.05, n) each:
+n = 100 (bench.py's default --sweep-evals, N = 200) and n = 50 (the demo's, N = 100).  Both are timed like
+main_sweep: wall clock of a whole sweep including the final device-to-host copy, after one warm-up sweep, the two
+alternated round by round.  The batched op's device time per call comes from CUDA events around `--device-iters`
+back-to-back calls.  The working set (one frame pair, ~2.5 MB) stays in L2, so no HBM roofline fraction is claimed.
+
+Usage: python tools/bench_photo_sweep.py [--rounds R] [--device-iters I]"""
+import argparse
+import json
+import os
+import statistics
+import subprocess
+import sys
+import time
+
+import torch
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+from tcsfm_b200 import pft, synth  # noqa: E402
+
+
+def card():
+    """(name, power limit) of the card, a read-only query."""
+    try:
+        out = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"],
+                             capture_output=True, text=True, timeout=60).stdout.strip().splitlines()
+        idx = torch.cuda.current_device()
+        name, power = [s.strip() for s in out[idx].split(",")]
+        return name, power
+    except (OSError, IndexError, ValueError, subprocess.SubprocessError):
+        return torch.cuda.get_device_name(), "unknown"
+
+
+def measure(fr, n, rounds, device_iters):
+    args = (fr["target"], fr["sources"][0], fr["depths"][0], fr["depths"][1])
+    deltas = torch.linspace(-0.05, 0.05, n)
+    deltas_dev = deltas.to(fr["K"].device)
+
+    def loop():                                     # bench.py main_sweep's loop body
+        vals = []
+        with torch.no_grad():
+            for axis in (2, 4):
+                for d in deltas:
+                    pose = fr["poses"][0].clone()
+                    pose[:, axis] += d
+                    r = pft.compute_photometric_error(*args, pose, fr["K"])
+                    vals.append((r["diff_img"] * r["valid_mask"] * r["weight_mask"]).sum() / r["valid_mask"].sum())
+        return torch.stack(vals)
+
+    def poses():
+        p = fr["poses"][0].repeat(2 * n, 1)
+        p[:n, 2] += deltas_dev
+        p[n:, 4] += deltas_dev
+        return p
+
+    def batch():
+        with torch.no_grad():
+            return pft.photometric_loss_surface(*args, poses(), fr["K"])["loss"]
+
+    def timed(fn):
+        torch.cuda.synchronize()
+        t0 = time.perf_counter()
+        host = fn().cpu()
+        return time.perf_counter() - t0, host
+
+    loop(), batch()                                 # warm-up sweeps
+    t_loop, t_batch = [], []
+    for _ in range(rounds):
+        dt, ref = timed(loop)
+        t_loop.append(dt)
+        dt, got = timed(batch)
+        t_batch.append(dt)
+    rel = ((got - ref).abs() / ref.abs()).max().item()
+
+    p = poses()
+    with torch.no_grad():
+        for _ in range(10):
+            pft.photometric_loss_surface(*args, p, fr["K"])
+        torch.cuda.synchronize()
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record()
+        for _ in range(device_iters):
+            pft.photometric_loss_surface(*args, p, fr["K"])
+        e1.record()
+        torch.cuda.synchronize()
+    ms_call = e0.elapsed_time(e1) / device_iters
+    evals = 2 * n
+    return {"N": evals,
+            "loop_evals_per_s": round(evals / statistics.median(t_loop), 1),
+            "batch_evals_per_s": round(evals / statistics.median(t_batch), 1),
+            "speedup": round(statistics.median(t_loop) / statistics.median(t_batch), 2),
+            "loop_ms_per_sweep": [round(t * 1e3, 3) for t in t_loop],
+            "batch_ms_per_sweep": [round(t * 1e3, 3) for t in t_batch],
+            "batch_device_ms_per_call": round(ms_call, 4),
+            "batch_device_us_per_eval": round(ms_call * 1e3 / evals, 3),
+            "device_calls_timed": device_iters,
+            "max_rel_diff_loss": rel}
+
+
+def main():
+    ap = argparse.ArgumentParser(description=__doc__.splitlines()[0])
+    ap.add_argument("--rounds", type=int, default=5, help="alternated loop / batch sweeps per configuration")
+    ap.add_argument("--device-iters", type=int, default=200, help="back-to-back calls timed with CUDA events")
+    args = ap.parse_args()
+    if not torch.cuda.is_available():
+        sys.exit("bench_photo_sweep.py needs a CUDA device")
+    dev = torch.device("cuda:0")
+    torch.cuda.set_device(dev)
+    fr = synth.make_frames(1, 192, 640, n_src=2, seed=0, device=dev, intrinsics=torch.tensor(synth.KITTI_K))
+    name, power = card()
+    line = {"metric": "loss-surface evaluations/s (B=1, 192x640, forward only): batch-1 loop vs one batched call",
+            "unit": "evals/s", "gpu": name, "power_limit": power, "dtype": "f32", "data": "synthetic",
+            "timing": "wall clock of a whole sweep incl. the final D2H, median of alternated rounds; device time from "
+                      "CUDA events",
+            "note": "working set (one frame pair, ~2.5 MB) is L2-resident: no HBM roofline fraction is claimed",
+            "configs": {"bench_sweep_default_100x2": measure(fr, 100, args.rounds, args.device_iters),
+                        "demo_50x2": measure(fr, 50, args.rounds, args.device_iters)}}
+    print(json.dumps(line))
+
+
+if __name__ == "__main__":
+    main()
