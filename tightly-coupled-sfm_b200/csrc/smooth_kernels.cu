@@ -43,9 +43,9 @@ smooth_fwd_kernel(const float* __restrict__ disp, const float* __restrict__ img,
     float part[2] = {0.f, 0.f};
     for (int p = blockIdx.x * kSmoothThreads + threadIdx.x; p < n; p += gridDim.x * kSmoothThreads) {
         const int y = p / W, x = p - y * W;
-        const float c = __ldg(d + p) * inv;
-        if (x + 1 < W) part[0] += fabsf(c - __ldg(d + p + 1) * inv) * edge_weight(im, img_sc, p, p + 1);
-        if (y + 1 < H) part[1] += fabsf(c - __ldg(d + p + W) * inv) * edge_weight(im, img_sc, p, p + W);
+        const float c = __fmul_rn(__ldg(d + p), inv);
+        if (x + 1 < W) part[0] += fabsf(c - __fmul_rn(__ldg(d + p + 1), inv)) * edge_weight(im, img_sc, p, p + 1);
+        if (y + 1 < H) part[1] += fabsf(c - __fmul_rn(__ldg(d + p + W), inv)) * edge_weight(im, img_sc, p, p + W);
     }
     block_atomic_accumulate<2>(part, red, acc, threadIdx.x, kSmoothThreads);
 }
@@ -68,12 +68,14 @@ smooth_bwd_kernel(const float* __restrict__ disp, const float* __restrict__ img,
     for (int p = blockIdx.x * kSmoothThreads + threadIdx.x; p < n; p += gridDim.x * kSmoothThreads) {
         const int y = p / W, x = p - y * W;
         const float dc = __ldg(d + p);
-        const float c = dc * inv;
+        // every normalised value rounded on its own (__fmul_rn: no FMA contraction into the difference), so equal
+        // neighbours differ by exactly 0 and get no gradient, like abs at 0 in eager PyTorch
+        const float c = __fmul_rn(dc, inv);
         float g = 0.f;
-        if (x + 1 < W) g += gx * sgn(c - __ldg(d + p + 1) * inv) * edge_weight(im, img_sc, p, p + 1);
-        if (x > 0) g -= gx * sgn(__ldg(d + p - 1) * inv - c) * edge_weight(im, img_sc, p - 1, p);
-        if (y + 1 < H) g += gy * sgn(c - __ldg(d + p + W) * inv) * edge_weight(im, img_sc, p, p + W);
-        if (y > 0) g -= gy * sgn(__ldg(d + p - W) * inv - c) * edge_weight(im, img_sc, p - W, p);
+        if (x + 1 < W) g += gx * sgn(c - __fmul_rn(__ldg(d + p + 1), inv)) * edge_weight(im, img_sc, p, p + 1);
+        if (x > 0) g -= gx * sgn(__fmul_rn(__ldg(d + p - 1), inv) - c) * edge_weight(im, img_sc, p - 1, p);
+        if (y + 1 < H) g += gy * sgn(c - __fmul_rn(__ldg(d + p + W), inv)) * edge_weight(im, img_sc, p, p + W);
+        if (y > 0) g -= gy * sgn(__fmul_rn(__ldg(d + p - W), inv) - c) * edge_weight(im, img_sc, p - W, p);
         g_norm[(int64_t)b * n + p] = g;
         part[0] += g * dc;
     }
