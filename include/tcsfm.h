@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define TCSFM_ABI_VERSION 18
+#define TCSFM_ABI_VERSION 19
 
 /* ---- flags ------------------------------------------------------------------ */
 /* Arithmetic flavour.  Eager PyTorch rounds after every operator, but a few ATen
@@ -188,6 +188,18 @@ int tcsfm_photo_sweep(const float* tgt, int64_t tgt_sc, const float* src, int64_
                       float* scratch, float* partials, float* sums,
                       float* rec, float* diff, float* mask, float* weight,
                       int N, int H, int W, float w_l1, float w_ssim, int flags, void* stream);
+/* The same sums, and the pose gradient of every hypothesis's loss_n = sums[n][0] / sums[n][1]:
+ *   g_proj[n] = d loss_n / d proj[n]   [N,12], already divided by sums[n][1] (NaN where it is 0)
+ * The mask (a comparison and the valid mask) and sums[n][1] carry no gradient; the gradient flows through diff (the
+ * warped image, over each pixel's 3x3 SSIM window with reflection padding) and through weight (the computed depth and
+ * the sampled source depth).  sums[n] has the bits tcsfm_photo_sweep gives.  partials
+ * [tcsfm_photo_sweep_grad_partial_floats(N, H, W)]: workspace, overwritten.  Three launches on `stream`; the forward
+ * is recomputed inside each CTA, so no workspace grows with N * H * W. */
+int64_t tcsfm_photo_sweep_grad_partial_floats(int N, int H, int W);
+int tcsfm_photo_sweep_grad(const float* tgt, int64_t tgt_sc, const float* src, int64_t src_sc,
+                           const float* tgt_depth, const float* src_depth, const float* kinv, const float* proj,
+                           float* scratch, float* partials, float* sums, float* g_proj,
+                           int N, int H, int W, float w_l1, float w_ssim, int flags, void* stream);
 
 /* ---- DepthOptimizer.compute_optimization_loss (optimization_experiments/optimizer.py:45-86): the
  *      reduction of the error maps of solve_pose_iteratively(return_errors=True) to the PFT loss --------

@@ -463,6 +463,32 @@ def photo_sweep(lib, tgt, src, tgt_depth, src_depth, kinv, proj, w_l1, w_ssim, f
     return sums, maps
 
 
+def photo_sweep_grad(lib, tgt, src, tgt_depth, src_depth, kinv, proj, w_l1, w_ssim, flags=0):
+    """photo_sweep's sums plus g_proj [N,3,4] = d (sums[n,0] / sums[n,1]) / d proj[n], three launches."""
+    n = proj.shape[0]
+    h, w = tgt.shape[-2], tgt.shape[-1]
+    _expect(tgt, (1, 3, h, w), "tgt")
+    _expect(src, (1, 3, h, w), "src")
+    _expect(tgt_depth, (1, 1, h, w), "tgt_depth")
+    _expect(src_depth, (1, 1, h, w), "src_depth")
+    _expect(kinv, (1, 3, 3), "kinv")
+    _expect(proj, (n, 3, 4), "proj")
+    tgt, _, tsc = image_view(tgt, "tgt")
+    src, _, ssc = image_view(src, "src")
+    td, sd = _f32c(tgt_depth, "tgt_depth"), _f32c(src_depth, "src_depth")
+    kinv, proj = _f32c(kinv, "kinv"), _f32c(proj, "proj")
+    dev = tgt.device
+    scratch = torch.empty((h, w), dtype=torch.float32, device=dev)
+    partials = torch.empty((lib.tcsfm_photo_sweep_grad_partial_floats(n, h, w),), dtype=torch.float32, device=dev)
+    sums = torch.empty((n, 2), dtype=torch.float32, device=dev)
+    g_proj = torch.empty((n, 3, 4), dtype=torch.float32, device=dev)
+    _call(lib, lib.tcsfm_photo_sweep_grad, "photo_sweep_grad", tgt.is_cuda,
+          _ptr(tgt), tsc, _ptr(src), ssc, _ptr(td), _ptr(sd), _ptr(kinv), _ptr(proj),
+          _ptr(scratch), _ptr(partials), _ptr(sums), _ptr(g_proj),
+          n, h, w, w_l1, w_ssim, flags, _stream(tgt), launches=3)
+    return sums, g_proj
+
+
 def _ptr_table(tensors):
     arr = (C.c_void_p * len(tensors))()
     for i, t in enumerate(tensors):

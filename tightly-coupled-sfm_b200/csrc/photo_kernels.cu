@@ -30,8 +30,10 @@ struct PhotoArgs {
     float w_l1, w_ssim, C1, C2;
 };
 
-// one channel of  w_l1 * clamp|x - y| + w_ssim * SSIM(x, y)  down a strip, x/y packed as float2
-template <bool kCoef>
+// one channel of  w_l1 * clamp|x - y| + w_ssim * SSIM(x, y)  down a strip, x/y packed as float2.
+// kCoef: the SSIM adjoint coefficients (Ay, B, Cc) of each pixel go to the [N,9,H,W] workspace planes at coef_ch;
+// kTileCoef: to the Tile<1> planes at coef_ch (plane stride kCells), at the strip's own cells, filler cells included.
+template <bool kCoef, bool kTileCoef = false>
 __device__ __forceinline__ void strip_channel(const float2* plane, int tx, int ty0, const PhotoArgs& P, bool first,
                                               float (&esum)[kPixPerThread], float* coef_ch, int gx, int gy0, int n) {
     using T1 = Tile<1>;
@@ -64,6 +66,11 @@ __device__ __forceinline__ void strip_channel(const float2* plane, int tx, int t
                 float* cp = coef_ch + gy * P.A.W + gx;
                 cp[0] = kf.Ay; cp[n] = kf.B; cp[2 * (int64_t)n] = kf.Cc;
             }
+        }
+        if (kTileCoef) {
+            const SsimCoef kf = ssim_coef(s, t, P.A.third * P.w_ssim);
+            float* cp = coef_ch + T1::cell(tx, ty0 + k);
+            cp[0] = kf.Ay; cp[T1::kCells] = kf.B; cp[2 * T1::kCells] = kf.Cc;
         }
     }
 }
@@ -330,12 +337,156 @@ __device__ __forceinline__ void sweep_ring_cell(int r, int& cx, int& cy) {
     else { cx = kTileW; cy = r - 2 * (kTileW + 2) - kTileH; }
 }
 
+// ---------------------------------------------------------------------------
+// d loss_n / d proj_n of the loss surface, loss_n = E_n / V_n with E_n = sum((diff * mask) * weight), V_n = sum(mask):
+// the mask is a comparison (no gradient) and V_n a constant, so the gradient is dE_n / d proj_n over V_n.  One CTA per
+// (hypothesis, tile) recomputes the tile's forward (photo_sweep_kernel<F, true>), then runs the adjoint in cell space over the
+// tile and its ring: a cell's warped value is read by the 3x3 SSIM windows of the own pixels around it, so its gradient
+// is the gather of their coefficients (the form of photo_bwd_kernel).  Ring cells at the image border hold the
+// reflected pixel itself, so the reflection needs no duplicate taps here.  Each cell then runs the bilinear and
+// projective adjoints of its own warp; own pixels add the weight term through the sampled source depth and Z.
+// ---------------------------------------------------------------------------
+constexpr int kSweepGradParts = 14;       // per CTA: E, V, d E / d proj [12]
+
+// g[ch] = d E / d (warped value of channel ch) of the image pixel (rx, ry); g_weight = d E / d weight at that pixel
+// (own pixels only).  Adds d E / d proj through this pixel's warp into acc (row-major K[R|t]).
 template <int F>
-__global__ void __launch_bounds__(kTileThreads, 3)
+__device__ __forceinline__ void sweep_cell_adjoint(const SweepArgs& S, const Cam& cam, int rx, int ry, const float (&g)[3],
+                                                   float g_weight, float (&acc)[12]) {
+    const Arith& A = S.P.A;
+    const int pix = ry * A.W + rx;
+    WarpPt p;
+    warp_point<F>(cam, A, rx, ry, __ldg(S.tdep + pix), p);
+    const TapIdx ti = make_taps(p, A.H, A.W);
+    Taps tc[3];
+#pragma unroll
+    for (int ch = 0; ch < 3; ++ch) tc[ch] = load_taps(S.P.src, (int)(ch * S.P.src_sc), ti, A.W);
+    float g_ix = 0.f, g_iy = 0.f, g_Z = 0.f;
+#pragma unroll
+    for (int ch = 0; ch < 3; ++ch) bilinear_grad(tc[ch], p, g[ch], g_ix, g_iy);
+    if (g_weight != 0.f) {
+        // weight = 1 - depth_inconsistency(Z, sampled source depth)
+        const Taps td = load_taps(S.sdep, 0, ti, A.W);
+        float g_pd = 0.f;
+        depth_inconsistency_adjoint(p.Z, blend(td, ti), -g_weight, g_Z, g_pd);
+        bilinear_grad(td, p, g_pd, g_ix, g_iy);
+    }
+    const GeomGrad gg = geom_adjoint(cam, A, p, g_ix, g_iy, g_Z);
+#pragma unroll
+    for (int i = 0; i < 3; ++i) {
+        acc[i * 4 + 0] += gg.gp[i] * p.cam[0];
+        acc[i * 4 + 1] += gg.gp[i] * p.cam[1];
+        acc[i * 4 + 2] += gg.gp[i] * p.cam[2];
+        acc[i * 4 + 3] += gg.gp[i];
+    }
+}
+
+// The adjoint of one tile for photo_sweep_kernel<F, true>, after its forward: scales the raw coefficients the strips left
+// in `cs` by the upstream, then accumulates d E / d proj of the tile's cells into acc.  Contains __syncthreads().
+template <int F>
+__device__ __forceinline__ void sweep_tile_adjoint(const SweepArgs& S, const Cam& cam, const float2* tw, float* cs, int x0, int y0,
+                                                   const float (&diff)[kPixPerThread], const float (&m)[kPixPerThread],
+                                                   const float (&wgt)[kPixPerThread], float (&acc)[12]) {
+    using T1 = Tile<1>;
+    const Arith& A = S.P.A;
+    const int H = A.H, W = A.W;
+    // coefficients: d E / d diff = mask * weight at each own pixel, zero for the filler cells of partial tiles and the ring
+    const int tx = threadIdx.x & (kTileW - 1);
+    const int ty0 = (threadIdx.x >> 6) * kPixPerThread;
+    const int gx = x0 + tx;
+#pragma unroll
+    for (int k = 0; k < kPixPerThread; ++k) {
+        const float u = m[k] * wgt[k];
+        const int c = T1::cell(tx, ty0 + k);
+#pragma unroll
+        for (int j = 0; j < kPhotoCoefPlanes; ++j) cs[j * T1::kCells + c] = (m[k] != 0.f) ? cs[j * T1::kCells + c] * u : 0.f;
+    }
+    if (threadIdx.x < kSweepRingCells) {
+        int cx, cy;
+        sweep_ring_cell(threadIdx.x, cx, cy);
+#pragma unroll
+        for (int j = 0; j < kPhotoCoefPlanes; ++j) cs[j * T1::kCells + T1::cell(cx, cy)] = 0.f;
+    }
+    __syncthreads();
+
+#pragma unroll
+    for (int i = 0; i < 12; ++i) acc[i] = 0.f;
+    const float l1_scale = A.third * S.P.w_l1;
+    // own cells: the 3x3 coefficient sums slide down the strip, three row sums of the nine planes live at a time
+    float h[3][kPhotoCoefPlanes];
+    auto hsum = [&](int r, float (&out)[kPhotoCoefPlanes]) {
+        const int c1 = T1::cell(tx, ty0 - 1 + r);
+#pragma unroll
+        for (int j = 0; j < kPhotoCoefPlanes; ++j) {
+            const float* pl = cs + j * T1::kCells + c1;
+            out[j] = (pl[-1] + pl[0]) + pl[1];
+        }
+    };
+    hsum(0, h[0]);
+    hsum(1, h[1]);
+#pragma unroll
+    for (int k = 0; k < kPixPerThread; ++k) {
+        hsum(k + 2, h[(k + 2) % 3]);
+        const int gy = y0 + ty0 + k;
+        if (gx > W || gy > H) continue;         // filler cells that no pixel's window reaches
+        const bool own = gx < W && gy < H;
+        const int c = T1::cell(tx, ty0 + k);
+        const float gl1 = own ? m[k] * wgt[k] * l1_scale : 0.f;
+        float g[3];
+#pragma unroll
+        for (int ch = 0; ch < 3; ++ch) {
+            float V[3];
+#pragma unroll
+            for (int j = 0; j < 3; ++j) {
+                const int q = 3 * ch + j;
+                V[j] = (h[k % 3][q] + h[(k + 1) % 3][q]) + h[(k + 2) % 3][q];
+            }
+            const float2 tv = tw[ch * T1::kCells + c];
+            const float dlt = tv.x - tv.y;
+            float gw = V[0] + 2.0f * tv.y * V[1] + tv.x * V[2];
+            if (fabsf(dlt) <= 1.0f) gw += (dlt > 0.f) ? -gl1 : ((dlt < 0.f) ? gl1 : 0.f);
+            g[ch] = gw;
+        }
+        // a filler cell one past the last row / column holds the reflection of the one before the last
+        sweep_cell_adjoint<F>(S, cam, gx < W ? gx : 2 * W - 2 - gx, gy < H ? gy : 2 * H - 2 - gy, g,
+                              own ? diff[k] * m[k] : 0.f, acc);
+    }
+    // ring cells: the coefficients of the own pixels among their 3x3 neighbours
+    if (threadIdx.x < kSweepRingCells) {
+        int cx, cy, ry = 0, rx = 0;
+        sweep_ring_cell(threadIdx.x, cx, cy);
+        const int c = T1::cell(cx, cy);
+        if (T1::cell_to_reflected(c, x0, y0, H, W, ry, rx)) {
+            float V[kPhotoCoefPlanes];
+#pragma unroll
+            for (int j = 0; j < kPhotoCoefPlanes; ++j) V[j] = 0.f;
+            for (int dy = -1; dy <= 1; ++dy)
+                for (int dx = -1; dx <= 1; ++dx) {
+                    const int nx = cx + dx, ny = cy + dy;
+                    if (nx < 0 || nx >= kTileW || ny < 0 || ny >= kTileH) continue;
+#pragma unroll
+                    for (int j = 0; j < kPhotoCoefPlanes; ++j) V[j] += cs[j * T1::kCells + T1::cell(nx, ny)];
+                }
+            float g[3];
+#pragma unroll
+            for (int ch = 0; ch < 3; ++ch) {
+                const float2 tv = tw[ch * T1::kCells + c];
+                g[ch] = V[3 * ch] + 2.0f * tv.y * V[3 * ch + 1] + tv.x * V[3 * ch + 2];
+            }
+            sweep_cell_adjoint<F>(S, cam, rx, ry, g, 0.f, acc);
+        }
+    }
+}
+
+// One CTA per (hypothesis, tile).  kGrad = false: the sums and optional maps of tcsfm_photo_sweep.  kGrad = true: the
+// same forward, instruction for instruction (so E and V keep their bits), whose strips also leave their SSIM adjoint
+// coefficients in shared memory; then the adjoint of the tile (sweep_tile_adjoint), and a partial (E, V, dE/dproj[12]).
+template <int F, bool kGrad>
+__global__ void __launch_bounds__(kTileThreads, kGrad ? 2 : 3)
 photo_sweep_kernel(const __grid_constant__ SweepArgs S) {
     using T1 = Tile<1>;
     TCSFM_DYN_SMEM(float2, tw);                                  // [3][cells] (target, warped source)
-    TCSFM_SHARED float red[2 * (kTileThreads / 32)];
+    TCSFM_SHARED float red[(kGrad ? kSweepGradParts : 2) * (kTileThreads / 32)];
     const Arith& A = S.P.A;
     const int H = A.H, W = A.W, n = H * W;
     const int hyp = blockIdx.x / S.tiles, tile = blockIdx.x - hyp * S.tiles;
@@ -346,6 +497,7 @@ photo_sweep_kernel(const __grid_constant__ SweepArgs S) {
     const int tx = threadIdx.x & (kTileW - 1);
     const int ty0 = (threadIdx.x >> 6) * kPixPerThread;
     const int gx = x0 + tx;
+    float* cs = kGrad ? reinterpret_cast<float*>(tw + 3 * T1::kCells) : nullptr;   // kGrad: [9][cells] coefficients
     // own pixels: the cell, plus valid and weight = 1 - depth_inconsistency(computed, projected depth) of the warp.
     // Own cells that no consumer reads (partial tiles) are filled from a clamped pixel, as in the pair forward.
     bool valid[kPixPerThread];
@@ -375,15 +527,20 @@ photo_sweep_kernel(const __grid_constant__ SweepArgs S) {
     __syncthreads();
     float esum[kPixPerThread];
 #pragma unroll
-    for (int ch = 0; ch < 3; ++ch) strip_channel<false>(tw + ch * T1::kCells, tx, ty0, S.P, ch == 0, esum, nullptr, gx, y0 + ty0, n);
+    for (int ch = 0; ch < 3; ++ch)
+        strip_channel<false, kGrad>(tw + ch * T1::kCells, tx, ty0, S.P, ch == 0, esum, kGrad ? cs + 3 * ch * T1::kCells : nullptr,
+                                    gx, y0 + ty0, n);
     float part_e = 0.f, part_m = 0.f;
+    float diff_k[kPixPerThread], m_k[kPixPerThread];             // kGrad: per own pixel, 0 for filler pixels
 #pragma unroll
     for (int k = 0; k < kPixPerThread; ++k) {
         const int gy = y0 + ty0 + k;
+        if constexpr (kGrad) { diff_k[k] = 0.f; m_k[k] = 0.f; }
         if (gx < W && gy < H) {
             const int pix = gy * W + gx;
             const float diff = mean3_of_sum<F>(esum[k], A);
             const float m = (diff < __ldg(S.P.auto_err + pix)) ? (valid[k] ? 1.f : 0.f) : 0.f;
+            if constexpr (kGrad) { diff_k[k] = diff; m_k[k] = m; }
             // (diff_img * valid_mask) * weight_mask, each product rounded like the eager expression
             part_e = __fadd_rn(part_e, __fmul_rn(__fmul_rn(diff, m), wgt[k]));
             part_m = __fadd_rn(part_m, m);
@@ -397,18 +554,41 @@ photo_sweep_kernel(const __grid_constant__ SweepArgs S) {
             }
         }
     }
-    // fixed-order block sum: butterfly within each warp, then the warps in index order
-    part_e = warp_sum(part_e);
-    part_m = warp_sum(part_m);
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    if (lane == 0) { red[warp] = part_e; red[kTileThreads / 32 + warp] = part_m; }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        float se = red[0], sm = red[kTileThreads / 32];
-        for (int w = 1; w < kTileThreads / 32; ++w) { se = __fadd_rn(se, red[w]); sm = __fadd_rn(sm, red[kTileThreads / 32 + w]); }
-        float* dst = S.partials + ((int64_t)tile * S.N + hyp) * 2;
-        dst[0] = se;
-        dst[1] = sm;
+    if constexpr (kGrad) {
+        float acc[12];
+        sweep_tile_adjoint<F>(S, cam, tw, cs, x0, y0, diff_k, m_k, wgt, acc);
+        float part[kSweepGradParts];
+        part[0] = part_e;
+        part[1] = part_m;
+#pragma unroll
+        for (int i = 0; i < 12; ++i) part[2 + i] = acc[i];
+        const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+        // fixed-order block sum: for every value the butterfly of warp_sum (so E and V get the forward's bits), then
+        // the warps in index order
+        const float s = warp_sum_transposed<kSweepGradParts>(part, lane);
+        const int idx = (lane >> 1) & 15;
+        if (!(lane & 1) && idx < kSweepGradParts) red[idx * (kTileThreads / 32) + warp] = s;
+        __syncthreads();
+        if (threadIdx.x < kSweepGradParts) {
+            const float* r = red + threadIdx.x * (kTileThreads / 32);
+            float v = r[0];
+            for (int w = 1; w < kTileThreads / 32; ++w) v = __fadd_rn(v, r[w]);
+            S.partials[((int64_t)tile * S.N + hyp) * kSweepGradParts + threadIdx.x] = v;
+        }
+    } else {
+        // fixed-order block sum: butterfly within each warp, then the warps in index order
+        part_e = warp_sum(part_e);
+        part_m = warp_sum(part_m);
+        const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+        if (lane == 0) { red[warp] = part_e; red[kTileThreads / 32 + warp] = part_m; }
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            float se = red[0], sm = red[kTileThreads / 32];
+            for (int w = 1; w < kTileThreads / 32; ++w) { se = __fadd_rn(se, red[w]); sm = __fadd_rn(sm, red[kTileThreads / 32 + w]); }
+            float* dst = S.partials + ((int64_t)tile * S.N + hyp) * 2;
+            dst[0] = se;
+            dst[1] = sm;
+        }
     }
 }
 
@@ -428,6 +608,30 @@ photo_sweep_finish_kernel(const float* __restrict__ partials, int tiles, int N, 
     }
     sums[2 * hyp] = (float)e;
     sums[2 * hyp + 1] = m;
+}
+
+// sums[n] exactly as photo_sweep_finish_kernel forms them; g_proj[n] = (d E / d proj, its partials added in tile
+// order in double) / valid_sum, NaN where no pixel is valid.
+__global__ void __launch_bounds__(kSweepFinishThreads)
+photo_sweep_grad_finish_kernel(const float* __restrict__ partials, int tiles, int N, float* __restrict__ sums,
+                               float* __restrict__ g_proj) {
+    const int hyp = blockIdx.x * kSweepFinishThreads + threadIdx.x;
+    if (hyp >= N) return;
+    double e = 0.0, g[12];
+    float m = 0.f;
+#pragma unroll
+    for (int i = 0; i < 12; ++i) g[i] = 0.0;
+    for (int t = 0; t < tiles; ++t) {
+        const float* p = partials + ((int64_t)t * N + hyp) * kSweepGradParts;
+        e += (double)__ldg(p);
+        m = __fadd_rn(m, __ldg(p + 1));
+#pragma unroll
+        for (int i = 0; i < 12; ++i) g[i] += (double)__ldg(p + 2 + i);
+    }
+    sums[2 * hyp] = (float)e;
+    sums[2 * hyp + 1] = m;
+#pragma unroll
+    for (int i = 0; i < 12; ++i) g_proj[12 * hyp + i] = (float)(g[i] / (double)m);
 }
 
 static int sweep_tiles(int H, int W) { return ((W + kTileW - 1) / kTileW) * ((H + kTileH - 1) / kTileH); }
@@ -492,12 +696,10 @@ extern "C" int64_t tcsfm_photo_sweep_partial_floats(int N, int H, int W) {
     return 2 * (int64_t)N * sweep_tiles(H, W);
 }
 
-extern "C" int tcsfm_photo_sweep(const float* tgt, int64_t tgt_sc, const float* src, int64_t src_sc,
-                                 const float* tgt_depth, const float* src_depth, const float* kinv, const float* proj,
-                                 float* scratch, float* partials, float* sums,
-                                 float* rec, float* diff, float* mask, float* weight,
-                                 int N, int H, int W, float w_l1, float w_ssim, int flags, void* stream) {
-    const char* who = "tcsfm_photo_sweep";
+// The argument checks and launch arguments shared by tcsfm_photo_sweep and tcsfm_photo_sweep_grad.
+static int fill_sweep(SweepArgs& S, const char* who, const float* tgt, int64_t tgt_sc, const float* src, int64_t src_sc,
+                      const float* tgt_depth, const float* src_depth, const float* kinv, const float* proj,
+                      float* scratch, float* partials, float* sums, int N, int H, int W, float w_l1, float w_ssim, int flags) {
     if (N <= 0 || H < 2 || W < 2) { set_error("%s: bad shape N=%d H=%d W=%d", who, N, H, W); return 1; }
     if (!tgt || !src || !tgt_depth || !src_depth || !kinv || !proj) { set_error("%s: null input pointer", who); return 1; }
     if (!scratch || !partials || !sums) { set_error("%s: null scratch, partials or sums", who); return 1; }
@@ -508,21 +710,66 @@ extern "C" int tcsfm_photo_sweep(const float* tgt, int64_t tgt_sc, const float* 
     if (tgt_sc < 0 || src_sc < 0 || 2 * tgt_sc + n > 0x7fffffff || 2 * src_sc + n > 0x7fffffff) {
         set_error("%s: channel strides %lld / %lld out of range", who, (long long)tgt_sc, (long long)src_sc); return 1;
     }
-    SweepArgs S;
     memset(&S, 0, sizeof(S));
     S.P.tgt = tgt; S.P.tgt_sc = tgt_sc; S.P.src = src; S.P.src_sc = src_sc; S.P.auto_err = scratch;
     S.P.A = make_arith(H, W, flags);
     S.P.w_l1 = w_l1; S.P.w_ssim = w_ssim;
     S.P.C1 = (float)(0.01 * 0.01); S.P.C2 = (float)(0.03 * 0.03);
     S.tdep = tgt_depth; S.sdep = src_depth; S.kinv = kinv; S.proj = proj; S.partials = partials;
-    S.rec = rec; S.diff = diff; S.mask = mask; S.weight = weight;
     S.N = N; S.tiles = tiles;
+    return 0;
+}
+
+extern "C" int tcsfm_photo_sweep(const float* tgt, int64_t tgt_sc, const float* src, int64_t src_sc,
+                                 const float* tgt_depth, const float* src_depth, const float* kinv, const float* proj,
+                                 float* scratch, float* partials, float* sums,
+                                 float* rec, float* diff, float* mask, float* weight,
+                                 int N, int H, int W, float w_l1, float w_ssim, int flags, void* stream) {
+    const char* who = "tcsfm_photo_sweep";
+    SweepArgs S;
+    if (int rc = fill_sweep(S, who, tgt, tgt_sc, src, src_sc, tgt_depth, src_depth, kinv, proj, scratch, partials, sums,
+                            N, H, W, w_l1, w_ssim, flags)) return rc;
+    S.rec = rec; S.diff = diff; S.mask = mask; S.weight = weight;
+    const int tiles = S.tiles;
     const size_t smem = 3 * Tile<1>::kCells * sizeof(float2);
     TCSFM_DISPATCH_FLAVOUR(flags, TCSFM_LAUNCH(photo_auto_err_kernel<F>, dim3(tiles), dim3(kTileThreads), smem, stream, S.P));
     if (int rc = check_launch(who)) return rc;
-    TCSFM_DISPATCH_FLAVOUR(flags, TCSFM_LAUNCH(photo_sweep_kernel<F>, dim3((unsigned)(tiles * N)), dim3(kTileThreads), smem, stream, S));
+    TCSFM_DISPATCH_FLAVOUR(flags, auto* sweep = photo_sweep_kernel<F, false>;
+                                  TCSFM_LAUNCH(sweep, dim3((unsigned)(tiles * N)), dim3(kTileThreads), smem, stream, S));
     if (int rc = check_launch(who)) return rc;
     TCSFM_LAUNCH(photo_sweep_finish_kernel, dim3((N + kSweepFinishThreads - 1) / kSweepFinishThreads), dim3(kSweepFinishThreads), 0,
                  stream, partials, tiles, N, sums);
+    return check_launch(who);
+}
+
+extern "C" int64_t tcsfm_photo_sweep_grad_partial_floats(int N, int H, int W) {
+    if (N <= 0 || H <= 0 || W <= 0) return 0;
+    return kSweepGradParts * (int64_t)N * sweep_tiles(H, W);
+}
+
+extern "C" int tcsfm_photo_sweep_grad(const float* tgt, int64_t tgt_sc, const float* src, int64_t src_sc,
+                                      const float* tgt_depth, const float* src_depth, const float* kinv, const float* proj,
+                                      float* scratch, float* partials, float* sums, float* g_proj,
+                                      int N, int H, int W, float w_l1, float w_ssim, int flags, void* stream) {
+    const char* who = "tcsfm_photo_sweep_grad";
+    SweepArgs S;
+    if (int rc = fill_sweep(S, who, tgt, tgt_sc, src, src_sc, tgt_depth, src_depth, kinv, proj, scratch, partials, sums,
+                            N, H, W, w_l1, w_ssim, flags)) return rc;
+    if (!g_proj) { set_error("%s: null g_proj", who); return 1; }
+    const int tiles = S.tiles;
+    const size_t smem_fwd = 3 * Tile<1>::kCells * sizeof(float2);
+    const size_t smem = smem_fwd + kPhotoCoefPlanes * Tile<1>::kCells * sizeof(float);
+#ifndef TCSFM_HOST_EMU
+    cudaError_t e = cudaSuccess;
+    TCSFM_DISPATCH_FLAVOUR(flags, e = cudaFuncSetAttribute(photo_sweep_kernel<F, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    if (e != cudaSuccess) { set_error("%s: cannot raise dynamic smem: %s", who, cudaGetErrorString(e)); return 2; }
+#endif
+    TCSFM_DISPATCH_FLAVOUR(flags, TCSFM_LAUNCH(photo_auto_err_kernel<F>, dim3(tiles), dim3(kTileThreads), smem_fwd, stream, S.P));
+    if (int rc = check_launch(who)) return rc;
+    TCSFM_DISPATCH_FLAVOUR(flags, auto* sweep = photo_sweep_kernel<F, true>;
+                                  TCSFM_LAUNCH(sweep, dim3((unsigned)(tiles * N)), dim3(kTileThreads), smem, stream, S));
+    if (int rc = check_launch(who)) return rc;
+    TCSFM_LAUNCH(photo_sweep_grad_finish_kernel, dim3((N + kSweepFinishThreads - 1) / kSweepFinishThreads), dim3(kSweepFinishThreads), 0,
+                 stream, partials, tiles, N, sums, g_proj);
     return check_launch(who);
 }

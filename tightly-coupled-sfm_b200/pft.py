@@ -4,7 +4,8 @@ optimizer.py:29-97) and ``compute_photometric_error`` (optimization_experiments/
 helpers.py:8-23).  The optimisation driver itself (deep copies of the depth net,
 Adam, plotting; optimizer.py:136-297) is the reference's harness and calls these.
 ``photometric_loss_surface`` evaluates ``compute_photometric_error`` for N pose hypotheses of one pair in one call
-(the loss-surface plots, plot_loss_surface.py:11-87).
+(the loss-surface plots, plot_loss_surface.py:11-87); ``photometric_loss_surface_and_grad`` also returns the pose
+gradient of every hypothesis's loss.
 """
 import torch
 
@@ -92,24 +93,59 @@ def photometric_loss_surface(target_img, source_img, target_depth, source_depth,
     ops._require_cuda(target_img, source_img, target_depth, source_depth, poses, intrinsics)
     if torch.is_grad_enabled() and any(t.requires_grad for t in (target_img, source_img, target_depth, source_depth,
                                                                      poses, intrinsics)):
-        raise NotImplementedError("photometric_loss_surface is forward only: no gradient of the surface is implemented")
-    if target_img.dim() != 4 or target_img.shape[0] != 1:
-        raise ValueError("photometric_loss_surface: one frame pair (batch 1) per call, got target_img %s"
-                         % list(target_img.shape))
-    if poses.dim() != 2 or poses.shape[0] < 1 or poses.shape[1] not in (6, 8):
-        raise ValueError("photometric_loss_surface: poses must be [N,6] or [N,8] with N >= 1, got %s" % list(poses.shape))
+        raise NotImplementedError("photometric_loss_surface is forward only: no gradient of the surface is implemented "
+                                  "(photometric_loss_surface_and_grad returns the pose gradient)")
+    _check_surface_args(target_img, poses)
     h, w = target_img.shape[2], target_img.shape[3]
     kinv = stn.inverse_intrinsics(intrinsics)
     with ops._guard(poses):
-        # every hypothesis as the batch-1 call of compute_photometric_error forms it: K @ [R|t] of -pose with the
-        # batch-1 rounding of the pose algebra, and the batch-1 warp arithmetic, whatever N is
-        if intrinsics.is_cuda:
-            proj = _raw.pose_proj_fwd(ops.lib(), poses[:, 0:6], intrinsics, -1.0, ops.pose_flags(1))
-        else:       # CPU tensors (test builds): the eager operators stn.projection_matrices takes there
-            proj = intrinsics @ stn.pose_vec2mat(-poses[:, 0:6])
+        proj = _surface_projections(poses, intrinsics)
         sums, maps = _raw.photo_sweep(ops.lib(), target_img, source_img, target_depth, source_depth, kinv, proj,
                                       0.15, 0.85, ops.arith_flags(1, h, w), want_maps=return_maps)
     out = {'loss': sums[:, 0] / sums[:, 1], 'error_sum': sums[:, 0], 'valid_sum': sums[:, 1]}
     if return_maps:
         out['img_rec'], out['diff_img'], out['valid_mask'], out['weight_mask'] = maps
     return out
+
+
+def photometric_loss_surface_and_grad(target_img, source_img, target_depth, source_depth, poses, intrinsics):
+    """photometric_loss_surface's 'loss', 'error_sum' and 'valid_sum' (the same bits) plus 'pose_grad', the shape of
+    `poses`: row n is d loss[n] / d poses[n] as autograd gives it for the batch-1 expression
+    sum(diff_img * valid_mask * weight_mask) / sum(valid_mask) of compute_photometric_error(..., poses[n:n+1], ...).
+    The masks carry no gradient; the target image, the depths and the intrinsics get none; columns 6: of [N,8] poses
+    are 0; a row with no valid pixel is NaN.
+
+    Functional, not autograd: no graph is recorded and the outputs do not require grad (inputs that require grad are
+    read as values).  Seven launches whatever N is: K^-1, K @ [R|t] of every hypothesis, the three of
+    tcsfm_photo_sweep_grad (the forward is recomputed inside each CTA, so no workspace grows with N * H * W), the chain
+    rule to the pose and the division; [N,8] poses add one for the zero columns."""
+    ops._require_cuda(target_img, source_img, target_depth, source_depth, poses, intrinsics)
+    _check_surface_args(target_img, poses)
+    h, w = target_img.shape[2], target_img.shape[3]
+    with torch.no_grad(), ops._guard(poses):
+        kinv = stn.inverse_intrinsics(intrinsics)
+        proj = _surface_projections(poses, intrinsics)
+        sums, g_proj = _raw.photo_sweep_grad(ops.lib(), target_img, source_img, target_depth, source_depth, kinv, proj,
+                                             0.15, 0.85, ops.arith_flags(1, h, w))
+        pose_grad = _raw.pose_proj_bwd(ops.lib(), poses[:, 0:6], intrinsics, -1.0, g_proj)
+        if poses.shape[1] > 6:
+            pose_grad = torch.nn.functional.pad(pose_grad, (0, poses.shape[1] - 6))
+        return {'loss': sums[:, 0] / sums[:, 1], 'error_sum': sums[:, 0], 'valid_sum': sums[:, 1],
+                'pose_grad': pose_grad}
+
+
+def _check_surface_args(target_img, poses):
+    if target_img.dim() != 4 or target_img.shape[0] != 1:
+        raise ValueError("photometric_loss_surface: one frame pair (batch 1) per call, got target_img %s"
+                         % list(target_img.shape))
+    if poses.dim() != 2 or poses.shape[0] < 1 or poses.shape[1] not in (6, 8):
+        raise ValueError("photometric_loss_surface: poses must be [N,6] or [N,8] with N >= 1, got %s" % list(poses.shape))
+
+
+def _surface_projections(poses, intrinsics):
+    """K @ [R|t] of -pose for every hypothesis, as the batch-1 call of compute_photometric_error forms it: with the
+    batch-1 rounding of the pose algebra (and, in the sweep, the batch-1 warp arithmetic) whatever N is."""
+    if intrinsics.is_cuda:
+        return _raw.pose_proj_fwd(ops.lib(), poses[:, 0:6], intrinsics, -1.0, ops.pose_flags(1))
+    # CPU tensors (test builds): the eager operators stn.projection_matrices takes there
+    return intrinsics @ stn.pose_vec2mat(-poses[:, 0:6])

@@ -4,12 +4,18 @@
          mean (diff_img * valid_mask * weight_mask).sum() / valid_mask.sum() per pose sample;
   batch  one pft.photometric_loss_surface call over all samples.
 
+and, for the pose gradient of every sample (the "grad" section):
+
+  loop   per sample one compute_photometric_error call with a pose that requires grad, the masked mean and
+         .backward(), then pose.grad;
+  batch  one pft.photometric_loss_surface_and_grad call over all samples (loss and pose_grad).
+
 Input: what `bench.py --workload sweep` evaluates, make_frames(1, 192, 640, n_src=2, seed=0, KITTI intrinsics) with a
 line of forward-translation (pose column 2) and a line of yaw (column 4) samples, linspace(-0.05, 0.05, n) each:
 n = 100 (bench.py's default --sweep-evals, N = 200) and n = 50 (the demo's, N = 100).  Both are timed like
 main_sweep: wall clock of a whole sweep including the final device-to-host copy, after one warm-up sweep, the two
 alternated round by round.  The batched op's device time per call comes from CUDA events around `--device-iters`
-back-to-back calls.  The working set (one frame pair, ~2.5 MB) stays in L2, so no HBM roofline fraction is claimed.
+back-to-back calls, next to the forward-only call's in the grad section.  The working set (one frame pair, ~2.5 MB) stays in L2, so no HBM roofline fraction is claimed.
 
 Usage: python tools/bench_photo_sweep.py [--rounds R] [--device-iters I]"""
 import argparse
@@ -105,6 +111,77 @@ def measure(fr, n, rounds, device_iters):
             "max_rel_diff_loss": rel}
 
 
+def measure_grad(fr, n, rounds, device_iters):
+    args = (fr["target"], fr["sources"][0], fr["depths"][0], fr["depths"][1])
+    deltas = torch.linspace(-0.05, 0.05, n)
+    deltas_dev = deltas.to(fr["K"].device)
+
+    def poses():
+        p = fr["poses"][0].repeat(2 * n, 1)
+        p[:n, 2] += deltas_dev
+        p[n:, 4] += deltas_dev
+        return p
+
+    def loop():
+        grads = []
+        for axis in (2, 4):
+            for d in deltas:
+                pose = fr["poses"][0].clone()
+                pose[:, axis] += d
+                pose.requires_grad_(True)
+                r = pft.compute_photometric_error(*args, pose, fr["K"])
+                ((r["diff_img"] * r["valid_mask"] * r["weight_mask"]).sum() / r["valid_mask"].sum()).backward()
+                grads.append(pose.grad[0])
+        return torch.stack(grads)
+
+    def batch():
+        return pft.photometric_loss_surface_and_grad(*args, poses(), fr["K"])["pose_grad"]
+
+    def timed(fn):
+        torch.cuda.synchronize()
+        t0 = time.perf_counter()
+        host = fn().cpu()
+        return time.perf_counter() - t0, host
+
+    loop(), batch()                                 # warm-up sweeps
+    t_loop, t_batch = [], []
+    for _ in range(rounds):
+        dt, ref = timed(loop)
+        t_loop.append(dt)
+        dt, got = timed(batch)
+        t_batch.append(dt)
+    rel = ((got.double() - ref.double()).norm(dim=1) / ref.double().norm(dim=1)).max().item()
+
+    def device_ms(fn):
+        for _ in range(10):
+            fn()
+        torch.cuda.synchronize()
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record()
+        for _ in range(device_iters):
+            fn()
+        e1.record()
+        torch.cuda.synchronize()
+        return e0.elapsed_time(e1) / device_iters
+
+    p = poses()
+    with torch.no_grad():
+        ms_grad = device_ms(lambda: pft.photometric_loss_surface_and_grad(*args, p, fr["K"]))
+        ms_fwd = device_ms(lambda: pft.photometric_loss_surface(*args, p, fr["K"]))
+    evals = 2 * n
+    return {"N": evals,
+            "loop_evals_per_s": round(evals / statistics.median(t_loop), 1),
+            "batch_evals_per_s": round(evals / statistics.median(t_batch), 1),
+            "speedup": round(statistics.median(t_loop) / statistics.median(t_batch), 2),
+            "loop_ms_per_sweep": [round(t * 1e3, 3) for t in t_loop],
+            "batch_ms_per_sweep": [round(t * 1e3, 3) for t in t_batch],
+            "grad_device_ms_per_call": round(ms_grad, 4),
+            "forward_device_ms_per_call": round(ms_fwd, 4),
+            "grad_device_us_per_eval": round(ms_grad * 1e3 / evals, 3),
+            "device_calls_timed": device_iters,
+            "max_rel_diff_pose_grad": rel}
+
+
 def main():
     ap = argparse.ArgumentParser(description=__doc__.splitlines()[0])
     ap.add_argument("--rounds", type=int, default=5, help="alternated loop / batch sweeps per configuration")
@@ -122,7 +199,12 @@ def main():
                       "CUDA events",
             "note": "working set (one frame pair, ~2.5 MB) is L2-resident: no HBM roofline fraction is claimed",
             "configs": {"bench_sweep_default_100x2": measure(fr, 100, args.rounds, args.device_iters),
-                        "demo_50x2": measure(fr, 50, args.rounds, args.device_iters)}}
+                        "demo_50x2": measure(fr, 50, args.rounds, args.device_iters)},
+            "grad": {"metric": "loss-surface evaluations with the pose gradient per s: batch-1 forward + backward loop "
+                               "vs one photometric_loss_surface_and_grad call",
+                     "max_rel_diff": "largest |pose_grad - loop| / |loop| over the rows",
+                     "configs": {"bench_sweep_default_100x2": measure_grad(fr, 100, args.rounds, args.device_iters),
+                                 "demo_50x2": measure_grad(fr, 50, args.rounds, args.device_iters)}}}
     print(json.dumps(line))
 
 
