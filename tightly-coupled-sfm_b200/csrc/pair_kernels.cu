@@ -653,19 +653,9 @@ pair_bwd_kernel(const __grid_constant__ PairLaunch L) {
             const int cell = pcell(tx, ty0 + k);
             const float dep = cs[6 * kPlane + cell], m = __ldg(mask + pix);
             const float d0 = depth_mask ? __ldg(coef + (9 * n + pix)) : 0.f;
-#ifdef TCSFM_BWD_D_STAGED
-            float tg3[3];
-#pragma unroll
-            for (int ch = 0; ch < 3; ++ch) tg3[ch] = __ldg(c.tgt + (ch * c.tgt_sc + pix));
-#endif
             WarpPt p;
             warp_point<F>(cam, A, gx, gy, dep, p);
             const TapIdx ti = make_taps(p, H, W);
-#ifdef TCSFM_BWD_D_STAGED
-            Taps tv3[3];
-#pragma unroll
-            for (int ch = 0; ch < 3; ++ch) tv3[ch] = load_taps(c.ref, ch * c.ref_sc, ti, W);
-#endif
             const float Gd = Gs[cell];
             // d loss / d dd = c_dep * mask - Gd * diff0   (diff = diff0 * (1 - dd), losses.py:176-177)
             const float Gdd = sc.c_dep * m - Gd * d0;
@@ -681,13 +671,8 @@ pair_bwd_kernel(const __grid_constant__ PairLaunch L) {
             const float gl1 = G0 * A.third * L.w_l1;
 #pragma unroll
             for (int ch = 0; ch < 3; ++ch) {
-#ifdef TCSFM_BWD_D_STAGED
-                const Taps tv = tv3[ch];
-                const float t = tg3[ch];
-#else
                 const Taps tv = load_taps(c.ref, ch * c.ref_sc, ti, W);
                 const float t = __ldg(c.tgt + (ch * c.tgt_sc + pix));
-#endif
                 const float w = blend(tv, ti);
                 const float dlt = t - w;
                 float gwc = cs[(2 * ch) * kPlane + cell] + w * cs[(2 * ch + 1) * kPlane + cell];
