@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define TCSFM_ABI_VERSION 19
+#define TCSFM_ABI_VERSION 20
 
 /* ---- flags ------------------------------------------------------------------ */
 /* Arithmetic flavour.  Eager PyTorch rounds after every operator, but a few ATen
@@ -200,6 +200,25 @@ int tcsfm_photo_sweep_grad(const float* tgt, int64_t tgt_sc, const float* src, i
                            const float* tgt_depth, const float* src_depth, const float* kinv, const float* proj,
                            float* scratch, float* partials, float* sums, float* g_proj,
                            int N, int H, int W, float w_l1, float w_ssim, int flags, void* stream);
+/* Multi-start refinement: `steps` Adam updates of each of the N poses [N,6] (in place, un-negated like the `pose` of
+ * compute_photometric_error) on its loss_n = sums[n][0] / sums[n][1] above.  K [9] is the intrinsics; K[R|t] of every
+ * pose is formed as tcsfm_pose_proj_fwd(poses, -1, K, 1, proj, N, pose_flags) forms it.  For t = 1 .. steps, with
+ *   c1 = lr / (1 - beta1^t),  c2 = sqrt(1 - beta2^t)
+ * and b1 = beta1, a1 = 1 - beta1, b2 = beta2, a2 = 1 - beta2, e = eps, each computed in double and rounded to fp32 once,
+ * and g the pose gradient of tcsfm_photo_sweep_grad + tcsfm_pose_proj_bwd (sign -1), every column updates as
+ *   m = b1*m + a1*g;  v = b2*v + a2*(g*g);  p = p - c1*(m / (sqrt(v)/c2 + e))
+ * with every operation rounded to fp32 (m = v = 0 at t = 1).  A pose whose sums[n][1] is 0 is not updated.
+ *   loss [(steps+1)*N]: row k = loss_n at the poses after k updates (NaN where no pixel is valid);
+ *   best_loss [N], best_step [N], best_pose [N,6]: the smallest finite loss of row n's history, the first k that
+ *   reaches it and the pose there (NaN, -1 and the starting pose when there is none).
+ * Workspace, overwritten: m, v [N,6], proj [N,12], scratch [H,W], partials [tcsfm_photo_sweep_grad_partial_floats(N, H,
+ * W)].  2*steps + 4 launches on `stream`; no allocation, no synchronisation, the same bits on every call. */
+int tcsfm_photo_refine(const float* tgt, int64_t tgt_sc, const float* src, int64_t src_sc,
+                       const float* tgt_depth, const float* src_depth, const float* kinv, const float* K,
+                       float* poses, float* m, float* v, float* proj, float* scratch, float* partials,
+                       float* loss, float* best_loss, int* best_step, float* best_pose,
+                       int N, int H, int W, int steps, double lr, double beta1, double beta2, double eps,
+                       float w_l1, float w_ssim, int flags, int pose_flags, void* stream);
 
 /* ---- DepthOptimizer.compute_optimization_loss (optimization_experiments/optimizer.py:45-86): the
  *      reduction of the error maps of solve_pose_iteratively(return_errors=True) to the PFT loss --------

@@ -489,6 +489,43 @@ def photo_sweep_grad(lib, tgt, src, tgt_depth, src_depth, kinv, proj, w_l1, w_ss
     return sums, g_proj
 
 
+def photo_refine(lib, tgt, src, tgt_depth, src_depth, kinv, K, poses, steps, lr, beta1, beta2, eps, w_l1, w_ssim,
+                 flags=0, pose_flags=0):
+    """`steps` Adam updates of each starting pose poses [N,6] on its photo_sweep loss, 2 * steps + 4 launches.  Returns
+    (poses [N,6] after the updates, loss [steps+1,N], best_loss [N], best_step int32 [N], best_pose [N,6]); `poses`
+    itself is not written."""
+    n = poses.shape[0]
+    h, w = tgt.shape[-2], tgt.shape[-1]
+    _expect(tgt, (1, 3, h, w), "tgt")
+    _expect(src, (1, 3, h, w), "src")
+    _expect(tgt_depth, (1, 1, h, w), "tgt_depth")
+    _expect(src_depth, (1, 1, h, w), "src_depth")
+    _expect(kinv, (1, 3, 3), "kinv")
+    _expect(K, (1, 3, 3), "K")
+    _expect(poses, (n, 6), "poses")
+    tgt, _, tsc = image_view(tgt, "tgt")
+    src, _, ssc = image_view(src, "src")
+    td, sd = _f32c(tgt_depth, "tgt_depth"), _f32c(src_depth, "src_depth")
+    kinv, K = _f32c(kinv, "kinv"), _f32c(K, "K")
+    out = _f32c(poses, "poses").clone()
+    dev = tgt.device
+    m = torch.empty((n, 6), dtype=torch.float32, device=dev)
+    v = torch.empty((n, 6), dtype=torch.float32, device=dev)
+    proj = torch.empty((n, 3, 4), dtype=torch.float32, device=dev)
+    scratch = torch.empty((h, w), dtype=torch.float32, device=dev)
+    partials = torch.empty((lib.tcsfm_photo_sweep_grad_partial_floats(n, h, w),), dtype=torch.float32, device=dev)
+    loss = torch.empty((steps + 1, n), dtype=torch.float32, device=dev)
+    best_loss = torch.empty((n,), dtype=torch.float32, device=dev)
+    best_step = torch.empty((n,), dtype=torch.int32, device=dev)
+    best_pose = torch.empty((n, 6), dtype=torch.float32, device=dev)
+    _call(lib, lib.tcsfm_photo_refine, "photo_refine", tgt.is_cuda,
+          _ptr(tgt), tsc, _ptr(src), ssc, _ptr(td), _ptr(sd), _ptr(kinv), _ptr(K),
+          _ptr(out), _ptr(m), _ptr(v), _ptr(proj), _ptr(scratch), _ptr(partials),
+          _ptr(loss), _ptr(best_loss), _ptr(best_step), _ptr(best_pose),
+          n, h, w, steps, lr, beta1, beta2, eps, w_l1, w_ssim, flags, pose_flags, _stream(tgt), launches=2 * steps + 4)
+    return out, loss, best_loss, best_step, best_pose
+
+
 def _ptr_table(tensors):
     arr = (C.c_void_p * len(tensors))()
     for i, t in enumerate(tensors):

@@ -592,20 +592,34 @@ photo_sweep_kernel(const __grid_constant__ SweepArgs S) {
     }
 }
 
-// sums[n] = (error_sum, valid_sum) of hypothesis n: its per-CTA partials added in tile order, the products in double
-// (one rounding to fp32 at the end), the mask counts in fp32 (exact: integers below 2^24).
+// Hypothesis hyp's per-CTA partials ([tiles][N][kParts]) added in tile order: the products E in double (the caller
+// rounds to fp32 once), the mask counts V in fp32 (exact: integers below 2^24) and, for kParts = kSweepGradParts,
+// d E / d proj in double.
+template <int kParts>
+__device__ __forceinline__ void sweep_partials_sum(const float* __restrict__ partials, int tiles, int N, int hyp, double& e,
+                                                   float& m, double (&g)[12]) {
+    e = 0.0;
+    m = 0.f;
+#pragma unroll
+    for (int i = 0; i < kParts - 2; ++i) g[i] = 0.0;
+    for (int t = 0; t < tiles; ++t) {
+        const float* p = partials + ((int64_t)t * N + hyp) * kParts;
+        e += (double)__ldg(p);
+        m = __fadd_rn(m, __ldg(p + 1));
+#pragma unroll
+        for (int i = 0; i < kParts - 2; ++i) g[i] += (double)__ldg(p + 2 + i);
+    }
+}
+
+// sums[n] = (error_sum, valid_sum) of hypothesis n from its per-CTA partials.
 constexpr int kSweepFinishThreads = 128;
 __global__ void __launch_bounds__(kSweepFinishThreads)
 photo_sweep_finish_kernel(const float* __restrict__ partials, int tiles, int N, float* __restrict__ sums) {
     const int hyp = blockIdx.x * kSweepFinishThreads + threadIdx.x;
     if (hyp >= N) return;
-    double e = 0.0;
-    float m = 0.f;
-    for (int t = 0; t < tiles; ++t) {
-        const float* p = partials + ((int64_t)t * N + hyp) * 2;
-        e += (double)__ldg(p);
-        m = __fadd_rn(m, __ldg(p + 1));
-    }
+    double e, g[12];
+    float m;
+    sweep_partials_sum<2>(partials, tiles, N, hyp, e, m, g);
     sums[2 * hyp] = (float)e;
     sums[2 * hyp + 1] = m;
 }
@@ -617,21 +631,94 @@ photo_sweep_grad_finish_kernel(const float* __restrict__ partials, int tiles, in
                                float* __restrict__ g_proj) {
     const int hyp = blockIdx.x * kSweepFinishThreads + threadIdx.x;
     if (hyp >= N) return;
-    double e = 0.0, g[12];
-    float m = 0.f;
-#pragma unroll
-    for (int i = 0; i < 12; ++i) g[i] = 0.0;
-    for (int t = 0; t < tiles; ++t) {
-        const float* p = partials + ((int64_t)t * N + hyp) * kSweepGradParts;
-        e += (double)__ldg(p);
-        m = __fadd_rn(m, __ldg(p + 1));
-#pragma unroll
-        for (int i = 0; i < 12; ++i) g[i] += (double)__ldg(p + 2 + i);
-    }
+    double e, g[12];
+    float m;
+    sweep_partials_sum<kSweepGradParts>(partials, tiles, N, hyp, e, m, g);
     sums[2 * hyp] = (float)e;
     sums[2 * hyp + 1] = m;
 #pragma unroll
     for (int i = 0; i < 12; ++i) g_proj[12 * hyp + i] = (float)(g[i] / (double)m);
+}
+
+// ---------------------------------------------------------------------------
+// Multi-start refinement: Adam on each hypothesis's pose, descending its loss surface value.  Per step the fused
+// forward + adjoint (photo_sweep_kernel<F, true>) and photo_refine_step_kernel, one thread per hypothesis, which
+// finishes the sums and the gradient like photo_sweep_grad_finish_kernel, keeps the loss history and the best
+// pose seen, maps the gradient to the pose (pose_proj_bwd_body), updates the pose and forms its next K[R|t]
+// (pose_proj_fwd_body).  Every operation of the update is a separately rounded fp32 operation, so a loop of torch
+// operators on fp32 tensors reproduces its bits.
+// ---------------------------------------------------------------------------
+struct RefineArgs {
+    const float* partials;     // [tiles][N][kSweepGradParts] (update) or [tiles][N][2] (last evaluation)
+    const float* K;            // [9]
+    float* poses;              // [N,6], updated in place
+    float* m; float* v;        // [N,6] Adam moments
+    float* proj;               // [N,12] K[R|t] of the poses, rewritten after the update
+    float* loss;               // [N]: the row of this evaluation
+    float* best_loss; int* best_step; float* best_pose;   // [N], [N], [N,6]
+    int tiles, N, step;        // step: the number of updates behind this evaluation
+};
+
+// The step's scalars, each rounded to fp32 once from double on the host.  first: the first evaluation of the call
+// (m = v = 0 and no best pose yet).
+struct AdamStep {
+    float b1, a1, b2, a2, c1, c2, e;
+    int first;
+};
+
+constexpr float kRefineSign = -1.f;       // inverse_warp2 takes -pose (compute_photometric_error, helpers.py:9)
+
+template <bool kUpdate, bool kNoFma>
+__global__ void __launch_bounds__(kSweepFinishThreads)
+photo_refine_step_kernel(const RefineArgs R, const AdamStep s) {
+    const int hyp = blockIdx.x * kSweepFinishThreads + threadIdx.x;
+    if (hyp >= R.N) return;
+    double e, g[12];
+    float V;
+    sweep_partials_sum<kUpdate ? kSweepGradParts : 2>(R.partials, R.tiles, R.N, hyp, e, V, g);
+    const float loss = __fdiv_rn((float)e, V);
+    R.loss[hyp] = loss;
+    float p[6];
+#pragma unroll
+    for (int j = 0; j < 6; ++j) p[j] = R.poses[hyp * 6 + j];
+    // best so far: the smallest finite loss, the first evaluation that reaches it
+    const int best = s.first ? -1 : R.best_step[hyp];
+    if (fabsf(loss) < INFINITY && (best < 0 || loss < R.best_loss[hyp])) {
+        R.best_loss[hyp] = loss;
+        R.best_step[hyp] = R.step;
+#pragma unroll
+        for (int j = 0; j < 6; ++j) R.best_pose[hyp * 6 + j] = p[j];
+    } else if (s.first) {
+        R.best_loss[hyp] = __int_as_float(0x7fffffff);
+        R.best_step[hyp] = -1;
+#pragma unroll
+        for (int j = 0; j < 6; ++j) R.best_pose[hyp * 6 + j] = p[j];
+    }
+    if constexpr (kUpdate) {
+        float* m = R.m + hyp * 6;
+        float* v = R.v + hyp * 6;
+        if (V > 0.f) {
+            float g_proj[12], gp[6];
+#pragma unroll
+            for (int i = 0; i < 12; ++i) g_proj[i] = (float)(g[i] / (double)V);
+            pose_proj_bwd_body(p, kRefineSign, R.K, 1, g_proj, gp, 0);
+#pragma unroll
+            for (int j = 0; j < 6; ++j) {
+                const float mj = __fadd_rn(__fmul_rn(s.b1, s.first ? 0.f : m[j]), __fmul_rn(s.a1, gp[j]));
+                const float vj = __fadd_rn(__fmul_rn(s.b2, s.first ? 0.f : v[j]), __fmul_rn(s.a2, __fmul_rn(gp[j], gp[j])));
+                const float den = __fadd_rn(__fdiv_rn(sqrtf(vj), s.c2), s.e);
+                p[j] = __fsub_rn(p[j], __fmul_rn(s.c1, __fdiv_rn(mj, den)));
+                m[j] = mj;
+                v[j] = vj;
+                R.poses[hyp * 6 + j] = p[j];
+            }
+            pose_proj_fwd_body<kNoFma>(p, kRefineSign, R.K, 1, R.proj, hyp);
+        } else if (s.first) {
+            // frozen: no valid pixel, so no gradient; the pose (and its K[R|t]) stays, the moments start at 0
+#pragma unroll
+            for (int j = 0; j < 6; ++j) { m[j] = 0.f; v[j] = 0.f; }
+        }
+    }
 }
 
 static int sweep_tiles(int H, int W) { return ((W + kTileW - 1) / kTileW) * ((H + kTileH - 1) / kTileH); }
@@ -771,5 +858,68 @@ extern "C" int tcsfm_photo_sweep_grad(const float* tgt, int64_t tgt_sc, const fl
     if (int rc = check_launch(who)) return rc;
     TCSFM_LAUNCH(photo_sweep_grad_finish_kernel, dim3((N + kSweepFinishThreads - 1) / kSweepFinishThreads), dim3(kSweepFinishThreads), 0,
                  stream, partials, tiles, N, sums, g_proj);
+    return check_launch(who);
+}
+
+extern "C" int tcsfm_photo_refine(const float* tgt, int64_t tgt_sc, const float* src, int64_t src_sc,
+                                  const float* tgt_depth, const float* src_depth, const float* kinv, const float* K,
+                                  float* poses, float* m, float* v, float* proj, float* scratch, float* partials,
+                                  float* loss, float* best_loss, int* best_step, float* best_pose,
+                                  int N, int H, int W, int steps, double lr, double beta1, double beta2, double eps,
+                                  float w_l1, float w_ssim, int flags, int pose_flags, void* stream) {
+    const char* who = "tcsfm_photo_refine";
+    if (!K || !poses || !m || !v || !best_loss || !best_step || !best_pose) { set_error("%s: null pointer", who); return 1; }
+    if (steps < 0) { set_error("%s: steps=%d is negative", who, steps); return 1; }
+    if (N > 0 && ((int64_t)steps + 1) * N > 0x7fffffff) {
+        set_error("%s: the loss history of %d steps x %d hypotheses exceeds 2^31 - 1 entries", who, steps, N); return 1;
+    }
+    if (!(lr > 0.0 && lr < INFINITY) || !(eps > 0.0 && eps < INFINITY) || !(beta1 >= 0.0 && beta1 < 1.0) ||
+        !(beta2 >= 0.0 && beta2 < 1.0)) {
+        set_error("%s: bad optimizer arguments lr=%g betas=(%g, %g) eps=%g", who, lr, beta1, beta2, eps); return 1;
+    }
+    // `loss` stands in for the sums of fill_sweep's checks: each row of it is written from the partials here
+    SweepArgs S;
+    if (int rc = fill_sweep(S, who, tgt, tgt_sc, src, src_sc, tgt_depth, src_depth, kinv, proj, scratch, partials, loss,
+                            N, H, W, w_l1, w_ssim, flags)) return rc;
+    const int tiles = S.tiles;
+    const size_t smem_fwd = 3 * Tile<1>::kCells * sizeof(float2);
+    const size_t smem = smem_fwd + kPhotoCoefPlanes * Tile<1>::kCells * sizeof(float);
+#ifndef TCSFM_HOST_EMU
+    cudaError_t e = cudaSuccess;
+    TCSFM_DISPATCH_FLAVOUR(flags, e = cudaFuncSetAttribute(photo_sweep_kernel<F, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    if (e != cudaSuccess) { set_error("%s: cannot raise dynamic smem: %s", who, cudaGetErrorString(e)); return 2; }
+#endif
+    TCSFM_DISPATCH_FLAVOUR(flags, TCSFM_LAUNCH(photo_auto_err_kernel<F>, dim3(tiles), dim3(kTileThreads), smem_fwd, stream, S.P));
+    if (int rc = check_launch(who)) return rc;
+    if (int rc = tcsfm_pose_proj_fwd(poses, kRefineSign, K, 1, proj, N, pose_flags, stream)) return rc;
+    auto* step = (pose_flags & TCSFM_ARITH_BMM_NOFMA) ? photo_refine_step_kernel<true, true> : photo_refine_step_kernel<true, false>;
+    const dim3 step_grid((N + kSweepFinishThreads - 1) / kSweepFinishThreads), step_block(kSweepFinishThreads);
+    RefineArgs R;
+    R.partials = partials; R.K = K; R.poses = poses; R.m = m; R.v = v; R.proj = proj;
+    R.best_loss = best_loss; R.best_step = best_step; R.best_pose = best_pose;
+    R.tiles = tiles; R.N = N;
+    AdamStep s;
+    s.b1 = (float)beta1; s.a1 = (float)(1.0 - beta1); s.b2 = (float)beta2; s.a2 = (float)(1.0 - beta2); s.e = (float)eps;
+    for (int t = 1; t <= steps; ++t) {
+        TCSFM_DISPATCH_FLAVOUR(flags, auto* sweep = photo_sweep_kernel<F, true>;
+                                      TCSFM_LAUNCH(sweep, dim3((unsigned)(tiles * N)), dim3(kTileThreads), smem, stream, S));
+        if (int rc = check_launch(who)) return rc;
+        s.c1 = (float)(lr / (1.0 - pow(beta1, (double)t)));
+        s.c2 = (float)sqrt(1.0 - pow(beta2, (double)t));
+        s.first = t == 1;
+        R.loss = loss + (int64_t)(t - 1) * N;
+        R.step = t - 1;
+        TCSFM_LAUNCH(step, step_grid, step_block, 0, stream, R, s);
+        if (int rc = check_launch(who)) return rc;
+    }
+    // the poses after the last update: their loss and the last chance to be the best
+    TCSFM_DISPATCH_FLAVOUR(flags, auto* sweep = photo_sweep_kernel<F, false>;
+                                  TCSFM_LAUNCH(sweep, dim3((unsigned)(tiles * N)), dim3(kTileThreads), smem_fwd, stream, S));
+    if (int rc = check_launch(who)) return rc;
+    s.first = steps == 0;
+    R.loss = loss + (int64_t)steps * N;
+    R.step = steps;
+    auto* last = photo_refine_step_kernel<false, false>;
+    TCSFM_LAUNCH(last, step_grid, step_block, 0, stream, R, s);
     return check_launch(who);
 }

@@ -5,8 +5,11 @@ helpers.py:8-23).  The optimisation driver itself (deep copies of the depth net,
 Adam, plotting; optimizer.py:136-297) is the reference's harness and calls these.
 ``photometric_loss_surface`` evaluates ``compute_photometric_error`` for N pose hypotheses of one pair in one call
 (the loss-surface plots, plot_loss_surface.py:11-87); ``photometric_loss_surface_and_grad`` also returns the pose
-gradient of every hypothesis's loss.
+gradient of every hypothesis's loss, and ``refine_pose_hypotheses`` descends the surface from every hypothesis.
 """
+import math
+import numbers
+
 import torch
 
 from . import _cabi, _raw, ops, stn
@@ -132,6 +135,63 @@ def photometric_loss_surface_and_grad(target_img, source_img, target_depth, sour
             pose_grad = torch.nn.functional.pad(pose_grad, (0, poses.shape[1] - 6))
         return {'loss': sums[:, 0] / sums[:, 1], 'error_sum': sums[:, 0], 'valid_sum': sums[:, 1],
                 'pose_grad': pose_grad}
+
+
+def refine_pose_hypotheses(target_img, source_img, target_depth, source_depth, poses, intrinsics,
+                           steps=50, lr=1e-3, betas=(0.9, 0.999), eps=1e-8):
+    """Multi-start photometric pose refinement: `steps` Adam updates of every hypothesis of photometric_loss_surface,
+    each on its own loss sum(diff_img * valid_mask * weight_mask) / sum(valid_mask), in one call.
+
+    The arguments are photometric_loss_surface's (poses [N,6] or [N,8], un-negated; columns 6: are carried through).
+    The update is Adam without weight decay, per column: for step t the scalars b1 = beta1, a1 = 1 - beta1,
+    b2 = beta2, a2 = 1 - beta2, eps, c1 = lr / (1 - beta1**t) and c2 = sqrt(1 - beta2**t) are formed in double and
+    rounded to fp32 once; with g the pose_grad photometric_loss_surface_and_grad gives at the current pose,
+        m = b1*m + a1*g;  v = b2*v + a2*(g*g);  p = p - c1*(m / (sqrt(v)/c2 + eps))
+    each operation rounded to fp32 (m = v = 0 at first).  A hypothesis with no valid pixel at its current pose is not
+    updated (its gradient is NaN), so it keeps that pose and a NaN loss from then on.
+
+    Returns {'poses': the poses after `steps` updates, 'loss': [steps+1, N] (row k at the poses after k updates),
+    'best_loss': [N] the smallest finite loss of each column (NaN if none), 'best_step': [N] int64 the first row that
+    reaches it (-1 if none), 'best_pose': the pose there (the starting pose if none)}.
+
+    Functional, not autograd: no graph is recorded, inputs that require grad are read as values and `poses` is not
+    written.  2 * steps + 6 launches for [N,6] poses: K^-1, the 2 * steps + 4 of tcsfm_photo_refine (the auto-mask
+    error, K[R|t] of the starting poses, per step the fused forward + adjoint and the update, then the last
+    evaluation) and best_step's int64 copy; [N,8] poses add two for their columns 6:.  No host work between the
+    steps, the same bits on every call, and capturable in a CUDA graph."""
+    ops._require_cuda(target_img, source_img, target_depth, source_depth, poses, intrinsics)
+    _check_surface_args(target_img, poses)
+    steps, lr, beta1, beta2, eps = _check_adam_args(steps, lr, betas, eps)
+    h, w = target_img.shape[2], target_img.shape[3]
+    with torch.no_grad(), ops._guard(poses):
+        kinv = stn.inverse_intrinsics(intrinsics)
+        final, loss, best_loss, best_step, best_pose = _raw.photo_refine(
+            ops.lib(), target_img, source_img, target_depth, source_depth, kinv, intrinsics, poses[:, 0:6], steps, lr,
+            beta1, beta2, eps, 0.15, 0.85, ops.arith_flags(1, h, w), ops.pose_flags(1))
+        if poses.shape[1] > 6:
+            final = torch.cat([final, poses[:, 6:]], 1)
+            best_pose = torch.cat([best_pose, poses[:, 6:]], 1)
+        return {'poses': final, 'loss': loss, 'best_loss': best_loss, 'best_step': best_step.long(),
+                'best_pose': best_pose}
+
+
+def _check_adam_args(steps, lr, betas, eps):
+    """(steps, lr, beta1, beta2, eps) as int and floats, or ValueError."""
+    if isinstance(steps, bool) or not isinstance(steps, numbers.Integral) or steps < 0:
+        raise ValueError("refine_pose_hypotheses: steps must be an int >= 0, got %r" % (steps,))
+    try:
+        lr, eps = float(lr), float(eps)
+        beta1, beta2 = (float(b) for b in betas)
+    except (TypeError, ValueError):
+        raise ValueError("refine_pose_hypotheses: lr and eps must be numbers and betas a pair of numbers, got lr=%r "
+                         "betas=%r eps=%r" % (lr, betas, eps)) from None
+    for name, x in (("lr", lr), ("eps", eps)):
+        if not (math.isfinite(x) and x > 0):
+            raise ValueError("refine_pose_hypotheses: %s must be finite and > 0, got %r" % (name, x))
+    for x in (beta1, beta2):
+        if not 0.0 <= x < 1.0:
+            raise ValueError("refine_pose_hypotheses: each beta must be in [0, 1), got %r" % (betas,))
+    return int(steps), lr, beta1, beta2, eps
 
 
 def _check_surface_args(target_img, poses):

@@ -10,6 +10,17 @@ and, for the pose gradient of every sample (the "grad" section):
          .backward(), then pose.grad;
   batch  one pft.photometric_loss_surface_and_grad call over all samples (loss and pose_grad).
 
+and, for multi-start refinement, `--refine-steps` Adam steps from every sample (the "refine" section):
+
+  loop   what a user writes with the surface functions: per step pft.photometric_loss_surface_and_grad and
+         torch.optim.Adam (defaults) on an [N,6] leaf, the NaN gradients of samples with no valid pixel zeroed, then
+         one pft.photometric_loss_surface for the final loss;
+  batch  one pft.refine_pose_hypotheses call (the loss history).
+
+The refine section runs N = 8, 100 (the demo's) and 200 (bench.py's); both ways end with the D2H copy of the
+[steps+1, N] loss history.  The two do not give the same bits (torch's Adam rounds differently), so no difference is
+reported for them.
+
 Input: what `bench.py --workload sweep` evaluates, make_frames(1, 192, 640, n_src=2, seed=0, KITTI intrinsics) with a
 line of forward-translation (pose column 2) and a line of yaw (column 4) samples, linspace(-0.05, 0.05, n) each:
 n = 100 (bench.py's default --sweep-evals, N = 200) and n = 50 (the demo's, N = 100).  Both are timed like
@@ -17,7 +28,7 @@ main_sweep: wall clock of a whole sweep including the final device-to-host copy,
 alternated round by round.  The batched op's device time per call comes from CUDA events around `--device-iters`
 back-to-back calls, next to the forward-only call's in the grad section.  The working set (one frame pair, ~2.5 MB) stays in L2, so no HBM roofline fraction is claimed.
 
-Usage: python tools/bench_photo_sweep.py [--rounds R] [--device-iters I]"""
+Usage: python tools/bench_photo_sweep.py [--rounds R] [--device-iters I] [--refine-steps S] [--refine-iters J]"""
 import argparse
 import json
 import os
@@ -182,10 +193,67 @@ def measure_grad(fr, n, rounds, device_iters):
             "max_rel_diff_pose_grad": rel}
 
 
+def measure_refine(fr, n, rounds, steps, device_iters):
+    args = (fr["target"], fr["sources"][0], fr["depths"][0], fr["depths"][1])
+    deltas = torch.linspace(-0.05, 0.05, n, device=fr["K"].device)
+    start = fr["poses"][0].repeat(2 * n, 1)
+    start[:n, 2] += deltas
+    start[n:, 4] += deltas
+
+    def loop():
+        leaf = start.clone().requires_grad_(True)
+        opt = torch.optim.Adam([leaf], lr=1e-3)
+        rows = []
+        for _ in range(steps):
+            r = pft.photometric_loss_surface_and_grad(*args, leaf, fr["K"])
+            rows.append(r["loss"])
+            leaf.grad = torch.where((r["valid_sum"] > 0)[:, None], r["pose_grad"], 0.0)
+            opt.step()
+        rows.append(pft.photometric_loss_surface(*args, leaf.detach(), fr["K"])["loss"])
+        return torch.stack(rows)
+
+    def batch():
+        return pft.refine_pose_hypotheses(*args, start, fr["K"], steps=steps)["loss"]
+
+    def timed(fn):
+        torch.cuda.synchronize()
+        t0 = time.perf_counter()
+        fn().cpu()
+        return time.perf_counter() - t0
+
+    loop(), batch()                                 # warm-up descents
+    t_loop, t_batch = [], []
+    for _ in range(rounds):
+        t_loop.append(timed(loop))
+        t_batch.append(timed(batch))
+    with torch.no_grad():
+        for _ in range(2):
+            batch()
+        torch.cuda.synchronize()
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record()
+        for _ in range(device_iters):
+            batch()
+        e1.record()
+        torch.cuda.synchronize()
+    ms_call = e0.elapsed_time(e1) / device_iters
+    return {"N": 2 * n, "steps": steps,
+            "loop_ms_per_descent": round(statistics.median(t_loop) * 1e3, 3),
+            "batch_ms_per_descent": round(statistics.median(t_batch) * 1e3, 3),
+            "speedup": round(statistics.median(t_loop) / statistics.median(t_batch), 2),
+            "loop_ms_rounds": [round(t * 1e3, 3) for t in t_loop],
+            "batch_ms_rounds": [round(t * 1e3, 3) for t in t_batch],
+            "batch_device_ms_per_call": round(ms_call, 4),
+            "batch_device_ms_per_step": round(ms_call / (steps + 1), 4),
+            "device_calls_timed": device_iters}
+
+
 def main():
     ap = argparse.ArgumentParser(description=__doc__.splitlines()[0])
     ap.add_argument("--rounds", type=int, default=5, help="alternated loop / batch sweeps per configuration")
     ap.add_argument("--device-iters", type=int, default=200, help="back-to-back calls timed with CUDA events")
+    ap.add_argument("--refine-steps", type=int, default=50, help="Adam steps per descent in the refine section")
+    ap.add_argument("--refine-iters", type=int, default=20, help="back-to-back refine calls timed with CUDA events")
     args = ap.parse_args()
     if not torch.cuda.is_available():
         sys.exit("bench_photo_sweep.py needs a CUDA device")
@@ -204,7 +272,11 @@ def main():
                                "vs one photometric_loss_surface_and_grad call",
                      "max_rel_diff": "largest |pose_grad - loop| / |loop| over the rows",
                      "configs": {"bench_sweep_default_100x2": measure_grad(fr, 100, args.rounds, args.device_iters),
-                                 "demo_50x2": measure_grad(fr, 50, args.rounds, args.device_iters)}}}
+                                 "demo_50x2": measure_grad(fr, 50, args.rounds, args.device_iters)}},
+            "refine": {"metric": "multi-start refinement, ms per descent of N starts: the surface_and_grad + "
+                                 "torch.optim.Adam loop vs one refine_pose_hypotheses call",
+                       "configs": {"N%d" % (2 * n): measure_refine(fr, n, args.rounds, args.refine_steps, args.refine_iters)
+                                   for n in (4, 50, 100)}}}
     print(json.dumps(line))
 
 
