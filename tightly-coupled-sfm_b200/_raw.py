@@ -431,22 +431,31 @@ def photo_bwd(lib, tgt, rec, proj_depth, comp_depth, coef, g_diff, g_weight, w_l
     return g_rec, g_pd, g_cd
 
 
-def photo_sweep(lib, tgt, src, tgt_depth, src_depth, kinv, proj, w_l1, w_ssim, flags=0, want_maps=False):
-    """compute_photometric_error of ONE pair (tgt / src [1,3,H,W] views, depths [1,1,H,W], kinv [1,3,3]) under each of
-    the N projections proj [N,3,4], three launches.  Returns (sums [N,2] = (sum(diff * mask * weight), sum(mask)),
-    maps) with maps = (rec [N,3,H,W], diff, mask, weight [N,1,H,W]) when `want_maps`, else None."""
-    n = proj.shape[0]
+def _single_pair(tgt, src, tgt_depth, src_depth, kinv, *expect):
+    """Checks and marshals the one frame pair of the photo_sweep family: tgt / src [1,3,H,W] views, depths [1,1,H,W]
+    and kinv [1,3,3].  `expect` holds (tensor, shape, name) checks of the caller's other arguments, made after these
+    and before any conversion.  Returns (tgt, its channel stride, src, its channel stride, tgt_depth, src_depth, kinv)."""
     h, w = tgt.shape[-2], tgt.shape[-1]
     _expect(tgt, (1, 3, h, w), "tgt")
     _expect(src, (1, 3, h, w), "src")
     _expect(tgt_depth, (1, 1, h, w), "tgt_depth")
     _expect(src_depth, (1, 1, h, w), "src_depth")
     _expect(kinv, (1, 3, 3), "kinv")
-    _expect(proj, (n, 3, 4), "proj")
+    for t, shape, name in expect:
+        _expect(t, shape, name)
     tgt, _, tsc = image_view(tgt, "tgt")
     src, _, ssc = image_view(src, "src")
-    td, sd = _f32c(tgt_depth, "tgt_depth"), _f32c(src_depth, "src_depth")
-    kinv, proj = _f32c(kinv, "kinv"), _f32c(proj, "proj")
+    return (tgt, tsc, src, ssc, _f32c(tgt_depth, "tgt_depth"), _f32c(src_depth, "src_depth"), _f32c(kinv, "kinv"))
+
+
+def photo_sweep(lib, tgt, src, tgt_depth, src_depth, kinv, proj, w_l1, w_ssim, flags=0, want_maps=False):
+    """compute_photometric_error of ONE pair (tgt / src [1,3,H,W] views, depths [1,1,H,W], kinv [1,3,3]) under each of
+    the N projections proj [N,3,4], three launches.  Returns (sums [N,2] = (sum(diff * mask * weight), sum(mask)),
+    maps) with maps = (rec [N,3,H,W], diff, mask, weight [N,1,H,W]) when `want_maps`, else None."""
+    n = proj.shape[0]
+    h, w = tgt.shape[-2], tgt.shape[-1]
+    tgt, tsc, src, ssc, td, sd, kinv = _single_pair(tgt, src, tgt_depth, src_depth, kinv, (proj, (n, 3, 4), "proj"))
+    proj = _f32c(proj, "proj")
     dev = tgt.device
     scratch = torch.empty((h, w), dtype=torch.float32, device=dev)
     partials = torch.empty((lib.tcsfm_photo_sweep_partial_floats(n, h, w),), dtype=torch.float32, device=dev)
@@ -467,16 +476,8 @@ def photo_sweep_grad(lib, tgt, src, tgt_depth, src_depth, kinv, proj, w_l1, w_ss
     """photo_sweep's sums plus g_proj [N,3,4] = d (sums[n,0] / sums[n,1]) / d proj[n], three launches."""
     n = proj.shape[0]
     h, w = tgt.shape[-2], tgt.shape[-1]
-    _expect(tgt, (1, 3, h, w), "tgt")
-    _expect(src, (1, 3, h, w), "src")
-    _expect(tgt_depth, (1, 1, h, w), "tgt_depth")
-    _expect(src_depth, (1, 1, h, w), "src_depth")
-    _expect(kinv, (1, 3, 3), "kinv")
-    _expect(proj, (n, 3, 4), "proj")
-    tgt, _, tsc = image_view(tgt, "tgt")
-    src, _, ssc = image_view(src, "src")
-    td, sd = _f32c(tgt_depth, "tgt_depth"), _f32c(src_depth, "src_depth")
-    kinv, proj = _f32c(kinv, "kinv"), _f32c(proj, "proj")
+    tgt, tsc, src, ssc, td, sd, kinv = _single_pair(tgt, src, tgt_depth, src_depth, kinv, (proj, (n, 3, 4), "proj"))
+    proj = _f32c(proj, "proj")
     dev = tgt.device
     scratch = torch.empty((h, w), dtype=torch.float32, device=dev)
     partials = torch.empty((lib.tcsfm_photo_sweep_grad_partial_floats(n, h, w),), dtype=torch.float32, device=dev)
@@ -496,17 +497,9 @@ def photo_refine(lib, tgt, src, tgt_depth, src_depth, kinv, K, poses, steps, lr,
     itself is not written."""
     n = poses.shape[0]
     h, w = tgt.shape[-2], tgt.shape[-1]
-    _expect(tgt, (1, 3, h, w), "tgt")
-    _expect(src, (1, 3, h, w), "src")
-    _expect(tgt_depth, (1, 1, h, w), "tgt_depth")
-    _expect(src_depth, (1, 1, h, w), "src_depth")
-    _expect(kinv, (1, 3, 3), "kinv")
-    _expect(K, (1, 3, 3), "K")
-    _expect(poses, (n, 6), "poses")
-    tgt, _, tsc = image_view(tgt, "tgt")
-    src, _, ssc = image_view(src, "src")
-    td, sd = _f32c(tgt_depth, "tgt_depth"), _f32c(src_depth, "src_depth")
-    kinv, K = _f32c(kinv, "kinv"), _f32c(K, "K")
+    tgt, tsc, src, ssc, td, sd, kinv = _single_pair(tgt, src, tgt_depth, src_depth, kinv,
+                                                    (K, (1, 3, 3), "K"), (poses, (n, 6), "poses"))
+    K = _f32c(K, "K")
     out = _f32c(poses, "poses").clone()
     dev = tgt.device
     m = torch.empty((n, 6), dtype=torch.float32, device=dev)

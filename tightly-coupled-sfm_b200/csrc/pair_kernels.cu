@@ -78,39 +78,6 @@ __device__ __forceinline__ PairCtx make_ctx(const tcsfm_pair_group& g, int b, in
     return c;
 }
 
-// Fills one shared-memory cell with (target, warped source) of the image pixel (rx, ry);
-// returns the validity of the warp and, when asked, the depth inconsistency at that pixel.
-template <int F>
-__device__ __forceinline__ void fill_cell(const PairCtx& c, const Cam& cam, const Arith& A, int rx, int ry,
-                                          float depth, float2* tw, int cells, int cell, bool want_dd,
-                                          bool& valid, float& dd) {
-    const int pix = ry * A.W + rx;
-    WarpPt p;
-    warp_point<F>(cam, A, rx, ry, depth, p);
-    const TapIdx ti = make_taps(p, A.H, A.W);
-#pragma unroll
-    for (int ch = 0; ch < 3; ++ch) {
-        const float w = blend(load_taps(c.ref, ch * c.ref_sc, ti, A.W), ti);
-        tw[ch * cells + cell] = make_float2(__ldg(c.tgt + (ch * c.tgt_sc + pix)), w);
-    }
-    valid = p.valid;
-    dd = want_dd ? depth_inconsistency(p.Z, blend(load_taps(c.rdep, 0, ti, A.W), ti)) : 0.f;
-}
-
-__device__ __forceinline__ void zero_cell(float2* tw, int cells, int cell) {
-#pragma unroll
-    for (int ch = 0; ch < 3; ++ch) tw[ch * cells + cell] = make_float2(0.f, 0.f);
-}
-
-// The halo ring of a Tile<1>, enumerated 0 .. 2*(kTileW+2) + 2*kTileH - 1.
-constexpr int kRingCells = 2 * (kTileW + 2) + 2 * kTileH;
-__device__ __forceinline__ void ring_cell(int r, int& cx, int& cy) {
-    if (r < kTileW + 2) { cx = r - 1; cy = -1; }
-    else if (r < 2 * (kTileW + 2)) { cx = r - (kTileW + 2) - 1; cy = kTileH; }
-    else if (r < 2 * (kTileW + 2) + kTileH) { cx = -1; cy = r - 2 * (kTileW + 2); }
-    else { cx = kTileW; cy = r - 2 * (kTileW + 2) - kTileH; }
-}
-
 template <int F>
 __global__ void __launch_bounds__(kTileThreads, TCSFM_FWD_MIN_BLOCKS)
 pair_fwd_kernel(const __grid_constant__ PairLaunch L) {
@@ -122,9 +89,8 @@ pair_fwd_kernel(const __grid_constant__ PairLaunch L) {
     const Arith& A = L.A;
     const int H = A.H, W = A.W, n = H * W;
     const int b = blockIdx.y;
-    const int tiles_x = (W + kTileW - 1) / kTileW;
-    const int tile_y = blockIdx.x / tiles_x, tile_x = blockIdx.x - tile_y * tiles_x;
-    const int x0 = tile_x * kTileW, y0 = tile_y * kTileH;
+    int x0, y0;
+    tile_origin(blockIdx.x, W, x0, y0);
     const Cam cam = load_cam(g.kinv, g.proj, b);
     const PairCtx c = make_ctx(g, b, n);
     const bool auto_mask = (L.flags & TCSFM_AUTO_MASK) != 0;
@@ -217,10 +183,9 @@ pair_fwd_kernel(const __grid_constant__ PairLaunch L) {
     }
     // ---- phase A': the halo ring (one cell per thread) ----
     if (threadIdx.x < kRingCells) {
-        bool valid;
-        float dd;
-        if (ring_ok) fill_cell<F>(c, cam, A, ring_x, ring_y, ring_depth, tw, T1::kCells, ring_at, false, valid, dd);
-        else zero_cell(tw, T1::kCells, ring_at);
+        WarpPt p;
+        if (ring_ok) fill_warped_cell<F>(cam, A, c.tgt, c.tgt_sc, c.ref, c.ref_sc, ring_x, ring_y, ring_depth, tw, ring_at, p);
+        else zero_cell(tw, ring_at);
     }
     __syncthreads();
 
@@ -229,32 +194,8 @@ pair_fwd_kernel(const __grid_constant__ PairLaunch L) {
     float* coef_base = pin_pointer(g.coef ? g.coef + (int64_t)b * kCoefPlanes * n : nullptr);   // offsets below: < 2^31 (fill_launch)
 #pragma unroll
     for (int ch = 0; ch < 3; ++ch) {
-        const float2* plane = tw + ch * T1::kCells;
-        // rolling 3-row window of (target, warped) taps; squares / products are formed per use
-        // (cheaper than keeping 27 more registers live across the strip)
-        float2 v[3][3];
-#pragma unroll
-        for (int r = 0; r < 2; ++r)
-#pragma unroll
-            for (int cc = 0; cc < 3; ++cc) v[r][cc] = plane[T1::cell(tx - 1 + cc, ty0 - 1 + r)];
-#pragma unroll
-        for (int k = 0; k < kPixPerThread; ++k) {
-#pragma unroll
-            for (int cc = 0; cc < 3; ++cc) v[(k + 2) % 3][cc] = plane[T1::cell(tx - 1 + cc, ty0 + 1 + k)];
-            float2 wv[9], wsq[9];
-            float wab[9];
-#pragma unroll
-            for (int i = 0; i < 9; ++i) {
-                wv[i] = v[(k + i / 3) % 3][i % 3];
-                wsq[i] = square2_rn(wv[i]);
-                wab[i] = __fmul_rn(wv[i].x, wv[i].y);
-            }
-            const SsimStats s = ssim_stats_packed(wv, wsq, wab);
-            const SsimTerms t = ssim_terms(s, L.C1, L.C2);
-            const float2 ctr = wv[4];
-            const float l1 = clamp01_nan(fabsf(__fsub_rn(ctr.x, ctr.y)));
-            const float e = __fadd_rn(__fmul_rn(l1, L.w_l1), __fmul_rn(clamp01_nan(t.raw), L.w_ssim));
-            esum[k] = (ch == 0) ? e : __fadd_rn(esum[k], e);
+        ssim_l1_strip(tw + ch * T1::kCells, tx, ty0, L, ch == 0, esum,
+                      [&](int k, const SsimStats& s, const SsimTerms& t) {
             const int gy = y0 + ty0 + k;
             if (coef_base && gx < W && gy < H) {
                 // d diff / d ssim_c = (1 - dd) * (1/3) * w_ssim ; the backward multiplies by its upstream
@@ -265,7 +206,7 @@ pair_fwd_kernel(const __grid_constant__ PairLaunch L) {
                 store_streaming(coef_base + (o + n), kf.B);
                 store_streaming(coef_base + (o + 2 * n), kf.Cc);
             }
-        }
+        });
     }
     float part[3] = {0.f, 0.f, 0.f};
 #pragma unroll
@@ -421,9 +362,8 @@ pair_bwd_kernel(const __grid_constant__ PairLaunch L) {
     const Arith& A = L.A;
     const int H = A.H, W = A.W, n = H * W;
     const int b = blockIdx.y;
-    const int tiles_x = (W + kTileW - 1) / kTileW;
-    const int tile_y = blockIdx.x / tiles_x, tile_x = blockIdx.x - tile_y * tiles_x;
-    const int x0 = tile_x * kTileW, y0 = tile_y * kTileH;
+    int x0, y0;
+    tile_origin(blockIdx.x, W, x0, y0);
     const Cam cam = load_cam(g.kinv, g.proj, b);
     const PairCtx c = make_ctx(g, b, n);
     const bool depth_mask = (L.flags & TCSFM_DEPTH_MASK) != 0;
@@ -898,7 +838,7 @@ static int fill_launch(PairLaunch& L, const tcsfm_pair_group* groups, int n, int
     }
     L.A = make_arith(H, W, flags);
     L.w_l1 = w_l1; L.w_ssim = w_ssim;
-    L.C1 = (float)(0.01 * 0.01); L.C2 = (float)(0.03 * 0.03);
+    L.C1 = kSsimC1; L.C2 = kSsimC2;
     L.flags = flags;
     return 0;
 }
@@ -918,7 +858,7 @@ extern "C" int tcsfm_pair_loss_fwd(const tcsfm_pair_group* groups, int n_groups,
     if (!groups || n_groups <= 0) { set_error("tcsfm_pair_loss_fwd: no groups"); return 1; }
     if (flags & TCSFM_ARITH_FAST) return tcsfm_pair_fast_fwd(groups, n_groups, B, H, W, w_l1, w_ssim, flags, stream);
     const size_t smem = 3 * Tile<1>::kCells * sizeof(float2);
-    const int tiles = ((W + kTileW - 1) / kTileW) * ((H + kTileH - 1) / kTileH);
+    const int tiles = tile_count(H, W);
     for (int base = 0; base < n_groups; base += kMaxGroups) {
         const int n = (n_groups - base < kMaxGroups) ? n_groups - base : kMaxGroups;
         PairLaunch L;
@@ -942,7 +882,7 @@ extern "C" int tcsfm_pair_loss_bwd(const tcsfm_pair_group* groups, int n_groups,
                                    float w_l1, float w_ssim, int flags, void* stream) {
     if (!groups || n_groups <= 0) { set_error("tcsfm_pair_loss_bwd: no groups"); return 1; }
     const size_t smem = kBwdSmemBytes;
-    const int tiles = ((W + kTileW - 1) / kTileW) * ((H + kTileH - 1) / kTileH);
+    const int tiles = tile_count(H, W);
     for (int base = 0; base < n_groups; base += kMaxGroups) {
         const int n = (n_groups - base < kMaxGroups) ? n_groups - base : kMaxGroups;
         PairLaunch L;

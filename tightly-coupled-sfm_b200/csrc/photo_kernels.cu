@@ -30,49 +30,14 @@ struct PhotoArgs {
     float w_l1, w_ssim, C1, C2;
 };
 
-// one channel of  w_l1 * clamp|x - y| + w_ssim * SSIM(x, y)  down a strip, x/y packed as float2.
-// kCoef: the SSIM adjoint coefficients (Ay, B, Cc) of each pixel go to the [N,9,H,W] workspace planes at coef_ch;
-// kTileCoef: to the Tile<1> planes at coef_ch (plane stride kCells), at the strip's own cells, filler cells included.
-template <bool kCoef, bool kTileCoef = false>
-__device__ __forceinline__ void strip_channel(const float2* plane, int tx, int ty0, const PhotoArgs& P, bool first,
-                                              float (&esum)[kPixPerThread], float* coef_ch, int gx, int gy0, int n) {
-    using T1 = Tile<1>;
-    float2 v[3][3];
-#pragma unroll
-    for (int r = 0; r < 2; ++r)
-#pragma unroll
-        for (int cc = 0; cc < 3; ++cc) v[r][cc] = plane[T1::cell(tx - 1 + cc, ty0 - 1 + r)];
-#pragma unroll
-    for (int k = 0; k < kPixPerThread; ++k) {
-#pragma unroll
-        for (int cc = 0; cc < 3; ++cc) v[(k + 2) % 3][cc] = plane[T1::cell(tx - 1 + cc, ty0 + 1 + k)];
-        float2 wv[9], wsq[9];
-        float wab[9];
-#pragma unroll
-        for (int i = 0; i < 9; ++i) {
-            wv[i] = v[(k + i / 3) % 3][i % 3];
-            wsq[i] = square2_rn(wv[i]);
-            wab[i] = __fmul_rn(wv[i].x, wv[i].y);
-        }
-        const SsimStats s = ssim_stats_packed(wv, wsq, wab);
-        const SsimTerms t = ssim_terms(s, P.C1, P.C2);
-        const float l1 = clamp01_nan(fabsf(__fsub_rn(wv[4].x, wv[4].y)));
-        const float e = __fadd_rn(__fmul_rn(l1, P.w_l1), __fmul_rn(clamp01_nan(t.raw), P.w_ssim));
-        esum[k] = first ? e : __fadd_rn(esum[k], e);
-        if (kCoef) {
-            const int gy = gy0 + k;
-            if (coef_ch && gx < P.A.W && gy < P.A.H) {
-                const SsimCoef kf = ssim_coef(s, t, P.A.third * P.w_ssim);     // x = target, y = reconstruction
-                float* cp = coef_ch + gy * P.A.W + gx;
-                cp[0] = kf.Ay; cp[n] = kf.B; cp[2 * (int64_t)n] = kf.Cc;
-            }
-        }
-        if (kTileCoef) {
-            const SsimCoef kf = ssim_coef(s, t, P.A.third * P.w_ssim);
-            float* cp = coef_ch + T1::cell(tx, ty0 + k);
-            cp[0] = kf.Ay; cp[T1::kCells] = kf.B; cp[2 * T1::kCells] = kf.Cc;
-        }
-    }
+// d E / d w of one channel's reconstructed value w at a cell with target t, from the 3x3 sums V0, V1, V2 of the
+// SSIM adjoint coefficients (Ay, B, Cc) of the windows that read the cell: V0 + 2 w V1 + t V2, plus the sign term of
+// the L1 adjoint `gl1` where |t - w| <= 1 (0 at cells that are no own pixel).
+__device__ __forceinline__ float rec_adjoint(float V0, float V1, float V2, float t, float w, float gl1) {
+    const float dlt = t - w;
+    float g = V0 + 2.0f * w * V1 + t * V2;
+    if (fabsf(dlt) <= 1.0f) g += (dlt > 0.f) ? -gl1 : ((dlt < 0.f) ? gl1 : 0.f);
+    return g;
 }
 
 template <int F>
@@ -84,9 +49,8 @@ photo_fwd_kernel(const __grid_constant__ PhotoArgs P) {
     const Arith& A = P.A;
     const int H = A.H, W = A.W, n = H * W;
     const int b = blockIdx.y;
-    const int tiles_x = (W + kTileW - 1) / kTileW;
-    const int tile_y = blockIdx.x / tiles_x, tile_x = blockIdx.x - tile_y * tiles_x;
-    const int x0 = tile_x * kTileW, y0 = tile_y * kTileH;
+    int x0, y0;
+    tile_origin(blockIdx.x, W, x0, y0);
     const float* tgt = P.tgt + b * P.tgt_sb;
     const float* src = P.src + b * P.src_sb;
     const float* rec = P.rec + (int64_t)b * 3 * n;
@@ -130,8 +94,18 @@ photo_fwd_kernel(const __grid_constant__ PhotoArgs P) {
     float* coef_b = P.coef ? P.coef + (int64_t)b * kPhotoCoefPlanes * n : nullptr;
 #pragma unroll
     for (int ch = 0; ch < 3; ++ch) {
-        strip_channel<true>(tr + ch * T1::kCells, tx, ty0, P, ch == 0, e_rec, coef_b ? coef_b + (int64_t)3 * ch * n : nullptr, gx, gy0, n);
-        strip_channel<false>(tsrc + ch * T1::kCells, tx, ty0, P, ch == 0, e_src, nullptr, gx, gy0, n);
+        // coef_ch captured by value and the bounds read from P: in this form the kernel keeps the SASS of its former
+        // own strip loop (other forms were scheduled differently, one of them measured 1 % slower)
+        ssim_l1_strip(tr + ch * T1::kCells, tx, ty0, P, ch == 0, e_rec,
+                      [&, coef_ch = coef_b ? coef_b + (int64_t)3 * ch * n : nullptr](int k, const SsimStats& s, const SsimTerms& t) {
+            const int gy = gy0 + k;
+            if (coef_ch && gx < P.A.W && gy < P.A.H) {
+                const SsimCoef kf = ssim_coef(s, t, P.A.third * P.w_ssim);     // x = target, y = reconstruction
+                float* cp = coef_ch + gy * P.A.W + gx;
+                cp[0] = kf.Ay; cp[n] = kf.B; cp[2 * (int64_t)n] = kf.Cc;
+            }
+        });
+        ssim_l1_strip(tsrc + ch * T1::kCells, tx, ty0, P, ch == 0, e_src, NoSsimSink());
     }
 #pragma unroll
     for (int k = 0; k < kPixPerThread; ++k) {
@@ -155,9 +129,8 @@ photo_bwd_kernel(const __grid_constant__ PhotoArgs P) {
     const Arith& A = P.A;
     const int H = A.H, W = A.W, n = H * W;
     const int b = blockIdx.y;
-    const int tiles_x = (W + kTileW - 1) / kTileW;
-    const int tile_y = blockIdx.x / tiles_x, tile_x = blockIdx.x - tile_y * tiles_x;
-    const int x0 = tile_x * kTileW, y0 = tile_y * kTileH;
+    int x0, y0;
+    tile_origin(blockIdx.x, W, x0, y0);
     const float* gdiff = P.g_diff ? P.g_diff + (int64_t)b * n : nullptr;
     const float* coef = P.coef + (int64_t)b * kPhotoCoefPlanes * n;
     // two cells per sweep: the twenty loads of both are in flight before the first product is stored
@@ -246,10 +219,7 @@ photo_bwd_kernel(const __grid_constant__ PhotoArgs P) {
                     if (dup_d) s += h[(k + 2) % 3][q];
                     V[j] = s;
                 }
-                const float t = tq[k][ch], w = wq[k][ch];
-                const float dlt = t - w;
-                float gw = V[0] + 2.0f * w * V[1] + t * V[2];
-                if (fabsf(dlt) <= 1.0f) gw += (dlt > 0.f) ? -gl1 : ((dlt < 0.f) ? gl1 : 0.f);
+                const float gw = rec_adjoint(V[0], V[1], V[2], tq[k][ch], wq[k][ch], gl1);
                 if (P.g_rec) P.g_rec[((int64_t)b * 3 + ch) * n + pix] = gw;
             }
             if (P.g_pd || P.g_cd) {
@@ -285,6 +255,7 @@ photo_auto_err_kernel(const __grid_constant__ PhotoArgs P) {
     using T1 = Tile<1>;
     TCSFM_DYN_SMEM(float2, ts);                                  // [3][cells] (target, src)
     const int H = P.A.H, W = P.A.W;
+    // tile_origin spelled out: with the call, ptxas schedules this kernel differently (measured 0.6 % slower)
     const int tiles_x = (W + kTileW - 1) / kTileW;
     const int tile_y = blockIdx.x / tiles_x, tile_x = blockIdx.x - tile_y * tiles_x;
     const int x0 = tile_x * kTileW, y0 = tile_y * kTileH;
@@ -303,38 +274,12 @@ photo_auto_err_kernel(const __grid_constant__ PhotoArgs P) {
     const int gx = x0 + tx;
     float e[kPixPerThread];
 #pragma unroll
-    for (int ch = 0; ch < 3; ++ch) strip_channel<false>(ts + ch * T1::kCells, tx, ty0, P, ch == 0, e, nullptr, gx, y0 + ty0, 0);
+    for (int ch = 0; ch < 3; ++ch) ssim_l1_strip(ts + ch * T1::kCells, tx, ty0, P, ch == 0, e, NoSsimSink());
 #pragma unroll
     for (int k = 0; k < kPixPerThread; ++k) {
         const int gy = y0 + ty0 + k;
         if (gx < W && gy < H) P.auto_err[gy * W + gx] = mean3_of_sum<F>(e[k], P.A);
     }
-}
-
-// Fills one cell of the (target, warped source) tile with the image pixel (rx, ry) under the camera `cam`, exactly as
-// warp_fwd_kernel forms projected_img there; returns the warp and its taps.
-template <int F>
-__device__ __forceinline__ TapIdx sweep_fill_cell(const SweepArgs& S, const Cam& cam, int rx, int ry, float2* tw, int cell,
-                                                  WarpPt& p) {
-    const Arith& A = S.P.A;
-    const int pix = ry * A.W + rx;
-    warp_point<F>(cam, A, rx, ry, __ldg(S.tdep + pix), p);
-    const TapIdx ti = make_taps(p, A.H, A.W);
-#pragma unroll
-    for (int ch = 0; ch < 3; ++ch) {
-        const float w = blend(load_taps(S.P.src, (int)(ch * S.P.src_sc), ti, A.W), ti);
-        tw[ch * Tile<1>::kCells + cell] = make_float2(__ldg(S.P.tgt + (ch * S.P.tgt_sc + pix)), w);
-    }
-    return ti;
-}
-
-// The halo ring of a Tile<1>, enumerated 0 .. kSweepRingCells - 1 (top row, bottom row, left column, right column).
-constexpr int kSweepRingCells = 2 * (kTileW + 2) + 2 * kTileH;
-__device__ __forceinline__ void sweep_ring_cell(int r, int& cx, int& cy) {
-    if (r < kTileW + 2) { cx = r - 1; cy = -1; }
-    else if (r < 2 * (kTileW + 2)) { cx = r - (kTileW + 2) - 1; cy = kTileH; }
-    else if (r < 2 * (kTileW + 2) + kTileH) { cx = -1; cy = r - 2 * (kTileW + 2); }
-    else { cx = kTileW; cy = r - 2 * (kTileW + 2) - kTileH; }
 }
 
 // ---------------------------------------------------------------------------
@@ -401,9 +346,9 @@ __device__ __forceinline__ void sweep_tile_adjoint(const SweepArgs& S, const Cam
 #pragma unroll
         for (int j = 0; j < kPhotoCoefPlanes; ++j) cs[j * T1::kCells + c] = (m[k] != 0.f) ? cs[j * T1::kCells + c] * u : 0.f;
     }
-    if (threadIdx.x < kSweepRingCells) {
+    if (threadIdx.x < kRingCells) {
         int cx, cy;
-        sweep_ring_cell(threadIdx.x, cx, cy);
+        ring_cell(threadIdx.x, cx, cy);
 #pragma unroll
         for (int j = 0; j < kPhotoCoefPlanes; ++j) cs[j * T1::kCells + T1::cell(cx, cy)] = 0.f;
     }
@@ -442,19 +387,16 @@ __device__ __forceinline__ void sweep_tile_adjoint(const SweepArgs& S, const Cam
                 V[j] = (h[k % 3][q] + h[(k + 1) % 3][q]) + h[(k + 2) % 3][q];
             }
             const float2 tv = tw[ch * T1::kCells + c];
-            const float dlt = tv.x - tv.y;
-            float gw = V[0] + 2.0f * tv.y * V[1] + tv.x * V[2];
-            if (fabsf(dlt) <= 1.0f) gw += (dlt > 0.f) ? -gl1 : ((dlt < 0.f) ? gl1 : 0.f);
-            g[ch] = gw;
+            g[ch] = rec_adjoint(V[0], V[1], V[2], tv.x, tv.y, gl1);
         }
         // a filler cell one past the last row / column holds the reflection of the one before the last
         sweep_cell_adjoint<F>(S, cam, gx < W ? gx : 2 * W - 2 - gx, gy < H ? gy : 2 * H - 2 - gy, g,
                               own ? diff[k] * m[k] : 0.f, acc);
     }
     // ring cells: the coefficients of the own pixels among their 3x3 neighbours
-    if (threadIdx.x < kSweepRingCells) {
+    if (threadIdx.x < kRingCells) {
         int cx, cy, ry = 0, rx = 0;
-        sweep_ring_cell(threadIdx.x, cx, cy);
+        ring_cell(threadIdx.x, cx, cy);
         const int c = T1::cell(cx, cy);
         if (T1::cell_to_reflected(c, x0, y0, H, W, ry, rx)) {
             float V[kPhotoCoefPlanes];
@@ -471,7 +413,7 @@ __device__ __forceinline__ void sweep_tile_adjoint(const SweepArgs& S, const Cam
 #pragma unroll
             for (int ch = 0; ch < 3; ++ch) {
                 const float2 tv = tw[ch * T1::kCells + c];
-                g[ch] = V[3 * ch] + 2.0f * tv.y * V[3 * ch + 1] + tv.x * V[3 * ch + 2];
+                g[ch] = rec_adjoint(V[3 * ch], V[3 * ch + 1], V[3 * ch + 2], tv.x, tv.y, 0.f);
             }
             sweep_cell_adjoint<F>(S, cam, rx, ry, g, 0.f, acc);
         }
@@ -490,14 +432,17 @@ photo_sweep_kernel(const __grid_constant__ SweepArgs S) {
     const Arith& A = S.P.A;
     const int H = A.H, W = A.W, n = H * W;
     const int hyp = blockIdx.x / S.tiles, tile = blockIdx.x - hyp * S.tiles;
-    const int tiles_x = (W + kTileW - 1) / kTileW;
-    const int tile_y = tile / tiles_x, tile_x = tile - tile_y * tiles_x;
-    const int x0 = tile_x * kTileW, y0 = tile_y * kTileH;
+    int x0, y0;
+    tile_origin(tile, W, x0, y0);
     const Cam cam = load_cam(S.kinv, S.proj + (int64_t)hyp * 12, 0);
     const int tx = threadIdx.x & (kTileW - 1);
     const int ty0 = (threadIdx.x >> 6) * kPixPerThread;
     const int gx = x0 + tx;
     float* cs = kGrad ? reinterpret_cast<float*>(tw + 3 * T1::kCells) : nullptr;   // kGrad: [9][cells] coefficients
+    auto fill = [&](int rx, int ry, int cell, WarpPt& p) {
+        return fill_warped_cell<F>(cam, A, S.P.tgt, (int)S.P.tgt_sc, S.P.src, (int)S.P.src_sc, rx, ry, __ldg(S.tdep + ry * W + rx), tw,
+                                   cell, p);
+    };
     // own pixels: the cell, plus valid and weight = 1 - depth_inconsistency(computed, projected depth) of the warp.
     // Own cells that no consumer reads (partial tiles) are filled from a clamped pixel, as in the pair forward.
     bool valid[kPixPerThread];
@@ -508,28 +453,31 @@ photo_sweep_kernel(const __grid_constant__ SweepArgs S) {
         const int sx = min(max(gx < W ? gx : 2 * W - 2 - gx, 0), W - 1);
         const int sy = min(max(gy < H ? gy : 2 * H - 2 - gy, 0), H - 1);
         WarpPt p;
-        const TapIdx ti = sweep_fill_cell<F>(S, cam, sx, sy, tw, T1::cell(tx, ty0 + k), p);
+        const TapIdx ti = fill(sx, sy, T1::cell(tx, ty0 + k), p);
         valid[k] = p.valid;
         wgt[k] = __fsub_rn(1.0f, depth_inconsistency(p.Z, blend(load_taps(S.sdep, 0, ti, W), ti)));
     }
-    if (threadIdx.x < kSweepRingCells) {
+    if (threadIdx.x < kRingCells) {
         int cx, cy, ry = 0, rx = 0;
-        sweep_ring_cell(threadIdx.x, cx, cy);
+        ring_cell(threadIdx.x, cx, cy);
         const int cell = T1::cell(cx, cy);
-        if (T1::cell_to_reflected(cell, x0, y0, H, W, ry, rx)) {
-            WarpPt p;
-            sweep_fill_cell<F>(S, cam, rx, ry, tw, cell, p);
-        } else {
-#pragma unroll
-            for (int ch = 0; ch < 3; ++ch) tw[ch * T1::kCells + cell] = make_float2(0.f, 0.f);
-        }
+        WarpPt p;
+        if (T1::cell_to_reflected(cell, x0, y0, H, W, ry, rx)) fill(rx, ry, cell, p);
+        else zero_cell(tw, cell);
     }
     __syncthreads();
     float esum[kPixPerThread];
 #pragma unroll
     for (int ch = 0; ch < 3; ++ch)
-        strip_channel<false, kGrad>(tw + ch * T1::kCells, tx, ty0, S.P, ch == 0, esum, kGrad ? cs + 3 * ch * T1::kCells : nullptr,
-                                    gx, y0 + ty0, n);
+        ssim_l1_strip(tw + ch * T1::kCells, tx, ty0, S.P, ch == 0, esum,
+                      [&](int k, const SsimStats& s, const SsimTerms& t) {
+            if constexpr (kGrad) {
+                // the raw coefficients of every own cell, filler cells included: sweep_tile_adjoint scales them
+                const SsimCoef kf = ssim_coef(s, t, A.third * S.P.w_ssim);
+                float* cp = cs + 3 * ch * T1::kCells + T1::cell(tx, ty0 + k);
+                cp[0] = kf.Ay; cp[T1::kCells] = kf.B; cp[2 * T1::kCells] = kf.Cc;
+            }
+        });
     float part_e = 0.f, part_m = 0.f;
     float diff_k[kPixPerThread], m_k[kPixPerThread];             // kGrad: per own pixel, 0 for filler pixels
 #pragma unroll
@@ -721,15 +669,19 @@ photo_refine_step_kernel(const RefineArgs R, const AdamStep s) {
     }
 }
 
-static int sweep_tiles(int H, int W) { return ((W + kTileW - 1) / kTileW) * ((H + kTileH - 1) / kTileH); }
-
-static int fill_photo(PhotoArgs& P, int N, int H, int W, float w_l1, float w_ssim, int flags, const char* who) {
+// The shape check and the launch arguments that every photometric entry point shares.
+static int fill_photo_common(PhotoArgs& P, const char* who, int N, int H, int W, float w_l1, float w_ssim, int flags) {
     if (N <= 0 || H < 2 || W < 2) { set_error("%s: bad shape N=%d H=%d W=%d", who, N, H, W); return 1; }
-    if (N > 65535) { set_error("%s: N=%d exceeds 65535", who, N); return 1; }
-    if (!P.tgt || !P.rec || !P.pd || !P.cd) { set_error("%s: null input pointer", who); return 1; }
     P.A = make_arith(H, W, flags);
     P.w_l1 = w_l1; P.w_ssim = w_ssim;
-    P.C1 = (float)(0.01 * 0.01); P.C2 = (float)(0.03 * 0.03);
+    P.C1 = kSsimC1; P.C2 = kSsimC2;
+    return 0;
+}
+
+static int fill_photo(PhotoArgs& P, int N, int H, int W, float w_l1, float w_ssim, int flags, const char* who) {
+    if (int rc = fill_photo_common(P, who, N, H, W, w_l1, w_ssim, flags)) return rc;
+    if (N > 65535) { set_error("%s: N=%d exceeds 65535", who, N); return 1; }
+    if (!P.tgt || !P.rec || !P.pd || !P.cd) { set_error("%s: null input pointer", who); return 1; }
     return 0;
 }
 
@@ -757,7 +709,7 @@ extern "C" int tcsfm_photo_fwd(const float* tgt, int64_t tgt_sb, int64_t tgt_sc,
     TCSFM_DISPATCH_FLAVOUR(flags, e = cudaFuncSetAttribute(photo_fwd_kernel<F>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     if (e != cudaSuccess) { set_error("tcsfm_photo_fwd: cannot raise dynamic smem: %s", cudaGetErrorString(e)); return 2; }
 #endif
-    dim3 grid(((W + kTileW - 1) / kTileW) * ((H + kTileH - 1) / kTileH), N), block(kTileThreads);
+    dim3 grid(tile_count(H, W), N), block(kTileThreads);
     TCSFM_DISPATCH_FLAVOUR(flags, TCSFM_LAUNCH(photo_fwd_kernel<F>, grid, block, smem, stream, P));
     return check_launch("tcsfm_photo_fwd");
 }
@@ -773,38 +725,51 @@ extern "C" int tcsfm_photo_bwd(const float* tgt, int64_t tgt_sb, int64_t tgt_sc,
     if (int rc = fill_photo(P, N, H, W, w_l1, w_ssim, flags, "tcsfm_photo_bwd")) return rc;
     if (!coef) { set_error("tcsfm_photo_bwd: the forward's coef workspace is required"); return 1; }
     const size_t smem = 9 * Tile<1>::kCells * sizeof(float);
-    dim3 grid(((W + kTileW - 1) / kTileW) * ((H + kTileH - 1) / kTileH), N), block(kTileThreads);
+    dim3 grid(tile_count(H, W), N), block(kTileThreads);
     TCSFM_LAUNCH(photo_bwd_kernel, grid, block, smem, stream, P);
     return check_launch("tcsfm_photo_bwd");
 }
 
 extern "C" int64_t tcsfm_photo_sweep_partial_floats(int N, int H, int W) {
     if (N <= 0 || H <= 0 || W <= 0) return 0;
-    return 2 * (int64_t)N * sweep_tiles(H, W);
+    return 2 * (int64_t)N * tile_count(H, W);
 }
 
-// The argument checks and launch arguments shared by tcsfm_photo_sweep and tcsfm_photo_sweep_grad.
+// The argument checks and launch arguments shared by tcsfm_photo_sweep, tcsfm_photo_sweep_grad and tcsfm_photo_refine.
 static int fill_sweep(SweepArgs& S, const char* who, const float* tgt, int64_t tgt_sc, const float* src, int64_t src_sc,
                       const float* tgt_depth, const float* src_depth, const float* kinv, const float* proj,
                       float* scratch, float* partials, float* sums, int N, int H, int W, float w_l1, float w_ssim, int flags) {
-    if (N <= 0 || H < 2 || W < 2) { set_error("%s: bad shape N=%d H=%d W=%d", who, N, H, W); return 1; }
+    memset(&S, 0, sizeof(S));
+    if (int rc = fill_photo_common(S.P, who, N, H, W, w_l1, w_ssim, flags)) return rc;
     if (!tgt || !src || !tgt_depth || !src_depth || !kinv || !proj) { set_error("%s: null input pointer", who); return 1; }
     if (!scratch || !partials || !sums) { set_error("%s: null scratch, partials or sums", who); return 1; }
-    const int tiles = sweep_tiles(H, W);
+    const int tiles = tile_count(H, W);
     if ((int64_t)tiles * N > 0x7fffffff) { set_error("%s: N=%d hypotheses of %d tiles exceed the grid", who, N, tiles); return 1; }
     // the kernels address a channel plane with 32-bit offsets
     const int64_t n = (int64_t)H * W;
     if (tgt_sc < 0 || src_sc < 0 || 2 * tgt_sc + n > 0x7fffffff || 2 * src_sc + n > 0x7fffffff) {
         set_error("%s: channel strides %lld / %lld out of range", who, (long long)tgt_sc, (long long)src_sc); return 1;
     }
-    memset(&S, 0, sizeof(S));
     S.P.tgt = tgt; S.P.tgt_sc = tgt_sc; S.P.src = src; S.P.src_sc = src_sc; S.P.auto_err = scratch;
-    S.P.A = make_arith(H, W, flags);
-    S.P.w_l1 = w_l1; S.P.w_ssim = w_ssim;
-    S.P.C1 = (float)(0.01 * 0.01); S.P.C2 = (float)(0.03 * 0.03);
     S.tdep = tgt_depth; S.sdep = src_depth; S.kinv = kinv; S.proj = proj; S.partials = partials;
     S.N = N; S.tiles = tiles;
     return 0;
+}
+
+// dynamic shared memory of photo_auto_err_kernel and photo_sweep_kernel<F, false>, and of photo_sweep_kernel<F, true>
+constexpr size_t kSweepSmem = 3 * Tile<1>::kCells * sizeof(float2);
+constexpr size_t kSweepGradSmem = kSweepSmem + kPhotoCoefPlanes * Tile<1>::kCells * sizeof(float);
+
+// What tcsfm_photo_sweep_grad and tcsfm_photo_refine do before their first photo_sweep_kernel<F, true>: raise that
+// kernel's dynamic shared-memory limit and launch the pair's auto-mask error into the scratch.
+static int sweep_grad_prologue(const SweepArgs& S, const char* who, int flags, void* stream) {
+#ifndef TCSFM_HOST_EMU
+    cudaError_t e = cudaSuccess;
+    TCSFM_DISPATCH_FLAVOUR(flags, e = cudaFuncSetAttribute(photo_sweep_kernel<F, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSweepGradSmem));
+    if (e != cudaSuccess) { set_error("%s: cannot raise dynamic smem: %s", who, cudaGetErrorString(e)); return 2; }
+#endif
+    TCSFM_DISPATCH_FLAVOUR(flags, TCSFM_LAUNCH(photo_auto_err_kernel<F>, dim3(S.tiles), dim3(kTileThreads), kSweepSmem, stream, S.P));
+    return check_launch(who);
 }
 
 extern "C" int tcsfm_photo_sweep(const float* tgt, int64_t tgt_sc, const float* src, int64_t src_sc,
@@ -818,11 +783,10 @@ extern "C" int tcsfm_photo_sweep(const float* tgt, int64_t tgt_sc, const float* 
                             N, H, W, w_l1, w_ssim, flags)) return rc;
     S.rec = rec; S.diff = diff; S.mask = mask; S.weight = weight;
     const int tiles = S.tiles;
-    const size_t smem = 3 * Tile<1>::kCells * sizeof(float2);
-    TCSFM_DISPATCH_FLAVOUR(flags, TCSFM_LAUNCH(photo_auto_err_kernel<F>, dim3(tiles), dim3(kTileThreads), smem, stream, S.P));
+    TCSFM_DISPATCH_FLAVOUR(flags, TCSFM_LAUNCH(photo_auto_err_kernel<F>, dim3(tiles), dim3(kTileThreads), kSweepSmem, stream, S.P));
     if (int rc = check_launch(who)) return rc;
     TCSFM_DISPATCH_FLAVOUR(flags, auto* sweep = photo_sweep_kernel<F, false>;
-                                  TCSFM_LAUNCH(sweep, dim3((unsigned)(tiles * N)), dim3(kTileThreads), smem, stream, S));
+                                  TCSFM_LAUNCH(sweep, dim3((unsigned)(tiles * N)), dim3(kTileThreads), kSweepSmem, stream, S));
     if (int rc = check_launch(who)) return rc;
     TCSFM_LAUNCH(photo_sweep_finish_kernel, dim3((N + kSweepFinishThreads - 1) / kSweepFinishThreads), dim3(kSweepFinishThreads), 0,
                  stream, partials, tiles, N, sums);
@@ -831,7 +795,7 @@ extern "C" int tcsfm_photo_sweep(const float* tgt, int64_t tgt_sc, const float* 
 
 extern "C" int64_t tcsfm_photo_sweep_grad_partial_floats(int N, int H, int W) {
     if (N <= 0 || H <= 0 || W <= 0) return 0;
-    return kSweepGradParts * (int64_t)N * sweep_tiles(H, W);
+    return kSweepGradParts * (int64_t)N * tile_count(H, W);
 }
 
 extern "C" int tcsfm_photo_sweep_grad(const float* tgt, int64_t tgt_sc, const float* src, int64_t src_sc,
@@ -844,17 +808,9 @@ extern "C" int tcsfm_photo_sweep_grad(const float* tgt, int64_t tgt_sc, const fl
                             N, H, W, w_l1, w_ssim, flags)) return rc;
     if (!g_proj) { set_error("%s: null g_proj", who); return 1; }
     const int tiles = S.tiles;
-    const size_t smem_fwd = 3 * Tile<1>::kCells * sizeof(float2);
-    const size_t smem = smem_fwd + kPhotoCoefPlanes * Tile<1>::kCells * sizeof(float);
-#ifndef TCSFM_HOST_EMU
-    cudaError_t e = cudaSuccess;
-    TCSFM_DISPATCH_FLAVOUR(flags, e = cudaFuncSetAttribute(photo_sweep_kernel<F, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    if (e != cudaSuccess) { set_error("%s: cannot raise dynamic smem: %s", who, cudaGetErrorString(e)); return 2; }
-#endif
-    TCSFM_DISPATCH_FLAVOUR(flags, TCSFM_LAUNCH(photo_auto_err_kernel<F>, dim3(tiles), dim3(kTileThreads), smem_fwd, stream, S.P));
-    if (int rc = check_launch(who)) return rc;
+    if (int rc = sweep_grad_prologue(S, who, flags, stream)) return rc;
     TCSFM_DISPATCH_FLAVOUR(flags, auto* sweep = photo_sweep_kernel<F, true>;
-                                  TCSFM_LAUNCH(sweep, dim3((unsigned)(tiles * N)), dim3(kTileThreads), smem, stream, S));
+                                  TCSFM_LAUNCH(sweep, dim3((unsigned)(tiles * N)), dim3(kTileThreads), kSweepGradSmem, stream, S));
     if (int rc = check_launch(who)) return rc;
     TCSFM_LAUNCH(photo_sweep_grad_finish_kernel, dim3((N + kSweepFinishThreads - 1) / kSweepFinishThreads), dim3(kSweepFinishThreads), 0,
                  stream, partials, tiles, N, sums, g_proj);
@@ -882,15 +838,7 @@ extern "C" int tcsfm_photo_refine(const float* tgt, int64_t tgt_sc, const float*
     if (int rc = fill_sweep(S, who, tgt, tgt_sc, src, src_sc, tgt_depth, src_depth, kinv, proj, scratch, partials, loss,
                             N, H, W, w_l1, w_ssim, flags)) return rc;
     const int tiles = S.tiles;
-    const size_t smem_fwd = 3 * Tile<1>::kCells * sizeof(float2);
-    const size_t smem = smem_fwd + kPhotoCoefPlanes * Tile<1>::kCells * sizeof(float);
-#ifndef TCSFM_HOST_EMU
-    cudaError_t e = cudaSuccess;
-    TCSFM_DISPATCH_FLAVOUR(flags, e = cudaFuncSetAttribute(photo_sweep_kernel<F, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    if (e != cudaSuccess) { set_error("%s: cannot raise dynamic smem: %s", who, cudaGetErrorString(e)); return 2; }
-#endif
-    TCSFM_DISPATCH_FLAVOUR(flags, TCSFM_LAUNCH(photo_auto_err_kernel<F>, dim3(tiles), dim3(kTileThreads), smem_fwd, stream, S.P));
-    if (int rc = check_launch(who)) return rc;
+    if (int rc = sweep_grad_prologue(S, who, flags, stream)) return rc;
     if (int rc = tcsfm_pose_proj_fwd(poses, kRefineSign, K, 1, proj, N, pose_flags, stream)) return rc;
     auto* step = (pose_flags & TCSFM_ARITH_BMM_NOFMA) ? photo_refine_step_kernel<true, true> : photo_refine_step_kernel<true, false>;
     const dim3 step_grid((N + kSweepFinishThreads - 1) / kSweepFinishThreads), step_block(kSweepFinishThreads);
@@ -902,7 +850,7 @@ extern "C" int tcsfm_photo_refine(const float* tgt, int64_t tgt_sc, const float*
     s.b1 = (float)beta1; s.a1 = (float)(1.0 - beta1); s.b2 = (float)beta2; s.a2 = (float)(1.0 - beta2); s.e = (float)eps;
     for (int t = 1; t <= steps; ++t) {
         TCSFM_DISPATCH_FLAVOUR(flags, auto* sweep = photo_sweep_kernel<F, true>;
-                                      TCSFM_LAUNCH(sweep, dim3((unsigned)(tiles * N)), dim3(kTileThreads), smem, stream, S));
+                                      TCSFM_LAUNCH(sweep, dim3((unsigned)(tiles * N)), dim3(kTileThreads), kSweepGradSmem, stream, S));
         if (int rc = check_launch(who)) return rc;
         s.c1 = (float)(lr / (1.0 - pow(beta1, (double)t)));
         s.c2 = (float)sqrt(1.0 - pow(beta2, (double)t));
@@ -914,7 +862,7 @@ extern "C" int tcsfm_photo_refine(const float* tgt, int64_t tgt_sc, const float*
     }
     // the poses after the last update: their loss and the last chance to be the best
     TCSFM_DISPATCH_FLAVOUR(flags, auto* sweep = photo_sweep_kernel<F, false>;
-                                  TCSFM_LAUNCH(sweep, dim3((unsigned)(tiles * N)), dim3(kTileThreads), smem_fwd, stream, S));
+                                  TCSFM_LAUNCH(sweep, dim3((unsigned)(tiles * N)), dim3(kTileThreads), kSweepSmem, stream, S));
     if (int rc = check_launch(who)) return rc;
     s.first = steps == 0;
     R.loss = loss + (int64_t)steps * N;

@@ -6,11 +6,6 @@
 
 namespace tcsfm {
 
-// C1/C2 exactly as eager PyTorch sees them: the Python doubles 0.01**2 and
-// 0.03**2 converted to fp32 when they meet an fp32 tensor.
-static const float kC1 = (float)(0.01 * 0.01);
-static const float kC2 = (float)(0.03 * 0.03);
-
 // kMean: instead of the map, accumulate mean(map) into out[0] (`scale` = 1 / element count): the
 // `.mean()` that follows SSIM_Loss in the PFT depth-initialisation term (optimizer.py:89-90)
 template <bool kMean>
@@ -121,9 +116,9 @@ extern "C" int tcsfm_ssim_fwd(const float* x, const float* y, float* out, int N,
     if (N <= 0 || H < 2 || W < 2) { set_error("tcsfm_ssim_fwd: bad shape N=%d H=%d W=%d", N, H, W); return 1; }
     if (!x || !y || !out) { set_error("tcsfm_ssim_fwd: null pointer"); return 1; }
     if (N > 65535) { set_error("tcsfm_ssim_fwd: N=%d exceeds 65535 planes", N); return 1; }
-    dim3 grid((W + kTileW - 1) / kTileW, (H + kTileH - 1) / kTileH, N), block(kTileThreads);
+    dim3 grid(tiles_x(W), tiles_y(H), N), block(kTileThreads);
     const size_t smem = 2 * Tile<1>::kCells * sizeof(float);
-    TCSFM_LAUNCH(ssim_fwd_kernel<false>, grid, block, smem, stream, x, y, out, H, W, kC1, kC2, 0.f);
+    TCSFM_LAUNCH(ssim_fwd_kernel<false>, grid, block, smem, stream, x, y, out, H, W, kSsimC1, kSsimC2, 0.f);
     return check_launch("tcsfm_ssim_fwd");
 }
 
@@ -132,11 +127,11 @@ extern "C" int tcsfm_ssim_mean_fwd(const float* x, const float* y, float* out_me
     if (N <= 0 || H < 2 || W < 2) { set_error("tcsfm_ssim_mean_fwd: bad shape N=%d H=%d W=%d", N, H, W); return 1; }
     if (!x || !y || !out_mean) { set_error("tcsfm_ssim_mean_fwd: null pointer"); return 1; }
     if (N > 65535) { set_error("tcsfm_ssim_mean_fwd: N=%d exceeds 65535 planes", N); return 1; }
-    dim3 grid((W + kTileW - 1) / kTileW, (H + kTileH - 1) / kTileH, N), block(kTileThreads);
+    dim3 grid(tiles_x(W), tiles_y(H), N), block(kTileThreads);
     const size_t smem = 2 * Tile<1>::kCells * sizeof(float);
     cudaMemsetAsync(out_mean, 0, sizeof(float), (cudaStream_t)stream);
     const float scale = (float)(1.0 / ((double)N * H * W));
-    TCSFM_LAUNCH(ssim_fwd_kernel<true>, grid, block, smem, stream, x, y, out_mean, H, W, kC1, kC2, scale);
+    TCSFM_LAUNCH(ssim_fwd_kernel<true>, grid, block, smem, stream, x, y, out_mean, H, W, kSsimC1, kSsimC2, scale);
     return check_launch("tcsfm_ssim_mean_fwd");
 }
 
@@ -146,9 +141,9 @@ extern "C" int tcsfm_ssim_bwd(const float* x, const float* y, const float* g_out
     if (N <= 0 || H < 2 || W < 2) { set_error("tcsfm_ssim_bwd: bad shape N=%d H=%d W=%d", N, H, W); return 1; }
     if (!x || !y || !g_out) { set_error("tcsfm_ssim_bwd: null pointer"); return 1; }
     if (N > 65535) { set_error("tcsfm_ssim_bwd: N=%d exceeds 65535 planes", N); return 1; }
-    dim3 grid((W + kTileW - 1) / kTileW, (H + kTileH - 1) / kTileH, N), block(kTileThreads);
+    dim3 grid(tiles_x(W), tiles_y(H), N), block(kTileThreads);
     const size_t smem = (2 * Tile<2>::kCells + 4 * Tile<1>::kCells) * sizeof(float);
-    TCSFM_LAUNCH(ssim_bwd_kernel, grid, block, smem, stream, x, y, g_out, (const float*)nullptr, 0.f, g_x, g_y, H, W, kC1, kC2);
+    TCSFM_LAUNCH(ssim_bwd_kernel, grid, block, smem, stream, x, y, g_out, (const float*)nullptr, 0.f, g_x, g_y, H, W, kSsimC1, kSsimC2);
     return check_launch("tcsfm_ssim_bwd");
 }
 
@@ -158,9 +153,9 @@ extern "C" int tcsfm_ssim_mean_bwd(const float* x, const float* y, const float* 
     if (N <= 0 || H < 2 || W < 2) { set_error("tcsfm_ssim_mean_bwd: bad shape N=%d H=%d W=%d", N, H, W); return 1; }
     if (!x || !y || !g_mean) { set_error("tcsfm_ssim_mean_bwd: null pointer"); return 1; }
     if (N > 65535) { set_error("tcsfm_ssim_mean_bwd: N=%d exceeds 65535 planes", N); return 1; }
-    dim3 grid((W + kTileW - 1) / kTileW, (H + kTileH - 1) / kTileH, N), block(kTileThreads);
+    dim3 grid(tiles_x(W), tiles_y(H), N), block(kTileThreads);
     const size_t smem = (2 * Tile<2>::kCells + 4 * Tile<1>::kCells) * sizeof(float);
     const float scale = (float)(1.0 / ((double)N * H * W));
-    TCSFM_LAUNCH(ssim_bwd_kernel, grid, block, smem, stream, x, y, (const float*)nullptr, g_mean, scale, g_x, g_y, H, W, kC1, kC2);
+    TCSFM_LAUNCH(ssim_bwd_kernel, grid, block, smem, stream, x, y, (const float*)nullptr, g_mean, scale, g_x, g_y, H, W, kSsimC1, kSsimC2);
     return check_launch("tcsfm_ssim_mean_bwd");
 }
