@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define TCSFM_ABI_VERSION 20
+#define TCSFM_ABI_VERSION 21
 
 /* ---- flags ------------------------------------------------------------------ */
 /* Arithmetic flavour.  Eager PyTorch rounds after every operator, but a few ATen
@@ -173,8 +173,9 @@ int tcsfm_photo_bwd(const float* tgt, int64_t tgt_sb, int64_t tgt_sc, const floa
 
 /* ---- compute_photometric_error (optimization_experiments/helpers.py:8-23) for N pose hypotheses of ONE frame
  *      pair, reduced to the loss-surface value of plot_loss_surface.py:11-87 -----------------------------------
- * tgt / src are [1,3,H,W] views (channel strides given; a single pair has no batch stride), tgt_depth / src_depth
- * [1,1,H,W] contiguous, kinv [9], proj [N,12] (hypothesis n's K @ [R|t], as tcsfm_pose_proj_fwd forms it).  For each
+ * tgt / src are [1,3,H,W] views (channel strides given; the *_pairs forms below take B pairs with batch strides),
+ * tgt_depth / src_depth [1,1,H,W] contiguous, kinv [9], proj [N,12] (hypothesis n's K @ [R|t], as
+ * tcsfm_pose_proj_fwd forms it).  For each
  * n, with the warp of tcsfm_warp_fwd under proj[n] and the maps of tcsfm_photo_fwd (valid folded into the mask):
  *   sums[n] = ( sum((diff * mask) * weight), sum(mask) )
  * The per-pixel products carry the eager expression's roundings; the sums are added in a fixed order (the same
@@ -219,6 +220,29 @@ int tcsfm_photo_refine(const float* tgt, int64_t tgt_sc, const float* src, int64
                        float* loss, float* best_loss, int* best_step, float* best_pose,
                        int N, int H, int W, int steps, double lr, double beta1, double beta2, double eps,
                        float w_l1, float w_ssim, int flags, int pose_flags, void* stream);
+
+/* The three calls above for B frame pairs of N hypotheses each, in one call with the same launch count whatever B is.
+ * tgt / src are [B,3,H,W] views: pair b's channel c starts b * *_sb + c * *_sc floats after the pointer (any
+ * *_sb >= 0, so channel slices of a [B,6,H,W] stack need no copy); tgt_depth / src_depth [B,1,H,W] contiguous,
+ * kinv [B,9] and K [B,9] (refine); scratch [B,H,W].  Hypotheses are pair-major: row h = b * N + n of proj, sums,
+ * g_proj, the maps, poses, m, v, best_loss, best_step and best_pose is start n of pair b, and the loss history is
+ * [(steps+1)*B*N].  Every row holds the bits the single-pair call on pair b with those N rows gives.  partials:
+ * tcsfm_photo_sweep_partial_floats / tcsfm_photo_sweep_grad_partial_floats of B * N. */
+int tcsfm_photo_sweep_pairs(const float* tgt, int64_t tgt_sb, int64_t tgt_sc, const float* src, int64_t src_sb,
+                            int64_t src_sc, const float* tgt_depth, const float* src_depth, const float* kinv,
+                            const float* proj, float* scratch, float* partials, float* sums,
+                            float* rec, float* diff, float* mask, float* weight,
+                            int B, int N, int H, int W, float w_l1, float w_ssim, int flags, void* stream);
+int tcsfm_photo_sweep_grad_pairs(const float* tgt, int64_t tgt_sb, int64_t tgt_sc, const float* src, int64_t src_sb,
+                                 int64_t src_sc, const float* tgt_depth, const float* src_depth, const float* kinv,
+                                 const float* proj, float* scratch, float* partials, float* sums, float* g_proj,
+                                 int B, int N, int H, int W, float w_l1, float w_ssim, int flags, void* stream);
+int tcsfm_photo_refine_pairs(const float* tgt, int64_t tgt_sb, int64_t tgt_sc, const float* src, int64_t src_sb,
+                             int64_t src_sc, const float* tgt_depth, const float* src_depth, const float* kinv,
+                             const float* K, float* poses, float* m, float* v, float* proj, float* scratch,
+                             float* partials, float* loss, float* best_loss, int* best_step, float* best_pose,
+                             int B, int N, int H, int W, int steps, double lr, double beta1, double beta2, double eps,
+                             float w_l1, float w_ssim, int flags, int pose_flags, void* stream);
 
 /* ---- DepthOptimizer.compute_optimization_loss (optimization_experiments/optimizer.py:45-86): the
  *      reduction of the error maps of solve_pose_iteratively(return_errors=True) to the PFT loss --------

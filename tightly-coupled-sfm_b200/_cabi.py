@@ -2,7 +2,7 @@
 package loader and by the test-only emulator binding)."""
 import ctypes as C
 
-ABI_VERSION = 20
+ABI_VERSION = 21
 
 ARITH_CPU = 1 << 0
 AUTO_MASK = 1 << 1
@@ -75,6 +75,13 @@ SIGNATURES = {
     "tcsfm_photo_refine": (C.c_int, [_fp, _i64, _fp, _i64] + [_fp] * 14 +
                            [C.c_int, C.c_int, C.c_int, C.c_int, C.c_double, C.c_double, C.c_double, C.c_double,
                             C.c_float, C.c_float, C.c_int, C.c_int, C.c_void_p]),
+    "tcsfm_photo_sweep_pairs": (C.c_int, [_fp, _i64, _i64, _fp, _i64, _i64] + [_fp] * 11 +
+                                    [C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, C.c_float, C.c_int, C.c_void_p]),
+    "tcsfm_photo_sweep_grad_pairs": (C.c_int, [_fp, _i64, _i64, _fp, _i64, _i64] + [_fp] * 8 +
+                                         [C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, C.c_float, C.c_int, C.c_void_p]),
+    "tcsfm_photo_refine_pairs": (C.c_int, [_fp, _i64, _i64, _fp, _i64, _i64] + [_fp] * 14 +
+                                 [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_double, C.c_double, C.c_double,
+                                  C.c_double, C.c_float, C.c_float, C.c_int, C.c_int, C.c_void_p]),
     "tcsfm_smooth_fwd": (C.c_int, [_fp, _fp, _i64, _i64, _fp, _fp, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "tcsfm_smooth_bwd": (C.c_int, [_fp, _fp, _i64, _i64, _fp, _fp, _fp, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "tcsfm_pose_proj_fwd": (C.c_int, [_fp, C.c_float, _fp, C.c_int, _fp, C.c_int, C.c_int, C.c_void_p]),

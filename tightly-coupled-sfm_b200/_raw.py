@@ -431,62 +431,77 @@ def photo_bwd(lib, tgt, rec, proj_depth, comp_depth, coef, g_diff, g_weight, w_l
     return g_rec, g_pd, g_cd
 
 
-def _single_pair(tgt, src, tgt_depth, src_depth, kinv, *expect):
-    """Checks and marshals the one frame pair of the photo_sweep family: tgt / src [1,3,H,W] views, depths [1,1,H,W]
-    and kinv [1,3,3].  `expect` holds (tensor, shape, name) checks of the caller's other arguments, made after these
-    and before any conversion.  Returns (tgt, its channel stride, src, its channel stride, tgt_depth, src_depth, kinv)."""
+def _pairs(b, tgt, src, tgt_depth, src_depth, kinv, *expect):
+    """Checks and marshals the b frame pairs of the photo_sweep family: tgt / src [b,3,H,W] views, depths [b,1,H,W]
+    and kinv [b,3,3].  `expect` holds (tensor, shape, name) checks of the caller's other arguments, made after these
+    and before any conversion.  Returns (tgt, its batch and channel strides, src, its batch and channel strides,
+    tgt_depth, src_depth, kinv)."""
     h, w = tgt.shape[-2], tgt.shape[-1]
-    _expect(tgt, (1, 3, h, w), "tgt")
-    _expect(src, (1, 3, h, w), "src")
-    _expect(tgt_depth, (1, 1, h, w), "tgt_depth")
-    _expect(src_depth, (1, 1, h, w), "src_depth")
-    _expect(kinv, (1, 3, 3), "kinv")
+    _expect(tgt, (b, 3, h, w), "tgt")
+    _expect(src, (b, 3, h, w), "src")
+    _expect(tgt_depth, (b, 1, h, w), "tgt_depth")
+    _expect(src_depth, (b, 1, h, w), "src_depth")
+    _expect(kinv, (b, 3, 3), "kinv")
     for t, shape, name in expect:
         _expect(t, shape, name)
-    tgt, _, tsc = image_view(tgt, "tgt")
-    src, _, ssc = image_view(src, "src")
-    return (tgt, tsc, src, ssc, _f32c(tgt_depth, "tgt_depth"), _f32c(src_depth, "src_depth"), _f32c(kinv, "kinv"))
+    tgt, tsb, tsc = image_view(tgt, "tgt")
+    src, ssb, ssc = image_view(src, "src")
+    return (tgt, tsb, tsc, src, ssb, ssc, _f32c(tgt_depth, "tgt_depth"), _f32c(src_depth, "src_depth"),
+            _f32c(kinv, "kinv"))
+
+
+def _hypotheses(rows, tail):
+    """(pairs b, hypotheses per pair n, the leading shape) of `rows`, which is [N] + tail for one pair or [B,N] + tail
+    for B pairs."""
+    if rows.dim() == len(tail) + 2:
+        return rows.shape[0], rows.shape[1], tuple(rows.shape[:2])
+    return 1, rows.shape[0], (rows.shape[0],)
 
 
 def photo_sweep(lib, tgt, src, tgt_depth, src_depth, kinv, proj, w_l1, w_ssim, flags=0, want_maps=False):
     """compute_photometric_error of ONE pair (tgt / src [1,3,H,W] views, depths [1,1,H,W], kinv [1,3,3]) under each of
     the N projections proj [N,3,4], three launches.  Returns (sums [N,2] = (sum(diff * mask * weight), sum(mask)),
-    maps) with maps = (rec [N,3,H,W], diff, mask, weight [N,1,H,W]) when `want_maps`, else None."""
-    n = proj.shape[0]
+    maps) with maps = (rec [N,3,H,W], diff, mask, weight [N,1,H,W]) when `want_maps`, else None.
+    With proj [B,N,3,4]: B pairs (tgt / src [B,3,H,W] views, depths [B,1,H,W], kinv [B,3,3]), still three launches;
+    the outputs gain the leading B ([B,N,2], [B,N,3,H,W], [B,N,1,H,W])."""
+    b, n, lead = _hypotheses(proj, (3, 4))
     h, w = tgt.shape[-2], tgt.shape[-1]
-    tgt, tsc, src, ssc, td, sd, kinv = _single_pair(tgt, src, tgt_depth, src_depth, kinv, (proj, (n, 3, 4), "proj"))
+    tgt, tsb, tsc, src, ssb, ssc, td, sd, kinv = _pairs(b, tgt, src, tgt_depth, src_depth, kinv,
+                                                        (proj, lead + (3, 4), "proj"))
     proj = _f32c(proj, "proj")
     dev = tgt.device
-    scratch = torch.empty((h, w), dtype=torch.float32, device=dev)
-    partials = torch.empty((lib.tcsfm_photo_sweep_partial_floats(n, h, w),), dtype=torch.float32, device=dev)
-    sums = torch.empty((n, 2), dtype=torch.float32, device=dev)
+    scratch = torch.empty((b, h, w), dtype=torch.float32, device=dev)
+    partials = torch.empty((lib.tcsfm_photo_sweep_partial_floats(b * n, h, w),), dtype=torch.float32, device=dev)
+    sums = torch.empty(lead + (2,), dtype=torch.float32, device=dev)
     maps = None
     if want_maps:
-        maps = (torch.empty((n, 3, h, w), dtype=torch.float32, device=dev),) + \
-            tuple(torch.empty((n, 1, h, w), dtype=torch.float32, device=dev) for _ in range(3))
+        maps = (torch.empty(lead + (3, h, w), dtype=torch.float32, device=dev),) + \
+            tuple(torch.empty(lead + (1, h, w), dtype=torch.float32, device=dev) for _ in range(3))
     rec, diff, mask, weight = maps if want_maps else (None,) * 4
-    _call(lib, lib.tcsfm_photo_sweep, "photo_sweep", tgt.is_cuda,
-          _ptr(tgt), tsc, _ptr(src), ssc, _ptr(td), _ptr(sd), _ptr(kinv), _ptr(proj),
+    _call(lib, lib.tcsfm_photo_sweep_pairs, "photo_sweep", tgt.is_cuda,
+          _ptr(tgt), tsb, tsc, _ptr(src), ssb, ssc, _ptr(td), _ptr(sd), _ptr(kinv), _ptr(proj),
           _ptr(scratch), _ptr(partials), _ptr(sums), _ptr(rec), _ptr(diff), _ptr(mask), _ptr(weight),
-          n, h, w, w_l1, w_ssim, flags, _stream(tgt), launches=3)
+          b, n, h, w, w_l1, w_ssim, flags, _stream(tgt), launches=3)
     return sums, maps
 
 
 def photo_sweep_grad(lib, tgt, src, tgt_depth, src_depth, kinv, proj, w_l1, w_ssim, flags=0):
-    """photo_sweep's sums plus g_proj [N,3,4] = d (sums[n,0] / sums[n,1]) / d proj[n], three launches."""
-    n = proj.shape[0]
+    """photo_sweep's sums plus g_proj [N,3,4] = d (sums[n,0] / sums[n,1]) / d proj[n], three launches; proj [B,N,3,4]
+    takes B pairs as photo_sweep does (sums [B,N,2], g_proj [B,N,3,4])."""
+    b, n, lead = _hypotheses(proj, (3, 4))
     h, w = tgt.shape[-2], tgt.shape[-1]
-    tgt, tsc, src, ssc, td, sd, kinv = _single_pair(tgt, src, tgt_depth, src_depth, kinv, (proj, (n, 3, 4), "proj"))
+    tgt, tsb, tsc, src, ssb, ssc, td, sd, kinv = _pairs(b, tgt, src, tgt_depth, src_depth, kinv,
+                                                        (proj, lead + (3, 4), "proj"))
     proj = _f32c(proj, "proj")
     dev = tgt.device
-    scratch = torch.empty((h, w), dtype=torch.float32, device=dev)
-    partials = torch.empty((lib.tcsfm_photo_sweep_grad_partial_floats(n, h, w),), dtype=torch.float32, device=dev)
-    sums = torch.empty((n, 2), dtype=torch.float32, device=dev)
-    g_proj = torch.empty((n, 3, 4), dtype=torch.float32, device=dev)
-    _call(lib, lib.tcsfm_photo_sweep_grad, "photo_sweep_grad", tgt.is_cuda,
-          _ptr(tgt), tsc, _ptr(src), ssc, _ptr(td), _ptr(sd), _ptr(kinv), _ptr(proj),
+    scratch = torch.empty((b, h, w), dtype=torch.float32, device=dev)
+    partials = torch.empty((lib.tcsfm_photo_sweep_grad_partial_floats(b * n, h, w),), dtype=torch.float32, device=dev)
+    sums = torch.empty(lead + (2,), dtype=torch.float32, device=dev)
+    g_proj = torch.empty(lead + (3, 4), dtype=torch.float32, device=dev)
+    _call(lib, lib.tcsfm_photo_sweep_grad_pairs, "photo_sweep_grad", tgt.is_cuda,
+          _ptr(tgt), tsb, tsc, _ptr(src), ssb, ssc, _ptr(td), _ptr(sd), _ptr(kinv), _ptr(proj),
           _ptr(scratch), _ptr(partials), _ptr(sums), _ptr(g_proj),
-          n, h, w, w_l1, w_ssim, flags, _stream(tgt), launches=3)
+          b, n, h, w, w_l1, w_ssim, flags, _stream(tgt), launches=3)
     return sums, g_proj
 
 
@@ -494,28 +509,30 @@ def photo_refine(lib, tgt, src, tgt_depth, src_depth, kinv, K, poses, steps, lr,
                  flags=0, pose_flags=0):
     """`steps` Adam updates of each starting pose poses [N,6] on its photo_sweep loss, 2 * steps + 4 launches.  Returns
     (poses [N,6] after the updates, loss [steps+1,N], best_loss [N], best_step int32 [N], best_pose [N,6]); `poses`
-    itself is not written."""
-    n = poses.shape[0]
+    itself is not written.  poses [B,N,6] with K [B,3,3] take B pairs as photo_sweep does, with the same launch count;
+    the outputs gain B after their step dimension ([B,N,6], [steps+1,B,N], [B,N])."""
+    b, n, lead = _hypotheses(poses, (6,))
     h, w = tgt.shape[-2], tgt.shape[-1]
-    tgt, tsc, src, ssc, td, sd, kinv = _single_pair(tgt, src, tgt_depth, src_depth, kinv,
-                                                    (K, (1, 3, 3), "K"), (poses, (n, 6), "poses"))
+    tgt, tsb, tsc, src, ssb, ssc, td, sd, kinv = _pairs(b, tgt, src, tgt_depth, src_depth, kinv,
+                                                        (K, (b, 3, 3), "K"), (poses, lead + (6,), "poses"))
     K = _f32c(K, "K")
     out = _f32c(poses, "poses").clone()
     dev = tgt.device
-    m = torch.empty((n, 6), dtype=torch.float32, device=dev)
-    v = torch.empty((n, 6), dtype=torch.float32, device=dev)
-    proj = torch.empty((n, 3, 4), dtype=torch.float32, device=dev)
-    scratch = torch.empty((h, w), dtype=torch.float32, device=dev)
-    partials = torch.empty((lib.tcsfm_photo_sweep_grad_partial_floats(n, h, w),), dtype=torch.float32, device=dev)
-    loss = torch.empty((steps + 1, n), dtype=torch.float32, device=dev)
-    best_loss = torch.empty((n,), dtype=torch.float32, device=dev)
-    best_step = torch.empty((n,), dtype=torch.int32, device=dev)
-    best_pose = torch.empty((n, 6), dtype=torch.float32, device=dev)
-    _call(lib, lib.tcsfm_photo_refine, "photo_refine", tgt.is_cuda,
-          _ptr(tgt), tsc, _ptr(src), ssc, _ptr(td), _ptr(sd), _ptr(kinv), _ptr(K),
+    m = torch.empty(lead + (6,), dtype=torch.float32, device=dev)
+    v = torch.empty(lead + (6,), dtype=torch.float32, device=dev)
+    proj = torch.empty(lead + (3, 4), dtype=torch.float32, device=dev)
+    scratch = torch.empty((b, h, w), dtype=torch.float32, device=dev)
+    partials = torch.empty((lib.tcsfm_photo_sweep_grad_partial_floats(b * n, h, w),), dtype=torch.float32, device=dev)
+    loss = torch.empty((steps + 1,) + lead, dtype=torch.float32, device=dev)
+    best_loss = torch.empty(lead, dtype=torch.float32, device=dev)
+    best_step = torch.empty(lead, dtype=torch.int32, device=dev)
+    best_pose = torch.empty(lead + (6,), dtype=torch.float32, device=dev)
+    _call(lib, lib.tcsfm_photo_refine_pairs, "photo_refine", tgt.is_cuda,
+          _ptr(tgt), tsb, tsc, _ptr(src), ssb, ssc, _ptr(td), _ptr(sd), _ptr(kinv), _ptr(K),
           _ptr(out), _ptr(m), _ptr(v), _ptr(proj), _ptr(scratch), _ptr(partials),
           _ptr(loss), _ptr(best_loss), _ptr(best_step), _ptr(best_pose),
-          n, h, w, steps, lr, beta1, beta2, eps, w_l1, w_ssim, flags, pose_flags, _stream(tgt), launches=2 * steps + 4)
+          b, n, h, w, steps, lr, beta1, beta2, eps, w_l1, w_ssim, flags, pose_flags, _stream(tgt),
+          launches=2 * steps + 4)
     return out, loss, best_loss, best_step, best_pose
 
 

@@ -233,23 +233,39 @@ photo_bwd_kernel(const __grid_constant__ PhotoArgs P) {
 }
 
 // ---------------------------------------------------------------------------
-// compute_photometric_error for N pose hypotheses of ONE frame pair (the loss-surface sweeps of
+// compute_photometric_error for `per` pose hypotheses of each of B frame pairs (the loss-surface sweeps of
 // plot_loss_surface.py:11-87): per hypothesis the warp of inverse_warp2, the maps above and the masked sums
 //   error_sum = sum((diff * auto_mask * valid) * weight)      valid_sum = sum(auto_mask * valid)
-// Three launches: the pose-independent auto-mask error once, one CTA per (hypothesis, tile), and a
-// fixed-order reduction of the per-CTA partials (no float atomics: the sums are deterministic).
+// Three launches: the pose-independent auto-mask error once per pair, one CTA per (hypothesis, tile), and a
+// fixed-order reduction of the per-CTA partials (no float atomics: the sums are deterministic).  Hypotheses are
+// pair-major: global hypothesis hyp is start hyp % per of pair hyp / per.
 // ---------------------------------------------------------------------------
 struct SweepArgs {
-    PhotoArgs P;                          // tgt / src views, auto_err scratch [H,W], weights, SSIM constants, arithmetic
-    const float* tdep; const float* sdep; // [H,W]
-    const float* kinv; const float* proj; // [9], [N,12]
+    PhotoArgs P;                          // tgt / src views of pair 0 and their batch strides, auto_err scratch [B,H,W],
+                                          // weights, SSIM constants, arithmetic
+    const float* tdep; const float* sdep; // [B,H,W]
+    const float* kinv; const float* proj; // [B,9], [N,12]
     float* partials;                      // [tiles][N][2]: per-CTA (sum of products, sum of the mask)
     float* rec; float* diff; float* mask; float* weight;   // optional maps [N,3,H,W], [N,1,H,W] x 3
-    int N, tiles;
+    int N, tiles, per;                    // N = B * per hypotheses in all, per of them for each pair
 };
 
-// auto_err = mean_c(w_l1 * clamp|tgt - src| + w_ssim * SSIM(tgt, src)) of the pair: photo_fwd_kernel's e_src
-template <int F>
+// The inputs of pair b: 64-bit bases, from which the per-pixel code keeps its 32-bit channel and pixel offsets.  The
+// kernels form them where they read them: held in registers across the tile fill, they cost photo_sweep_kernel<F, false>
+// a spill.
+struct SweepPair {
+    const float* tgt; const float* src; const float* tdep; const float* sdep;
+};
+
+__device__ __forceinline__ SweepPair sweep_pair(const SweepArgs& S, int b) {
+    const int64_t n = (int64_t)S.P.A.H * S.P.A.W;
+    return SweepPair{S.P.tgt + b * S.P.tgt_sb, S.P.src + b * S.P.src_sb, S.tdep + b * n, S.sdep + b * n};
+}
+
+// auto_err = mean_c(w_l1 * clamp|tgt - src| + w_ssim * SSIM(tgt, src)) of pair blockIdx.y: photo_fwd_kernel's e_src.
+// kPairs = false: one pair, read without any pair arithmetic (this kernel and photo_sweep_kernel then keep the
+// instructions they had before B pairs; the pair arithmetic measured 5-12 % slower on one pair).
+template <int F, bool kPairs>
 __global__ void __launch_bounds__(kTileThreads)
 photo_auto_err_kernel(const __grid_constant__ PhotoArgs P) {
     using T1 = Tile<1>;
@@ -259,13 +275,15 @@ photo_auto_err_kernel(const __grid_constant__ PhotoArgs P) {
     const int tiles_x = (W + kTileW - 1) / kTileW;
     const int tile_y = blockIdx.x / tiles_x, tile_x = blockIdx.x - tile_y * tiles_x;
     const int x0 = tile_x * kTileW, y0 = tile_y * kTileH;
+    const int64_t b = kPairs ? blockIdx.y : 0;
     for (int cell = threadIdx.x; cell < T1::kCells; cell += kTileThreads) {
         int ry = 0, rx = 0;
         const bool ok = T1::cell_to_reflected(cell, x0, y0, H, W, ry, rx);
         const int pix = ok ? ry * W + rx : 0;
 #pragma unroll
         for (int ch = 0; ch < 3; ++ch)
-            ts[ch * T1::kCells + cell] = ok ? make_float2(__ldg(P.tgt + ch * P.tgt_sc + pix), __ldg(P.src + ch * P.src_sc + pix))
+            ts[ch * T1::kCells + cell] = ok ? make_float2(__ldg(P.tgt + b * P.tgt_sb + ch * P.tgt_sc + pix),
+                                                          __ldg(P.src + b * P.src_sb + ch * P.src_sc + pix))
                                             : make_float2(0.f, 0.f);
     }
     __syncthreads();
@@ -278,7 +296,7 @@ photo_auto_err_kernel(const __grid_constant__ PhotoArgs P) {
 #pragma unroll
     for (int k = 0; k < kPixPerThread; ++k) {
         const int gy = y0 + ty0 + k;
-        if (gx < W && gy < H) P.auto_err[gy * W + gx] = mean3_of_sum<F>(e[k], P.A);
+        if (gx < W && gy < H) (P.auto_err + b * H * W)[gy * W + gx] = mean3_of_sum<F>(e[k], P.A);
     }
 }
 
@@ -296,22 +314,23 @@ constexpr int kSweepGradParts = 14;       // per CTA: E, V, d E / d proj [12]
 // g[ch] = d E / d (warped value of channel ch) of the image pixel (rx, ry); g_weight = d E / d weight at that pixel
 // (own pixels only).  Adds d E / d proj through this pixel's warp into acc (row-major K[R|t]).
 template <int F>
-__device__ __forceinline__ void sweep_cell_adjoint(const SweepArgs& S, const Cam& cam, int rx, int ry, const float (&g)[3],
-                                                   float g_weight, float (&acc)[12]) {
+__device__ __forceinline__ void sweep_cell_adjoint(const SweepArgs& S, int b, const Cam& cam, int rx, int ry,
+                                                   const float (&g)[3], float g_weight, float (&acc)[12]) {
     const Arith& A = S.P.A;
+    const SweepPair pr = sweep_pair(S, b);
     const int pix = ry * A.W + rx;
     WarpPt p;
-    warp_point<F>(cam, A, rx, ry, __ldg(S.tdep + pix), p);
+    warp_point<F>(cam, A, rx, ry, __ldg(pr.tdep + pix), p);
     const TapIdx ti = make_taps(p, A.H, A.W);
     Taps tc[3];
 #pragma unroll
-    for (int ch = 0; ch < 3; ++ch) tc[ch] = load_taps(S.P.src, (int)(ch * S.P.src_sc), ti, A.W);
+    for (int ch = 0; ch < 3; ++ch) tc[ch] = load_taps(pr.src, (int)(ch * S.P.src_sc), ti, A.W);
     float g_ix = 0.f, g_iy = 0.f, g_Z = 0.f;
 #pragma unroll
     for (int ch = 0; ch < 3; ++ch) bilinear_grad(tc[ch], p, g[ch], g_ix, g_iy);
     if (g_weight != 0.f) {
         // weight = 1 - depth_inconsistency(Z, sampled source depth)
-        const Taps td = load_taps(S.sdep, 0, ti, A.W);
+        const Taps td = load_taps(pr.sdep, 0, ti, A.W);
         float g_pd = 0.f;
         depth_inconsistency_adjoint(p.Z, blend(td, ti), -g_weight, g_Z, g_pd);
         bilinear_grad(td, p, g_pd, g_ix, g_iy);
@@ -329,7 +348,8 @@ __device__ __forceinline__ void sweep_cell_adjoint(const SweepArgs& S, const Cam
 // The adjoint of one tile for photo_sweep_kernel<F, true>, after its forward: scales the raw coefficients the strips left
 // in `cs` by the upstream, then accumulates d E / d proj of the tile's cells into acc.  Contains __syncthreads().
 template <int F>
-__device__ __forceinline__ void sweep_tile_adjoint(const SweepArgs& S, const Cam& cam, const float2* tw, float* cs, int x0, int y0,
+__device__ __forceinline__ void sweep_tile_adjoint(const SweepArgs& S, int b, const Cam& cam, const float2* tw, float* cs,
+                                                   int x0, int y0,
                                                    const float (&diff)[kPixPerThread], const float (&m)[kPixPerThread],
                                                    const float (&wgt)[kPixPerThread], float (&acc)[12]) {
     using T1 = Tile<1>;
@@ -390,7 +410,7 @@ __device__ __forceinline__ void sweep_tile_adjoint(const SweepArgs& S, const Cam
             g[ch] = rec_adjoint(V[0], V[1], V[2], tv.x, tv.y, gl1);
         }
         // a filler cell one past the last row / column holds the reflection of the one before the last
-        sweep_cell_adjoint<F>(S, cam, gx < W ? gx : 2 * W - 2 - gx, gy < H ? gy : 2 * H - 2 - gy, g,
+        sweep_cell_adjoint<F>(S, b, cam, gx < W ? gx : 2 * W - 2 - gx, gy < H ? gy : 2 * H - 2 - gy, g,
                               own ? diff[k] * m[k] : 0.f, acc);
     }
     // ring cells: the coefficients of the own pixels among their 3x3 neighbours
@@ -415,7 +435,7 @@ __device__ __forceinline__ void sweep_tile_adjoint(const SweepArgs& S, const Cam
                 const float2 tv = tw[ch * T1::kCells + c];
                 g[ch] = rec_adjoint(V[3 * ch], V[3 * ch + 1], V[3 * ch + 2], tv.x, tv.y, 0.f);
             }
-            sweep_cell_adjoint<F>(S, cam, rx, ry, g, 0.f, acc);
+            sweep_cell_adjoint<F>(S, b, cam, rx, ry, g, 0.f, acc);
         }
     }
 }
@@ -423,7 +443,8 @@ __device__ __forceinline__ void sweep_tile_adjoint(const SweepArgs& S, const Cam
 // One CTA per (hypothesis, tile).  kGrad = false: the sums and optional maps of tcsfm_photo_sweep.  kGrad = true: the
 // same forward, instruction for instruction (so E and V keep their bits), whose strips also leave their SSIM adjoint
 // coefficients in shared memory; then the adjoint of the tile (sweep_tile_adjoint), and a partial (E, V, dE/dproj[12]).
-template <int F, bool kGrad>
+// kPairs as in photo_auto_err_kernel.
+template <int F, bool kGrad, bool kPairs>
 __global__ void __launch_bounds__(kTileThreads, kGrad ? 2 : 3)
 photo_sweep_kernel(const __grid_constant__ SweepArgs S) {
     using T1 = Tile<1>;
@@ -432,15 +453,17 @@ photo_sweep_kernel(const __grid_constant__ SweepArgs S) {
     const Arith& A = S.P.A;
     const int H = A.H, W = A.W, n = H * W;
     const int hyp = blockIdx.x / S.tiles, tile = blockIdx.x - hyp * S.tiles;
+    const int b = kPairs ? hyp / S.per : 0;
     int x0, y0;
     tile_origin(tile, W, x0, y0);
-    const Cam cam = load_cam(S.kinv, S.proj + (int64_t)hyp * 12, 0);
+    const Cam cam = load_cam(S.kinv + 9 * (int64_t)b, S.proj + (int64_t)hyp * 12, 0);
     const int tx = threadIdx.x & (kTileW - 1);
     const int ty0 = (threadIdx.x >> 6) * kPixPerThread;
     const int gx = x0 + tx;
     float* cs = kGrad ? reinterpret_cast<float*>(tw + 3 * T1::kCells) : nullptr;   // kGrad: [9][cells] coefficients
     auto fill = [&](int rx, int ry, int cell, WarpPt& p) {
-        return fill_warped_cell<F>(cam, A, S.P.tgt, (int)S.P.tgt_sc, S.P.src, (int)S.P.src_sc, rx, ry, __ldg(S.tdep + ry * W + rx), tw,
+        const SweepPair pr = sweep_pair(S, b);
+        return fill_warped_cell<F>(cam, A, pr.tgt, (int)S.P.tgt_sc, pr.src, (int)S.P.src_sc, rx, ry, __ldg(pr.tdep + ry * W + rx), tw,
                                    cell, p);
     };
     // own pixels: the cell, plus valid and weight = 1 - depth_inconsistency(computed, projected depth) of the warp.
@@ -455,7 +478,7 @@ photo_sweep_kernel(const __grid_constant__ SweepArgs S) {
         WarpPt p;
         const TapIdx ti = fill(sx, sy, T1::cell(tx, ty0 + k), p);
         valid[k] = p.valid;
-        wgt[k] = __fsub_rn(1.0f, depth_inconsistency(p.Z, blend(load_taps(S.sdep, 0, ti, W), ti)));
+        wgt[k] = __fsub_rn(1.0f, depth_inconsistency(p.Z, blend(load_taps(sweep_pair(S, b).sdep, 0, ti, W), ti)));
     }
     if (threadIdx.x < kRingCells) {
         int cx, cy, ry = 0, rx = 0;
@@ -487,7 +510,7 @@ photo_sweep_kernel(const __grid_constant__ SweepArgs S) {
         if (gx < W && gy < H) {
             const int pix = gy * W + gx;
             const float diff = mean3_of_sum<F>(esum[k], A);
-            const float m = (diff < __ldg(S.P.auto_err + pix)) ? (valid[k] ? 1.f : 0.f) : 0.f;
+            const float m = (diff < __ldg(S.P.auto_err + (int64_t)b * n + pix)) ? (valid[k] ? 1.f : 0.f) : 0.f;
             if constexpr (kGrad) { diff_k[k] = diff; m_k[k] = m; }
             // (diff_img * valid_mask) * weight_mask, each product rounded like the eager expression
             part_e = __fadd_rn(part_e, __fmul_rn(__fmul_rn(diff, m), wgt[k]));
@@ -504,7 +527,7 @@ photo_sweep_kernel(const __grid_constant__ SweepArgs S) {
     }
     if constexpr (kGrad) {
         float acc[12];
-        sweep_tile_adjoint<F>(S, cam, tw, cs, x0, y0, diff_k, m_k, wgt, acc);
+        sweep_tile_adjoint<F>(S, b, cam, tw, cs, x0, y0, diff_k, m_k, wgt, acc);
         float part[kSweepGradParts];
         part[0] = part_e;
         part[1] = part_m;
@@ -593,18 +616,19 @@ photo_sweep_grad_finish_kernel(const float* __restrict__ partials, int tiles, in
 // forward + adjoint (photo_sweep_kernel<F, true>) and photo_refine_step_kernel, one thread per hypothesis, which
 // finishes the sums and the gradient like photo_sweep_grad_finish_kernel, keeps the loss history and the best
 // pose seen, maps the gradient to the pose (pose_proj_bwd_body), updates the pose and forms its next K[R|t]
-// (pose_proj_fwd_body).  Every operation of the update is a separately rounded fp32 operation, so a loop of torch
-// operators on fp32 tensors reproduces its bits.
+// (pose_proj_fwd_body) with the K of its pair.  Every operation of the update is a separately rounded fp32 operation,
+// so a loop of torch operators on fp32 tensors reproduces its bits.
 // ---------------------------------------------------------------------------
 struct RefineArgs {
     const float* partials;     // [tiles][N][kSweepGradParts] (update) or [tiles][N][2] (last evaluation)
-    const float* K;            // [9]
+    const float* K;            // [B,9]
     float* poses;              // [N,6], updated in place
     float* m; float* v;        // [N,6] Adam moments
     float* proj;               // [N,12] K[R|t] of the poses, rewritten after the update
     float* loss;               // [N]: the row of this evaluation
     float* best_loss; int* best_step; float* best_pose;   // [N], [N], [N,6]
-    int tiles, N, step;        // step: the number of updates behind this evaluation
+    int tiles, N, per, step;   // N = B * per pair-major hypotheses; step: the number of updates behind this evaluation
+    int project;               // instead of an evaluation: K[R|t] of the starting poses into proj
 };
 
 // The step's scalars, each rounded to fp32 once from double on the host.  first: the first evaluation of the call
@@ -621,6 +645,11 @@ __global__ void __launch_bounds__(kSweepFinishThreads)
 photo_refine_step_kernel(const RefineArgs R, const AdamStep s) {
     const int hyp = blockIdx.x * kSweepFinishThreads + threadIdx.x;
     if (hyp >= R.N) return;
+    const float* K = R.K + 9 * (hyp / R.per);
+    if (R.project) {
+        pose_proj_fwd_body<kNoFma>(R.poses + hyp * 6, kRefineSign, K, 1, R.proj, hyp);
+        return;
+    }
     double e, g[12];
     float V;
     sweep_partials_sum<kUpdate ? kSweepGradParts : 2>(R.partials, R.tiles, R.N, hyp, e, V, g);
@@ -649,7 +678,7 @@ photo_refine_step_kernel(const RefineArgs R, const AdamStep s) {
             float g_proj[12], gp[6];
 #pragma unroll
             for (int i = 0; i < 12; ++i) g_proj[i] = (float)(g[i] / (double)V);
-            pose_proj_bwd_body(p, kRefineSign, R.K, 1, g_proj, gp, 0);
+            pose_proj_bwd_body(p, kRefineSign, K, 1, g_proj, gp, 0);
 #pragma unroll
             for (int j = 0; j < 6; ++j) {
                 const float mj = __fadd_rn(__fmul_rn(s.b1, s.first ? 0.f : m[j]), __fmul_rn(s.a1, gp[j]));
@@ -660,7 +689,7 @@ photo_refine_step_kernel(const RefineArgs R, const AdamStep s) {
                 v[j] = vj;
                 R.poses[hyp * 6 + j] = p[j];
             }
-            pose_proj_fwd_body<kNoFma>(p, kRefineSign, R.K, 1, R.proj, hyp);
+            pose_proj_fwd_body<kNoFma>(p, kRefineSign, K, 1, R.proj, hyp);
         } else if (s.first) {
             // frozen: no valid pixel, so no gradient; the pose (and its K[R|t]) stays, the moments start at 0
 #pragma unroll
@@ -735,24 +764,34 @@ extern "C" int64_t tcsfm_photo_sweep_partial_floats(int N, int H, int W) {
     return 2 * (int64_t)N * tile_count(H, W);
 }
 
-// The argument checks and launch arguments shared by tcsfm_photo_sweep, tcsfm_photo_sweep_grad and tcsfm_photo_refine.
-static int fill_sweep(SweepArgs& S, const char* who, const float* tgt, int64_t tgt_sc, const float* src, int64_t src_sc,
-                      const float* tgt_depth, const float* src_depth, const float* kinv, const float* proj,
-                      float* scratch, float* partials, float* sums, int N, int H, int W, float w_l1, float w_ssim, int flags) {
+// The argument checks and launch arguments shared by the sweep, sweep_grad and refine entry points: B pairs of N
+// hypotheses each, whose images are `*_sb` floats apart.
+static int fill_sweep(SweepArgs& S, const char* who, int B, const float* tgt, int64_t tgt_sb, int64_t tgt_sc, const float* src,
+                      int64_t src_sb, int64_t src_sc, const float* tgt_depth, const float* src_depth, const float* kinv,
+                      const float* proj, float* scratch, float* partials, float* sums, int N, int H, int W, float w_l1,
+                      float w_ssim, int flags) {
     memset(&S, 0, sizeof(S));
     if (int rc = fill_photo_common(S.P, who, N, H, W, w_l1, w_ssim, flags)) return rc;
+    if (B < 1) { set_error("%s: bad pair count B=%d", who, B); return 1; }
+    if ((int64_t)B * N > 0x7fffffff) { set_error("%s: B=%d pairs x N=%d hypotheses exceed 2^31 - 1", who, B, N); return 1; }
     if (!tgt || !src || !tgt_depth || !src_depth || !kinv || !proj) { set_error("%s: null input pointer", who); return 1; }
     if (!scratch || !partials || !sums) { set_error("%s: null scratch, partials or sums", who); return 1; }
-    const int tiles = tile_count(H, W);
-    if ((int64_t)tiles * N > 0x7fffffff) { set_error("%s: N=%d hypotheses of %d tiles exceed the grid", who, N, tiles); return 1; }
-    // the kernels address a channel plane with 32-bit offsets
+    const int tiles = tile_count(H, W), total = B * N;
+    if ((int64_t)tiles * total > 0x7fffffff) {
+        set_error("%s: %s%d hypotheses of %d tiles exceed the grid", who, B > 1 ? "B x N = " : "N=", total, tiles); return 1;
+    }
+    // the kernels address a channel plane with 32-bit offsets from the pair's base
     const int64_t n = (int64_t)H * W;
     if (tgt_sc < 0 || src_sc < 0 || 2 * tgt_sc + n > 0x7fffffff || 2 * src_sc + n > 0x7fffffff) {
         set_error("%s: channel strides %lld / %lld out of range", who, (long long)tgt_sc, (long long)src_sc); return 1;
     }
-    S.P.tgt = tgt; S.P.tgt_sc = tgt_sc; S.P.src = src; S.P.src_sc = src_sc; S.P.auto_err = scratch;
+    if (tgt_sb < 0 || src_sb < 0) {
+        set_error("%s: batch strides %lld / %lld are negative", who, (long long)tgt_sb, (long long)src_sb); return 1;
+    }
+    S.P.tgt = tgt; S.P.tgt_sb = tgt_sb; S.P.tgt_sc = tgt_sc; S.P.src = src; S.P.src_sb = src_sb; S.P.src_sc = src_sc;
+    S.P.auto_err = scratch;
     S.tdep = tgt_depth; S.sdep = src_depth; S.kinv = kinv; S.proj = proj; S.partials = partials;
-    S.N = N; S.tiles = tiles;
+    S.N = total; S.tiles = tiles; S.per = N;
     return 0;
 }
 
@@ -760,36 +799,131 @@ static int fill_sweep(SweepArgs& S, const char* who, const float* tgt, int64_t t
 constexpr size_t kSweepSmem = 3 * Tile<1>::kCells * sizeof(float2);
 constexpr size_t kSweepGradSmem = kSweepSmem + kPhotoCoefPlanes * Tile<1>::kCells * sizeof(float);
 
-// What tcsfm_photo_sweep_grad and tcsfm_photo_refine do before their first photo_sweep_kernel<F, true>: raise that
-// kernel's dynamic shared-memory limit and launch the pair's auto-mask error into the scratch.
-static int sweep_grad_prologue(const SweepArgs& S, const char* who, int flags, void* stream) {
-#ifndef TCSFM_HOST_EMU
-    cudaError_t e = cudaSuccess;
-    TCSFM_DISPATCH_FLAVOUR(flags, e = cudaFuncSetAttribute(photo_sweep_kernel<F, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSweepGradSmem));
-    if (e != cudaSuccess) { set_error("%s: cannot raise dynamic smem: %s", who, cudaGetErrorString(e)); return 2; }
-#endif
-    TCSFM_DISPATCH_FLAVOUR(flags, TCSFM_LAUNCH(photo_auto_err_kernel<F>, dim3(S.tiles), dim3(kTileThreads), kSweepSmem, stream, S.P));
+// The kernels for B pairs: B = 1 takes the instantiations without pair arithmetic.
+template <int F>
+static auto auto_err_kernel(int B) { return B > 1 ? photo_auto_err_kernel<F, true> : photo_auto_err_kernel<F, false>; }
+template <int F, bool kGrad>
+static auto sweep_kernel(int B) { return B > 1 ? photo_sweep_kernel<F, kGrad, true> : photo_sweep_kernel<F, kGrad, false>; }
+
+// The auto-mask error of every pair into the scratch: tiles x B CTAs.
+static int sweep_auto_err(const SweepArgs& S, const char* who, int B, int flags, void* stream) {
+    TCSFM_DISPATCH_FLAVOUR(flags, auto* auto_err = auto_err_kernel<F>(B);
+                                  TCSFM_LAUNCH(auto_err, dim3(S.tiles, B), dim3(kTileThreads), kSweepSmem, stream, S.P));
     return check_launch(who);
 }
 
-extern "C" int tcsfm_photo_sweep(const float* tgt, int64_t tgt_sc, const float* src, int64_t src_sc,
-                                 const float* tgt_depth, const float* src_depth, const float* kinv, const float* proj,
-                                 float* scratch, float* partials, float* sums,
-                                 float* rec, float* diff, float* mask, float* weight,
-                                 int N, int H, int W, float w_l1, float w_ssim, int flags, void* stream) {
-    const char* who = "tcsfm_photo_sweep";
+// What the sweep_grad and refine entry points do before their first photo_sweep_kernel<F, true>: raise that kernel's
+// dynamic shared-memory limit and launch the pairs' auto-mask error into the scratch.
+static int sweep_grad_prologue(const SweepArgs& S, const char* who, int B, int flags, void* stream) {
+#ifndef TCSFM_HOST_EMU
+    cudaError_t e = cudaSuccess;
+    TCSFM_DISPATCH_FLAVOUR(flags, e = cudaFuncSetAttribute(sweep_kernel<F, true>(B), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSweepGradSmem));
+    if (e != cudaSuccess) { set_error("%s: cannot raise dynamic smem: %s", who, cudaGetErrorString(e)); return 2; }
+#endif
+    return sweep_auto_err(S, who, B, flags, stream);
+}
+
+static int photo_sweep(const char* who, int B, const float* tgt, int64_t tgt_sb, int64_t tgt_sc, const float* src,
+                       int64_t src_sb, int64_t src_sc, const float* tgt_depth, const float* src_depth, const float* kinv,
+                       const float* proj, float* scratch, float* partials, float* sums,
+                       float* rec, float* diff, float* mask, float* weight,
+                       int N, int H, int W, float w_l1, float w_ssim, int flags, void* stream) {
     SweepArgs S;
-    if (int rc = fill_sweep(S, who, tgt, tgt_sc, src, src_sc, tgt_depth, src_depth, kinv, proj, scratch, partials, sums,
-                            N, H, W, w_l1, w_ssim, flags)) return rc;
+    if (int rc = fill_sweep(S, who, B, tgt, tgt_sb, tgt_sc, src, src_sb, src_sc, tgt_depth, src_depth, kinv, proj, scratch,
+                            partials, sums, N, H, W, w_l1, w_ssim, flags)) return rc;
     S.rec = rec; S.diff = diff; S.mask = mask; S.weight = weight;
-    const int tiles = S.tiles;
-    TCSFM_DISPATCH_FLAVOUR(flags, TCSFM_LAUNCH(photo_auto_err_kernel<F>, dim3(tiles), dim3(kTileThreads), kSweepSmem, stream, S.P));
+    const int tiles = S.tiles, total = S.N;
+    if (int rc = sweep_auto_err(S, who, B, flags, stream)) return rc;
+    TCSFM_DISPATCH_FLAVOUR(flags, auto* sweep = sweep_kernel<F, false>(B);
+                                  TCSFM_LAUNCH(sweep, dim3((unsigned)(tiles * total)), dim3(kTileThreads), kSweepSmem, stream, S));
     if (int rc = check_launch(who)) return rc;
-    TCSFM_DISPATCH_FLAVOUR(flags, auto* sweep = photo_sweep_kernel<F, false>;
-                                  TCSFM_LAUNCH(sweep, dim3((unsigned)(tiles * N)), dim3(kTileThreads), kSweepSmem, stream, S));
+    TCSFM_LAUNCH(photo_sweep_finish_kernel, dim3((total + kSweepFinishThreads - 1) / kSweepFinishThreads), dim3(kSweepFinishThreads),
+                 0, stream, partials, tiles, total, sums);
+    return check_launch(who);
+}
+
+static int photo_sweep_grad(const char* who, int B, const float* tgt, int64_t tgt_sb, int64_t tgt_sc, const float* src,
+                            int64_t src_sb, int64_t src_sc, const float* tgt_depth, const float* src_depth, const float* kinv,
+                            const float* proj, float* scratch, float* partials, float* sums, float* g_proj,
+                            int N, int H, int W, float w_l1, float w_ssim, int flags, void* stream) {
+    SweepArgs S;
+    if (int rc = fill_sweep(S, who, B, tgt, tgt_sb, tgt_sc, src, src_sb, src_sc, tgt_depth, src_depth, kinv, proj, scratch,
+                            partials, sums, N, H, W, w_l1, w_ssim, flags)) return rc;
+    if (!g_proj) { set_error("%s: null g_proj", who); return 1; }
+    const int tiles = S.tiles, total = S.N;
+    if (int rc = sweep_grad_prologue(S, who, B, flags, stream)) return rc;
+    TCSFM_DISPATCH_FLAVOUR(flags, auto* sweep = sweep_kernel<F, true>(B);
+                                  TCSFM_LAUNCH(sweep, dim3((unsigned)(tiles * total)), dim3(kTileThreads), kSweepGradSmem, stream, S));
     if (int rc = check_launch(who)) return rc;
-    TCSFM_LAUNCH(photo_sweep_finish_kernel, dim3((N + kSweepFinishThreads - 1) / kSweepFinishThreads), dim3(kSweepFinishThreads), 0,
-                 stream, partials, tiles, N, sums);
+    TCSFM_LAUNCH(photo_sweep_grad_finish_kernel, dim3((total + kSweepFinishThreads - 1) / kSweepFinishThreads),
+                 dim3(kSweepFinishThreads), 0, stream, partials, tiles, total, sums, g_proj);
+    return check_launch(who);
+}
+
+static int photo_refine(const char* who, int B, const float* tgt, int64_t tgt_sb, int64_t tgt_sc, const float* src,
+                        int64_t src_sb, int64_t src_sc, const float* tgt_depth, const float* src_depth, const float* kinv,
+                        const float* K, float* poses, float* m, float* v, float* proj, float* scratch, float* partials,
+                        float* loss, float* best_loss, int* best_step, float* best_pose,
+                        int N, int H, int W, int steps, double lr, double beta1, double beta2, double eps,
+                        float w_l1, float w_ssim, int flags, int pose_flags, void* stream) {
+    if (!K || !poses || !m || !v || !best_loss || !best_step || !best_pose) { set_error("%s: null pointer", who); return 1; }
+    if (steps < 0) { set_error("%s: steps=%d is negative", who, steps); return 1; }
+    if (B > 0 && N > 0 && ((int64_t)steps + 1) * B * N > 0x7fffffff) {
+        set_error("%s: the loss history of %d steps x %lld hypotheses exceeds 2^31 - 1 entries", who, steps,
+                  (long long)B * N);
+        return 1;
+    }
+    if (!(lr > 0.0 && lr < INFINITY) || !(eps > 0.0 && eps < INFINITY) || !(beta1 >= 0.0 && beta1 < 1.0) ||
+        !(beta2 >= 0.0 && beta2 < 1.0)) {
+        set_error("%s: bad optimizer arguments lr=%g betas=(%g, %g) eps=%g", who, lr, beta1, beta2, eps); return 1;
+    }
+    // `loss` stands in for the sums of fill_sweep's checks: each row of it is written from the partials here
+    SweepArgs S;
+    if (int rc = fill_sweep(S, who, B, tgt, tgt_sb, tgt_sc, src, src_sb, src_sc, tgt_depth, src_depth, kinv, proj, scratch,
+                            partials, loss, N, H, W, w_l1, w_ssim, flags)) return rc;
+    const int tiles = S.tiles, total = S.N;
+    if (int rc = sweep_grad_prologue(S, who, B, flags, stream)) return rc;
+    auto* step = (pose_flags & TCSFM_ARITH_BMM_NOFMA) ? photo_refine_step_kernel<true, true> : photo_refine_step_kernel<true, false>;
+    const dim3 step_grid((total + kSweepFinishThreads - 1) / kSweepFinishThreads), step_block(kSweepFinishThreads);
+    RefineArgs R;
+    memset(&R, 0, sizeof(R));
+    R.partials = partials; R.K = K; R.poses = poses; R.m = m; R.v = v; R.proj = proj;
+    R.best_loss = best_loss; R.best_step = best_step; R.best_pose = best_pose;
+    R.tiles = tiles; R.N = total; R.per = N;
+    AdamStep s;
+    s.b1 = (float)beta1; s.a1 = (float)(1.0 - beta1); s.b2 = (float)beta2; s.a2 = (float)(1.0 - beta2); s.e = (float)eps;
+    s.c1 = s.c2 = 0.f;
+    s.first = 1;
+    // K[R|t] of the starting poses: one pair reads K[i % 1] in the pose kernel, B pairs their own K in the step kernel
+    if (B == 1) {
+        if (int rc = tcsfm_pose_proj_fwd(poses, kRefineSign, K, 1, proj, N, pose_flags, stream)) return rc;
+    } else {
+        R.project = 1;
+        TCSFM_LAUNCH(step, step_grid, step_block, 0, stream, R, s);
+        if (int rc = check_launch(who)) return rc;
+        R.project = 0;
+    }
+    for (int t = 1; t <= steps; ++t) {
+        TCSFM_DISPATCH_FLAVOUR(flags, auto* sweep = sweep_kernel<F, true>(B);
+                                      TCSFM_LAUNCH(sweep, dim3((unsigned)(tiles * total)), dim3(kTileThreads), kSweepGradSmem, stream, S));
+        if (int rc = check_launch(who)) return rc;
+        s.c1 = (float)(lr / (1.0 - pow(beta1, (double)t)));
+        s.c2 = (float)sqrt(1.0 - pow(beta2, (double)t));
+        s.first = t == 1;
+        R.loss = loss + (int64_t)(t - 1) * total;
+        R.step = t - 1;
+        TCSFM_LAUNCH(step, step_grid, step_block, 0, stream, R, s);
+        if (int rc = check_launch(who)) return rc;
+    }
+    // the poses after the last update: their loss and the last chance to be the best
+    TCSFM_DISPATCH_FLAVOUR(flags, auto* sweep = sweep_kernel<F, false>(B);
+                                  TCSFM_LAUNCH(sweep, dim3((unsigned)(tiles * total)), dim3(kTileThreads), kSweepSmem, stream, S));
+    if (int rc = check_launch(who)) return rc;
+    s.first = steps == 0;
+    R.loss = loss + (int64_t)steps * total;
+    R.step = steps;
+    auto* last = photo_refine_step_kernel<false, false>;
+    TCSFM_LAUNCH(last, step_grid, step_block, 0, stream, R, s);
     return check_launch(who);
 }
 
@@ -798,23 +932,39 @@ extern "C" int64_t tcsfm_photo_sweep_grad_partial_floats(int N, int H, int W) {
     return kSweepGradParts * (int64_t)N * tile_count(H, W);
 }
 
+extern "C" int tcsfm_photo_sweep(const float* tgt, int64_t tgt_sc, const float* src, int64_t src_sc,
+                                 const float* tgt_depth, const float* src_depth, const float* kinv, const float* proj,
+                                 float* scratch, float* partials, float* sums,
+                                 float* rec, float* diff, float* mask, float* weight,
+                                 int N, int H, int W, float w_l1, float w_ssim, int flags, void* stream) {
+    return photo_sweep("tcsfm_photo_sweep", 1, tgt, 0, tgt_sc, src, 0, src_sc, tgt_depth, src_depth, kinv, proj, scratch,
+                       partials, sums, rec, diff, mask, weight, N, H, W, w_l1, w_ssim, flags, stream);
+}
+
+extern "C" int tcsfm_photo_sweep_pairs(const float* tgt, int64_t tgt_sb, int64_t tgt_sc, const float* src, int64_t src_sb,
+                                       int64_t src_sc, const float* tgt_depth, const float* src_depth, const float* kinv,
+                                       const float* proj, float* scratch, float* partials, float* sums,
+                                       float* rec, float* diff, float* mask, float* weight,
+                                       int B, int N, int H, int W, float w_l1, float w_ssim, int flags, void* stream) {
+    return photo_sweep("tcsfm_photo_sweep_pairs", B, tgt, tgt_sb, tgt_sc, src, src_sb, src_sc, tgt_depth, src_depth, kinv,
+                       proj, scratch, partials, sums, rec, diff, mask, weight, N, H, W, w_l1, w_ssim, flags, stream);
+}
+
 extern "C" int tcsfm_photo_sweep_grad(const float* tgt, int64_t tgt_sc, const float* src, int64_t src_sc,
                                       const float* tgt_depth, const float* src_depth, const float* kinv, const float* proj,
                                       float* scratch, float* partials, float* sums, float* g_proj,
                                       int N, int H, int W, float w_l1, float w_ssim, int flags, void* stream) {
-    const char* who = "tcsfm_photo_sweep_grad";
-    SweepArgs S;
-    if (int rc = fill_sweep(S, who, tgt, tgt_sc, src, src_sc, tgt_depth, src_depth, kinv, proj, scratch, partials, sums,
-                            N, H, W, w_l1, w_ssim, flags)) return rc;
-    if (!g_proj) { set_error("%s: null g_proj", who); return 1; }
-    const int tiles = S.tiles;
-    if (int rc = sweep_grad_prologue(S, who, flags, stream)) return rc;
-    TCSFM_DISPATCH_FLAVOUR(flags, auto* sweep = photo_sweep_kernel<F, true>;
-                                  TCSFM_LAUNCH(sweep, dim3((unsigned)(tiles * N)), dim3(kTileThreads), kSweepGradSmem, stream, S));
-    if (int rc = check_launch(who)) return rc;
-    TCSFM_LAUNCH(photo_sweep_grad_finish_kernel, dim3((N + kSweepFinishThreads - 1) / kSweepFinishThreads), dim3(kSweepFinishThreads), 0,
-                 stream, partials, tiles, N, sums, g_proj);
-    return check_launch(who);
+    return photo_sweep_grad("tcsfm_photo_sweep_grad", 1, tgt, 0, tgt_sc, src, 0, src_sc, tgt_depth, src_depth, kinv, proj,
+                            scratch, partials, sums, g_proj, N, H, W, w_l1, w_ssim, flags, stream);
+}
+
+extern "C" int tcsfm_photo_sweep_grad_pairs(const float* tgt, int64_t tgt_sb, int64_t tgt_sc, const float* src,
+                                            int64_t src_sb, int64_t src_sc, const float* tgt_depth, const float* src_depth,
+                                            const float* kinv, const float* proj, float* scratch, float* partials,
+                                            float* sums, float* g_proj,
+                                            int B, int N, int H, int W, float w_l1, float w_ssim, int flags, void* stream) {
+    return photo_sweep_grad("tcsfm_photo_sweep_grad_pairs", B, tgt, tgt_sb, tgt_sc, src, src_sb, src_sc, tgt_depth, src_depth,
+                            kinv, proj, scratch, partials, sums, g_proj, N, H, W, w_l1, w_ssim, flags, stream);
 }
 
 extern "C" int tcsfm_photo_refine(const float* tgt, int64_t tgt_sc, const float* src, int64_t src_sc,
@@ -823,51 +973,18 @@ extern "C" int tcsfm_photo_refine(const float* tgt, int64_t tgt_sc, const float*
                                   float* loss, float* best_loss, int* best_step, float* best_pose,
                                   int N, int H, int W, int steps, double lr, double beta1, double beta2, double eps,
                                   float w_l1, float w_ssim, int flags, int pose_flags, void* stream) {
-    const char* who = "tcsfm_photo_refine";
-    if (!K || !poses || !m || !v || !best_loss || !best_step || !best_pose) { set_error("%s: null pointer", who); return 1; }
-    if (steps < 0) { set_error("%s: steps=%d is negative", who, steps); return 1; }
-    if (N > 0 && ((int64_t)steps + 1) * N > 0x7fffffff) {
-        set_error("%s: the loss history of %d steps x %d hypotheses exceeds 2^31 - 1 entries", who, steps, N); return 1;
-    }
-    if (!(lr > 0.0 && lr < INFINITY) || !(eps > 0.0 && eps < INFINITY) || !(beta1 >= 0.0 && beta1 < 1.0) ||
-        !(beta2 >= 0.0 && beta2 < 1.0)) {
-        set_error("%s: bad optimizer arguments lr=%g betas=(%g, %g) eps=%g", who, lr, beta1, beta2, eps); return 1;
-    }
-    // `loss` stands in for the sums of fill_sweep's checks: each row of it is written from the partials here
-    SweepArgs S;
-    if (int rc = fill_sweep(S, who, tgt, tgt_sc, src, src_sc, tgt_depth, src_depth, kinv, proj, scratch, partials, loss,
-                            N, H, W, w_l1, w_ssim, flags)) return rc;
-    const int tiles = S.tiles;
-    if (int rc = sweep_grad_prologue(S, who, flags, stream)) return rc;
-    if (int rc = tcsfm_pose_proj_fwd(poses, kRefineSign, K, 1, proj, N, pose_flags, stream)) return rc;
-    auto* step = (pose_flags & TCSFM_ARITH_BMM_NOFMA) ? photo_refine_step_kernel<true, true> : photo_refine_step_kernel<true, false>;
-    const dim3 step_grid((N + kSweepFinishThreads - 1) / kSweepFinishThreads), step_block(kSweepFinishThreads);
-    RefineArgs R;
-    R.partials = partials; R.K = K; R.poses = poses; R.m = m; R.v = v; R.proj = proj;
-    R.best_loss = best_loss; R.best_step = best_step; R.best_pose = best_pose;
-    R.tiles = tiles; R.N = N;
-    AdamStep s;
-    s.b1 = (float)beta1; s.a1 = (float)(1.0 - beta1); s.b2 = (float)beta2; s.a2 = (float)(1.0 - beta2); s.e = (float)eps;
-    for (int t = 1; t <= steps; ++t) {
-        TCSFM_DISPATCH_FLAVOUR(flags, auto* sweep = photo_sweep_kernel<F, true>;
-                                      TCSFM_LAUNCH(sweep, dim3((unsigned)(tiles * N)), dim3(kTileThreads), kSweepGradSmem, stream, S));
-        if (int rc = check_launch(who)) return rc;
-        s.c1 = (float)(lr / (1.0 - pow(beta1, (double)t)));
-        s.c2 = (float)sqrt(1.0 - pow(beta2, (double)t));
-        s.first = t == 1;
-        R.loss = loss + (int64_t)(t - 1) * N;
-        R.step = t - 1;
-        TCSFM_LAUNCH(step, step_grid, step_block, 0, stream, R, s);
-        if (int rc = check_launch(who)) return rc;
-    }
-    // the poses after the last update: their loss and the last chance to be the best
-    TCSFM_DISPATCH_FLAVOUR(flags, auto* sweep = photo_sweep_kernel<F, false>;
-                                  TCSFM_LAUNCH(sweep, dim3((unsigned)(tiles * N)), dim3(kTileThreads), kSweepSmem, stream, S));
-    if (int rc = check_launch(who)) return rc;
-    s.first = steps == 0;
-    R.loss = loss + (int64_t)steps * N;
-    R.step = steps;
-    auto* last = photo_refine_step_kernel<false, false>;
-    TCSFM_LAUNCH(last, step_grid, step_block, 0, stream, R, s);
-    return check_launch(who);
+    return photo_refine("tcsfm_photo_refine", 1, tgt, 0, tgt_sc, src, 0, src_sc, tgt_depth, src_depth, kinv, K, poses, m, v,
+                        proj, scratch, partials, loss, best_loss, best_step, best_pose, N, H, W, steps, lr, beta1, beta2,
+                        eps, w_l1, w_ssim, flags, pose_flags, stream);
+}
+
+extern "C" int tcsfm_photo_refine_pairs(const float* tgt, int64_t tgt_sb, int64_t tgt_sc, const float* src, int64_t src_sb,
+                                        int64_t src_sc, const float* tgt_depth, const float* src_depth, const float* kinv,
+                                        const float* K, float* poses, float* m, float* v, float* proj, float* scratch,
+                                        float* partials, float* loss, float* best_loss, int* best_step, float* best_pose,
+                                        int B, int N, int H, int W, int steps, double lr, double beta1, double beta2,
+                                        double eps, float w_l1, float w_ssim, int flags, int pose_flags, void* stream) {
+    return photo_refine("tcsfm_photo_refine_pairs", B, tgt, tgt_sb, tgt_sc, src, src_sb, src_sc, tgt_depth, src_depth, kinv,
+                        K, poses, m, v, proj, scratch, partials, loss, best_loss, best_step, best_pose, N, H, W, steps, lr,
+                        beta1, beta2, eps, w_l1, w_ssim, flags, pose_flags, stream);
 }

@@ -5,7 +5,8 @@ helpers.py:8-23).  The optimisation driver itself (deep copies of the depth net,
 Adam, plotting; optimizer.py:136-297) is the reference's harness and calls these.
 ``photometric_loss_surface`` evaluates ``compute_photometric_error`` for N pose hypotheses of one pair in one call
 (the loss-surface plots, plot_loss_surface.py:11-87); ``photometric_loss_surface_and_grad`` also returns the pose
-gradient of every hypothesis's loss, and ``refine_pose_hypotheses`` descends the surface from every hypothesis.
+gradient of every hypothesis's loss, and ``refine_pose_hypotheses`` descends the surface from every hypothesis.  Given
+poses [B,N,6] all three do the same for B frame pairs of N hypotheses each, in one call.
 """
 import math
 import numbers
@@ -92,20 +93,25 @@ def photometric_loss_surface(target_img, source_img, target_depth, source_depth,
     and 'weight_mask' stacked over the N hypotheses.  The maps are bit-identical to N batch-1 calls of
     compute_photometric_error; the sums are added in a fixed order (deterministic), loss = error_sum / valid_sum
     (NaN where no pixel is valid).  Six launches whatever N is: K^-1, K @ [R|t] of every hypothesis, the three of
-    tcsfm_photo_sweep and the division.  Forward only."""
+    tcsfm_photo_sweep and the division.  Forward only.
+
+    B frame pairs of N hypotheses each: poses [B,N,6] or [B,N,8], target_img / source_img [B,3,H,W] (may be channel
+    slices), depths [B,1,H,W], intrinsics [B,3,3].  The outputs gain the leading B ([B,N] sums, [B,N,C,H,W] maps),
+    and row (b, n) holds the bits of the single-pair call on pair b with poses[b].  One more launch, for the rows of
+    K, whatever B is."""
     ops._require_cuda(target_img, source_img, target_depth, source_depth, poses, intrinsics)
     if torch.is_grad_enabled() and any(t.requires_grad for t in (target_img, source_img, target_depth, source_depth,
                                                                      poses, intrinsics)):
         raise NotImplementedError("photometric_loss_surface is forward only: no gradient of the surface is implemented "
                                   "(photometric_loss_surface_and_grad returns the pose gradient)")
-    _check_surface_args(target_img, poses)
+    _check_surface_args(target_img, poses, source_img, target_depth, source_depth, intrinsics)
     h, w = target_img.shape[2], target_img.shape[3]
     kinv = stn.inverse_intrinsics(intrinsics)
     with ops._guard(poses):
-        proj = _surface_projections(poses, intrinsics)
+        proj = _surface_projections(*_hypothesis_rows(poses, intrinsics)).view(poses.shape[:-1] + (3, 4))
         sums, maps = _raw.photo_sweep(ops.lib(), target_img, source_img, target_depth, source_depth, kinv, proj,
                                       0.15, 0.85, ops.arith_flags(1, h, w), want_maps=return_maps)
-    out = {'loss': sums[:, 0] / sums[:, 1], 'error_sum': sums[:, 0], 'valid_sum': sums[:, 1]}
+    out = {'loss': sums[..., 0] / sums[..., 1], 'error_sum': sums[..., 0], 'valid_sum': sums[..., 1]}
     if return_maps:
         out['img_rec'], out['diff_img'], out['valid_mask'], out['weight_mask'] = maps
     return out
@@ -121,19 +127,24 @@ def photometric_loss_surface_and_grad(target_img, source_img, target_depth, sour
     Functional, not autograd: no graph is recorded and the outputs do not require grad (inputs that require grad are
     read as values).  Seven launches whatever N is: K^-1, K @ [R|t] of every hypothesis, the three of
     tcsfm_photo_sweep_grad (the forward is recomputed inside each CTA, so no workspace grows with N * H * W), the chain
-    rule to the pose and the division; [N,8] poses add one for the zero columns."""
+    rule to the pose and the division; [N,8] poses add one for the zero columns.
+
+    B frame pairs as in photometric_loss_surface (poses [B,N,6|8]): [B,N] sums and pose_grad [B,N,6|8], row (b, n)
+    with the bits of the single-pair call on pair b; one more launch, for the rows of K."""
     ops._require_cuda(target_img, source_img, target_depth, source_depth, poses, intrinsics)
-    _check_surface_args(target_img, poses)
+    _check_surface_args(target_img, poses, source_img, target_depth, source_depth, intrinsics)
     h, w = target_img.shape[2], target_img.shape[3]
     with torch.no_grad(), ops._guard(poses):
         kinv = stn.inverse_intrinsics(intrinsics)
-        proj = _surface_projections(poses, intrinsics)
+        rows, k_rows = _hypothesis_rows(poses, intrinsics)
+        proj = _surface_projections(rows, k_rows).view(poses.shape[:-1] + (3, 4))
         sums, g_proj = _raw.photo_sweep_grad(ops.lib(), target_img, source_img, target_depth, source_depth, kinv, proj,
                                              0.15, 0.85, ops.arith_flags(1, h, w))
-        pose_grad = _raw.pose_proj_bwd(ops.lib(), poses[:, 0:6], intrinsics, -1.0, g_proj)
-        if poses.shape[1] > 6:
-            pose_grad = torch.nn.functional.pad(pose_grad, (0, poses.shape[1] - 6))
-        return {'loss': sums[:, 0] / sums[:, 1], 'error_sum': sums[:, 0], 'valid_sum': sums[:, 1],
+        pose_grad = _raw.pose_proj_bwd(ops.lib(), rows[:, 0:6], k_rows, -1.0, g_proj.view(-1, 3, 4))
+        pose_grad = pose_grad.view(poses.shape[:-1] + (6,))
+        if poses.shape[-1] > 6:
+            pose_grad = torch.nn.functional.pad(pose_grad, (0, poses.shape[-1] - 6))
+        return {'loss': sums[..., 0] / sums[..., 1], 'error_sum': sums[..., 0], 'valid_sum': sums[..., 1],
                 'pose_grad': pose_grad}
 
 
@@ -158,19 +169,23 @@ def refine_pose_hypotheses(target_img, source_img, target_depth, source_depth, p
     written.  2 * steps + 6 launches for [N,6] poses: K^-1, the 2 * steps + 4 of tcsfm_photo_refine (the auto-mask
     error, K[R|t] of the starting poses, per step the fused forward + adjoint and the update, then the last
     evaluation) and best_step's int64 copy; [N,8] poses add two for their columns 6:.  No host work between the
-    steps, the same bits on every call, and capturable in a CUDA graph."""
+    steps, the same bits on every call, and capturable in a CUDA graph.
+
+    B frame pairs as in photometric_loss_surface (poses [B,N,6|8], each pair descending with its own intrinsics), with
+    the same launch count: 'poses' and 'best_pose' [B,N,6|8], 'loss' [steps+1,B,N], 'best_loss' and 'best_step'
+    [B,N]; entry (b, n) has the bits of the single-pair call on pair b with poses[b]."""
     ops._require_cuda(target_img, source_img, target_depth, source_depth, poses, intrinsics)
-    _check_surface_args(target_img, poses)
+    _check_surface_args(target_img, poses, source_img, target_depth, source_depth, intrinsics)
     steps, lr, beta1, beta2, eps = _check_adam_args(steps, lr, betas, eps)
     h, w = target_img.shape[2], target_img.shape[3]
     with torch.no_grad(), ops._guard(poses):
         kinv = stn.inverse_intrinsics(intrinsics)
         final, loss, best_loss, best_step, best_pose = _raw.photo_refine(
-            ops.lib(), target_img, source_img, target_depth, source_depth, kinv, intrinsics, poses[:, 0:6], steps, lr,
+            ops.lib(), target_img, source_img, target_depth, source_depth, kinv, intrinsics, poses[..., 0:6], steps, lr,
             beta1, beta2, eps, 0.15, 0.85, ops.arith_flags(1, h, w), ops.pose_flags(1))
-        if poses.shape[1] > 6:
-            final = torch.cat([final, poses[:, 6:]], 1)
-            best_pose = torch.cat([best_pose, poses[:, 6:]], 1)
+        if poses.shape[-1] > 6:
+            final = torch.cat([final, poses[..., 6:]], -1)
+            best_pose = torch.cat([best_pose, poses[..., 6:]], -1)
         return {'poses': final, 'loss': loss, 'best_loss': best_loss, 'best_step': best_step.long(),
                 'best_pose': best_pose}
 
@@ -194,12 +209,36 @@ def _check_adam_args(steps, lr, betas, eps):
     return int(steps), lr, beta1, beta2, eps
 
 
-def _check_surface_args(target_img, poses):
+def _check_surface_args(target_img, poses, source_img, target_depth, source_depth, intrinsics):
+    """poses [N,6|8]: one frame pair (batch-1 inputs); poses [B,N,6|8]: B pairs, whose inputs must all have batch B."""
+    if poses.dim() == 3:
+        b = poses.shape[0]
+        if b < 1 or poses.shape[1] < 1 or poses.shape[2] not in (6, 8):
+            raise ValueError("photometric_loss_surface: poses must be [B,N,6] or [B,N,8] with B, N >= 1, got %s"
+                             % list(poses.shape))
+        for t, c, name in ((target_img, 3, "target_img"), (source_img, 3, "source_img"),
+                           (target_depth, 1, "target_depth"), (source_depth, 1, "source_depth")):
+            if t.dim() != 4 or t.shape[0] != b or t.shape[1] != c:
+                raise ValueError("photometric_loss_surface: %s must be [B,%d,H,W] with the B = %d of poses [B,N,%d], "
+                                 "got %s" % (name, c, b, poses.shape[2], list(t.shape)))
+        if tuple(intrinsics.shape) != (b, 3, 3):
+            raise ValueError("photometric_loss_surface: intrinsics must be [B,3,3] with the B = %d of poses, got %s"
+                             % (b, list(intrinsics.shape)))
+        return
     if target_img.dim() != 4 or target_img.shape[0] != 1:
-        raise ValueError("photometric_loss_surface: one frame pair (batch 1) per call, got target_img %s"
-                         % list(target_img.shape))
+        raise ValueError("photometric_loss_surface: one frame pair (batch 1) per call, or pass poses [B,N,6] for B "
+                         "pairs, got target_img %s" % list(target_img.shape))
     if poses.dim() != 2 or poses.shape[0] < 1 or poses.shape[1] not in (6, 8):
         raise ValueError("photometric_loss_surface: poses must be [N,6] or [N,8] with N >= 1, got %s" % list(poses.shape))
+
+
+def _hypothesis_rows(poses, intrinsics):
+    """(pose rows [R,6|8], intrinsics [R,3,3] or [1,3,3]) with row r the intrinsics of pose row r: the rows of
+    [B,N,6|8] poses are pair-major, so pair b's K is repeated N times."""
+    if poses.dim() == 3:
+        b, n = poses.shape[0], poses.shape[1]
+        return poses.reshape(b * n, poses.shape[2]), intrinsics[:, None].expand(b, n, 3, 3).reshape(b * n, 3, 3)
+    return poses, intrinsics
 
 
 def _surface_projections(poses, intrinsics):

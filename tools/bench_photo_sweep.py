@@ -21,6 +21,17 @@ The refine section runs N = 8, 100 (the demo's) and 200 (bench.py's); both ways 
 [steps+1, N] loss history.  The two do not give the same bits (torch's Adam rounds differently), so no difference is
 reported for them.
 
+and, for B frame pairs of N hypotheses each (the "pairs" section), surface and refine:
+
+  loop   a Python loop of B single-pair calls (photometric_loss_surface, or refine_pose_hypotheses with
+         `--refine-steps`), the results stacked;
+  batch  one call with poses [B,N,6].
+
+B = 4, N = 100 is the demo's four surfaces per epoch; B = 32, N = 8 is config 2's 2*S*B pose / pair combinations of
+a minibatch with a few starts each.  The frames are make_frames(B, 192, 640, ...) with the same seed and intrinsics
+as above, and each pair's N hypotheses are the two +-0.05 lines of N / 2 samples around its pose.  Both ways give the
+same bits ("identical").
+
 Input: what `bench.py --workload sweep` evaluates, make_frames(1, 192, 640, n_src=2, seed=0, KITTI intrinsics) with a
 line of forward-translation (pose column 2) and a line of yaw (column 4) samples, linspace(-0.05, 0.05, n) each:
 n = 100 (bench.py's default --sweep-evals, N = 200) and n = 50 (the demo's, N = 100).  Both are timed like
@@ -28,7 +39,8 @@ main_sweep: wall clock of a whole sweep including the final device-to-host copy,
 alternated round by round.  The batched op's device time per call comes from CUDA events around `--device-iters`
 back-to-back calls, next to the forward-only call's in the grad section.  The working set (one frame pair, ~2.5 MB) stays in L2, so no HBM roofline fraction is claimed.
 
-Usage: python tools/bench_photo_sweep.py [--rounds R] [--device-iters I] [--refine-steps S] [--refine-iters J]"""
+Usage: python tools/bench_photo_sweep.py [--rounds R] [--device-iters I] [--refine-steps S] [--refine-iters J]
+                                        [--sections surface,grad,refine,pairs]"""
 import argparse
 import json
 import os
@@ -248,13 +260,72 @@ def measure_refine(fr, n, rounds, steps, device_iters):
             "device_calls_timed": device_iters}
 
 
+def measure_pairs(B, n, rounds, steps, device_iters, refine_iters):
+    """B pairs of 2 * n hypotheses: a loop of B single-pair calls against one batched call, surface and refine."""
+    dev = torch.device("cuda:0")
+    fr = synth.make_frames(B, 192, 640, n_src=2, seed=0, device=dev, intrinsics=torch.tensor(synth.KITTI_K))
+    args = (fr["target"], fr["sources"][0], fr["depths"][0], fr["depths"][1])
+    K = fr["K"]
+    deltas = torch.linspace(-0.05, 0.05, n, device=dev)
+    poses = fr["poses"][0][:, None].repeat(1, 2 * n, 1)
+    poses[:, :n, 2] += deltas
+    poses[:, n:, 4] += deltas
+
+    def pair(b):
+        return tuple(a[b:b + 1] for a in args)
+
+    fns = {
+        "surface": (lambda: torch.stack([pft.photometric_loss_surface(*pair(b), poses[b], K[b:b + 1])["loss"]
+                                         for b in range(B)]),
+                    lambda: pft.photometric_loss_surface(*args, poses, K)["loss"], device_iters),
+        "refine": (lambda: torch.stack([pft.refine_pose_hypotheses(*pair(b), poses[b], K[b:b + 1], steps=steps)["loss"]
+                                        for b in range(B)], 1),
+                   lambda: pft.refine_pose_hypotheses(*args, poses, K, steps=steps)["loss"], refine_iters),
+    }
+    out = {"B": B, "N": 2 * n, "steps": steps}
+    with torch.no_grad():
+        for name, (loop, batch, iters) in fns.items():
+            def timed(fn):
+                torch.cuda.synchronize()
+                t0 = time.perf_counter()
+                host = fn().cpu()
+                return time.perf_counter() - t0, host
+
+            loop(), batch()                         # warm-up
+            t_loop, t_batch = [], []
+            for _ in range(rounds):
+                dt, ref = timed(loop)
+                t_loop.append(dt)
+                dt, got = timed(batch)
+                t_batch.append(dt)
+            torch.cuda.synchronize()
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            e0.record()
+            for _ in range(iters):
+                batch()
+            e1.record()
+            torch.cuda.synchronize()
+            out[name] = {"loop_ms": round(statistics.median(t_loop) * 1e3, 3),
+                         "batch_ms": round(statistics.median(t_batch) * 1e3, 3),
+                         "speedup": round(statistics.median(t_loop) / statistics.median(t_batch), 2),
+                         "loop_ms_rounds": [round(t * 1e3, 3) for t in t_loop],
+                         "batch_ms_rounds": [round(t * 1e3, 3) for t in t_batch],
+                         "batch_device_ms_per_call": round(e0.elapsed_time(e1) / iters, 4),
+                         "device_calls_timed": iters,
+                         "identical": bool(torch.equal(got.isnan(), ref.isnan())
+                                           and torch.equal(got.nan_to_num(), ref.nan_to_num()))}
+    return out
+
+
 def main():
     ap = argparse.ArgumentParser(description=__doc__.splitlines()[0])
     ap.add_argument("--rounds", type=int, default=5, help="alternated loop / batch sweeps per configuration")
     ap.add_argument("--device-iters", type=int, default=200, help="back-to-back calls timed with CUDA events")
     ap.add_argument("--refine-steps", type=int, default=50, help="Adam steps per descent in the refine section")
     ap.add_argument("--refine-iters", type=int, default=20, help="back-to-back refine calls timed with CUDA events")
+    ap.add_argument("--sections", default="surface,grad,refine,pairs", help="comma-separated sections to run")
     args = ap.parse_args()
+    sections = set(args.sections.split(","))
     if not torch.cuda.is_available():
         sys.exit("bench_photo_sweep.py needs a CUDA device")
     dev = torch.device("cuda:0")
@@ -265,18 +336,27 @@ def main():
             "unit": "evals/s", "gpu": name, "power_limit": power, "dtype": "f32", "data": "synthetic",
             "timing": "wall clock of a whole sweep incl. the final D2H, median of alternated rounds; device time from "
                       "CUDA events",
-            "note": "working set (one frame pair, ~2.5 MB) is L2-resident: no HBM roofline fraction is claimed",
-            "configs": {"bench_sweep_default_100x2": measure(fr, 100, args.rounds, args.device_iters),
-                        "demo_50x2": measure(fr, 50, args.rounds, args.device_iters)},
-            "grad": {"metric": "loss-surface evaluations with the pose gradient per s: batch-1 forward + backward loop "
-                               "vs one photometric_loss_surface_and_grad call",
-                     "max_rel_diff": "largest |pose_grad - loop| / |loop| over the rows",
-                     "configs": {"bench_sweep_default_100x2": measure_grad(fr, 100, args.rounds, args.device_iters),
-                                 "demo_50x2": measure_grad(fr, 50, args.rounds, args.device_iters)}},
-            "refine": {"metric": "multi-start refinement, ms per descent of N starts: the surface_and_grad + "
-                                 "torch.optim.Adam loop vs one refine_pose_hypotheses call",
-                       "configs": {"N%d" % (2 * n): measure_refine(fr, n, args.rounds, args.refine_steps, args.refine_iters)
-                                   for n in (4, 50, 100)}}}
+            "note": "working set (one frame pair, ~2.5 MB) is L2-resident: no HBM roofline fraction is claimed"}
+    if "surface" in sections:
+        line["configs"] = {"bench_sweep_default_100x2": measure(fr, 100, args.rounds, args.device_iters),
+                           "demo_50x2": measure(fr, 50, args.rounds, args.device_iters)}
+    if "grad" in sections:
+        line["grad"] = {"metric": "loss-surface evaluations with the pose gradient per s: batch-1 forward + backward "
+                                  "loop vs one photometric_loss_surface_and_grad call",
+                        "max_rel_diff": "largest |pose_grad - loop| / |loop| over the rows",
+                        "configs": {"bench_sweep_default_100x2": measure_grad(fr, 100, args.rounds, args.device_iters),
+                                    "demo_50x2": measure_grad(fr, 50, args.rounds, args.device_iters)}}
+    if "refine" in sections:
+        line["refine"] = {"metric": "multi-start refinement, ms per descent of N starts: the surface_and_grad + "
+                                    "torch.optim.Adam loop vs one refine_pose_hypotheses call",
+                          "configs": {"N%d" % (2 * n): measure_refine(fr, n, args.rounds, args.refine_steps,
+                                                                      args.refine_iters) for n in (4, 50, 100)}}
+    if "pairs" in sections:
+        line["pairs"] = {"metric": "B frame pairs of N hypotheses, ms per call: a loop of B single-pair calls vs one "
+                                   "call with poses [B,N,6] (surface, and refine with --refine-steps)",
+                         "configs": {"B%d_N%d" % (B, 2 * n): measure_pairs(B, n, args.rounds, args.refine_steps,
+                                                                             args.device_iters, args.refine_iters)
+                                     for B, n in ((4, 50), (32, 4))}}
     print(json.dumps(line))
 
 
